@@ -2,6 +2,7 @@
 """bench.py -- throughput of the pixel-pipeline hot path on B200, one process per GPU.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg4|cfg3|cfg2|cfg5]
+                    [--dump-outputs DIR]
 
 Workload (default): BASELINE.json configs[3], the 4K batch `metric` is quoted on -- 1024 frames of
 3840x2160 RGB24 per GPU, 4:2:0 (a=2,b=0) -> spatial f=2 -> 8/8/8 bits, BUNDLE128 output, one fused
@@ -270,6 +271,40 @@ class Env:
         return outt.tolist()
 
 
+def make_inputs(torch, frames, H, W, ipb, seed):
+    """The batch a run times: uniform random bytes generated in HBM from `seed`, the same in every run."""
+    gen = torch.Generator(device="cuda").manual_seed(seed)
+    rgb = torch.empty((frames, H, W, ipb), dtype=torch.uint8, device="cuda")
+    step_f = max(1, (1 << 29) // (W * H * ipb))      # chunked: randint materialises int64 temporaries for some dtypes
+    for i in range(0, frames, step_f):
+        rgb[i:i + step_f] = torch.randint(0, 256, rgb[i:i + step_f].shape, dtype=torch.uint8, device="cuda", generator=gen)
+    return rgb
+
+
+DUMP_SAMPLES = 1 << 22      # 16 MB of float32 values + 32 MB of float64 positions: under 64 MB for any workload
+
+
+def dump_index(total, n=DUMP_SAMPLES):
+    """Flat positions of the output bytes --dump-outputs writes: all of them when there are at most n, else a fixed
+    seeded sample of n distinct positions, ascending."""
+    import numpy as np
+    if total <= n:
+        return np.arange(total, dtype=np.int64)
+    return np.sort(np.random.default_rng(0xD0).choice(total, size=n, replace=False))
+
+
+def dump_outputs(dirpath, out):
+    """Writes the output of the last timed step (`out`, uint8 [frames, bytes per frame]) as DIR/out.npy (float32 byte
+    values) and DIR/out_index.npy (float64 flat positions in `out`: frame * bytes_per_frame + byte)."""
+    import numpy as np
+    import torch
+    idx = dump_index(out.numel())
+    vals = out.reshape(-1)[torch.from_numpy(idx).to(out.device)].cpu().numpy()
+    os.makedirs(dirpath, exist_ok=True)
+    np.save(os.path.join(dirpath, "out.npy"), vals.astype(np.float32))
+    np.save(os.path.join(dirpath, "out_index.npy"), idx.astype(np.float64))
+
+
 def device_run(env, ctx, name, frames, shard, steps, warmup, graph, in_format=0, verify=True, replays=1, one_gpu_too=False):
     """Inputs resident in HBM, one kernel launch per step, CUDA events on the launching stream, max over ranks.
     Every rank does the same untimed work first (parity spot check, full-batch cross-check, W warm-up steps).
@@ -286,11 +321,7 @@ def device_run(env, ctx, name, frames, shard, steps, warmup, graph, in_format=0,
     ipb = 3 if in_format == 0 else 4
     _, out_h, _, out_fb = csic.out_shape(p)
 
-    gen = torch.Generator(device="cuda").manual_seed(0x5EED + (env.rank if shard == "frames" else 0))
-    rgb = torch.empty((frames, H, W, ipb), dtype=torch.uint8, device="cuda")
-    step_f = max(1, (1 << 29) // (W * H * ipb))      # chunked: randint materialises int64 temporaries for some dtypes
-    for i in range(0, frames, step_f):
-        rgb[i:i + step_f] = torch.randint(0, 256, rgb[i:i + step_f].shape, dtype=torch.uint8, device="cuda", generator=gen)
+    rgb = make_inputs(torch, frames, H, W, ipb, 0x5EED + (env.rank if shard == "frames" else 0))
     out = torch.empty((frames, out_fb), dtype=torch.uint8, device="cuda")
 
     # parity spot check (outside the timed region, on every rank): one frame against the oracle
@@ -583,7 +614,12 @@ def main():
     ap.add_argument("--shard", default="frames", choices=["frames", "bands"],
                     help="frames: every rank owns its own batch (weak scaling).  bands: every rank owns one aligned "
                          "row band of EVERY frame of one shared batch (strong scaling; BASELINE configs[4])")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write rank 0's output of the last step to DIR/out.npy with the flat "
+                         "positions in DIR/out_index.npy (every byte, or a fixed seeded sample of 4 Mi of them)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     wl = WORKLOADS[args.workload]
     if args.impl == "reference":
@@ -612,10 +648,14 @@ def main():
     if args.chunk_mb:
         ctx.set_option(1, args.chunk_mb << 20)
     default_run = args.workload == "cfg4" and args.shard == "frames" and not args.family
+    if args.dump_outputs and args.shard == "bands" and env.world > 1:
+        sys.exit("--dump-outputs with --shard bands needs one GPU: rank 0 computes only its own band")
 
     main_res = device_run(env, ctx, args.workload, frames, args.shard, args.steps, args.warmup, args.graph,
                           in_format=args.in_format, verify=not args.no_verify, replays=args.replays)
     p, rgb, out, ipb, out_fb = main_res.pop("_state")
+    if args.dump_outputs and env.rank == 0:
+        dump_outputs(args.dump_outputs, out)
     tp = os.path.join(ROOT, "profiles", "traffic.json")
     if os.path.exists(tp) and args.shard == "frames":
         try:

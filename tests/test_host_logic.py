@@ -215,3 +215,40 @@ def test_bench_reference_arm_contract():
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["e2e"]["d2h_bytes_per_step"] == 0 and "workload" in line["config"]
     r = subprocess.run(cmd, capture_output=True, text=True, timeout=300, env=dict(os.environ, RANK="1", WORLD_SIZE="2"))
     assert r.returncode == 0 and r.stdout.strip() == ""
+
+
+def test_bench_rejects_zero_steps():
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True, timeout=120)
+    assert r.returncode == 2 and "--steps must be at least 1" in r.stderr
+
+
+@pytest.mark.gpu
+def test_bench_dump_outputs_are_the_timed_outputs(tmp_path):
+    """--dump-outputs: two runs with the same arguments write the same files (float32 values, float64 positions, at most
+    64 MB), which equal the oracle on the bench's own inputs at the sampled positions; --steps sets the timed launches."""
+    import json
+    import torch
+    import bench
+    import oracle
+    name, frames = "cfg2", 32                         # 6.3 MB of output: more than the sample, so the seeded sample is taken
+    W, H, _, a, b, q, f, order, fmt, _ = bench.WORKLOADS[name]
+    dumps = []
+    for run in range(2):
+        d = tmp_path / f"run{run}"
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", name, "--frames", str(frames),
+                            "--steps", "4", "--warmup", "0", "--no-e2e", "--no-cpu", "--no-verify", "--dump-outputs", str(d)],
+                           capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, r.stderr[-2000:]
+        line = json.loads(r.stdout.strip().splitlines()[-1])
+        assert line["steps"] == 4 and line["gpu_launches"] == 4
+        assert sorted(os.listdir(d)) == ["out.npy", "out_index.npy"]
+        assert sum(os.path.getsize(d / n) for n in os.listdir(d)) <= 64 << 20
+        vals, idx = np.load(d / "out.npy"), np.load(d / "out_index.npy")
+        assert vals.dtype == np.float32 and idx.dtype == np.float64
+        dumps.append((vals, idx))
+    assert np.array_equal(dumps[0][0], dumps[1][0]) and np.array_equal(dumps[0][1], dumps[1][1])
+    rgb = bench.make_inputs(torch, frames, H, W, 3, 0x5EED).cpu().numpy()
+    want = oracle.process(oracle.make_params(W, H, a, b, q, f, order, out_format=fmt), rgb, threads=4).reshape(-1)
+    vals, idx = dumps[0]
+    assert want.size > bench.DUMP_SAMPLES and np.array_equal(idx, bench.dump_index(want.size))
+    assert np.array_equal(vals, want[idx.astype(np.int64)])
