@@ -1,10 +1,11 @@
-// Device half of the C ABI: contexts, plan construction, the device / band / host entry points.
+// Device half of the C ABI: contexts, the device / band / host entry points (plans come from csic_plan.cpp).
 // No CPU compute path exists here: every process call ends in a kernel launch or an error code.
 #include <cuda_runtime.h>
 
 #include <algorithm>
 #include <atomic>
 #include <cstdio>
+#include <cstdlib>
 #include <cstring>
 #include <new>
 #include <string>
@@ -57,8 +58,7 @@ int guarded(const char* where, F&& body) {
 
 struct csic_ctx {
   int device = 0;
-  int sm_count = 0;
-  size_t max_smem_optin = 0;
+  csic::DeviceLimits dev = {};
   cudaStream_t stream = nullptr;             // default compute stream
   cudaStream_t s_h2d = nullptr, s_d2h = nullptr;
   void* d_in[kPipe] = {nullptr, nullptr, nullptr};
@@ -71,12 +71,8 @@ struct csic_ctx {
   int opt_no_bounce = 0;
   int last_family = 0;
   int64_t launches = 0;
-  int opt_family = 0;
+  csic::PlanOptions opt;                     // csic_set_option's planner knobs
   size_t opt_chunk_bytes = kDefaultChunkBytes;
-  int opt_ctas_per_sm = 0;
-  int opt_stages = 0;
-  uint32_t opt_tile_bytes = 0;
-  int opt_block_threads = 0;
   int opt_no_compact = 0;
   uint64_t h2d_bytes = 0;    // bytes csic_process_host has shipped host -> device so far
 };
@@ -101,119 +97,28 @@ bool can_compact(const csic_params& p) {
   return p.pool_mode == CSIC_POOL_DECIMATE && p.factor > 1 && p.height % p.factor == 0;
 }
 
-// Optional non-dense device layout: row pitches and frame strides in bytes (0 = dense).
-struct Layout {
-  size_t in_pitch = 0, in_frame = 0, out_pitch = 0, out_frame = 0;
-  bool short_frames = false;   // the buffers hold only one row band of each frame (host band path)
-};
-
-int build_plan(const csic_params& p, const void* d_rgb, void* d_out, size_t n_frames, int32_t row0,
-               int32_t rows, bool compact, const Layout& lay, csic::KPlan& k) {
-  const csic::Geometry g = csic::geometry(p);
-  std::memset(&k, 0, sizeof(k));
-  k.in = static_cast<const uint8_t*>(d_rgb);
-  k.out = static_cast<uint8_t*>(d_out);
-  k.compact = compact ? 1 : 0;
-  k.row_step = compact ? 1 : p.factor;
-  k.in_frame_bytes = compact ? g.in_row_bytes * (size_t)g.out_h : g.in_frame_bytes;
-  k.out_frame_bytes = g.out_frame_bytes;
-  if (g.in_row_bytes > 0xFFFFFFFFull || g.out_row_bytes > 0xFFFFFFFFull) return CSIC_EINVAL_DIMS;
-  if ((uint64_t)g.out_w * (uint64_t)g.out_h >= (1ull << 31) || (uint64_t)p.width * p.height >= (1ull << 31))
-    return CSIC_EINVAL_DIMS;   // the reference's counters are far narrower; 2^31 pixels per frame is our limit
-  k.in_row_bytes = (uint32_t)g.in_row_bytes;
-  k.out_row_bytes = (uint32_t)g.out_row_bytes;
-  if (lay.in_pitch) {
-    if (lay.in_pitch < g.in_row_bytes || lay.in_pitch > 0xFFFFFFFFull) return CSIC_EINVAL_ARG;
-    k.in_row_bytes = (uint32_t)lay.in_pitch;
-    k.in_frame_bytes = (size_t)lay.in_pitch * (size_t)(compact ? g.out_h : p.height);
-  }
-  if (lay.in_frame) {
-    if (lay.in_frame < k.in_frame_bytes && !lay.short_frames) return CSIC_EINVAL_ARG;
-    k.in_frame_bytes = lay.in_frame;
-  }
-  if ((lay.out_pitch || lay.out_frame || lay.short_frames) && p.out_format == CSIC_OUT_PLANAR)
-    return CSIC_EINVAL_MODE;   // three planes per frame: no pitched / banded host layout
-  if (lay.out_pitch) {
-    if (lay.out_pitch < g.out_row_bytes || lay.out_pitch > 0xFFFFFFFFull) return CSIC_EINVAL_ARG;
-    k.out_row_bytes = (uint32_t)lay.out_pitch;
-    k.out_frame_bytes = (size_t)lay.out_pitch * (size_t)g.out_h;
-  }
-  if (lay.out_frame) {
-    if (lay.out_frame < k.out_frame_bytes && !lay.short_frames) return CSIC_EINVAL_ARG;
-    k.out_frame_bytes = lay.out_frame;
-  }
-  k.in_px_bytes = g.in_px_bytes;
-  auto swap_rb = [](uint32_t c) { return (c & 0xFF00FF00u) | ((c & 0xFFu) << 16) | ((c >> 16) & 0xFFu); };
-  const bool bgr = p.in_format == CSIC_IN_BGRA32;
-  k.coef_y = bgr ? swap_rb(0x001D964Du) : 0x001D964Du;      //  77, 150,  29, 0
-  k.coef_ncb = bgr ? swap_rb(0x0080552Bu) : 0x0080552Bu;    //  43,  85,-128, 0  (negated Cb row)
-  k.coef_ncr = bgr ? swap_rb(0x00156B80u) : 0x00156B80u;    //-128, 107,  21, 0  (negated Cr row)
-  k.W = p.width;
-  k.H = p.height;
-  k.Wo = g.out_w;
-  k.Ho = g.out_h;
-  k.f = p.factor;
-  k.hf = g.hf;
-  k.vf = g.vf;
-  k.last_sample_col = ((p.width - 1) / g.hf) * g.hf;
-  // Spatial before chroma runs the chroma stage with misaligned counters (ImageCompressorTop.scala:52-58) -- which only
-  // matters when that stage holds anything: with 4:4:4 (hf == vf == 1, the application's default) every element is its
-  // own sample point whatever the counters say, so any width takes the fast kernels.
-  k.case_b = (!g.chroma_first && p.factor > 1 && (g.hf > 1 || g.vf > 1)) ? 1 : 0;
-  k.quant_first = g.quant_first ? 1 : 0;
-  k.trunc = p.round_mode == CSIC_ROUND_TRUNC;
-  k.average = (p.pool_mode == CSIC_POOL_AVERAGE && p.factor > 1) ? 1 : 0;
-  if (p.out_format == CSIC_OUT_YCC888) k.kformat = csic::KF_YCC888;
-  else if (p.out_format == CSIC_OUT_RGB888) k.kformat = csic::KF_RGB888;
-  else if (p.out_format == CSIC_OUT_PLANAR) k.kformat = csic::KF_PLANAR;
-  else k.kformat = g.out_px_bytes == 1 ? csic::KF_SLOT8 : (g.out_px_bytes == 2 ? csic::KF_SLOT16 : csic::KF_SLOT32);
-  k.slot_bytes = g.out_px_bytes;
-  k.slots_per_row = (k.kformat <= csic::KF_RGB888 || k.kformat == csic::KF_PLANAR)
-                        ? g.out_w : (int32_t)(g.out_row_bytes / (size_t)g.out_px_bytes);
-  k.planar_hs = g.planar_hs; k.planar_vs = g.planar_vs; k.planar_cw = g.planar_cw; k.planar_ch = g.planar_ch;
-  k.planar_cb_off = (uint64_t)g.out_w * (uint64_t)g.out_h;
-  k.planar_cr_off = k.planar_cb_off + (uint64_t)g.planar_cw * (uint64_t)g.planar_ch;
-  k.sy = 8 - p.y_bits;
-  k.scb = 8 - p.cb_bits;
-  k.scr = 8 - p.cr_bits;
-  k.cb_bits = p.cb_bits;
-  k.cr_bits = p.cr_bits;
-  k.qmask = ((0xFFu << k.sy) & 0xFFu) | (((0xFFu << k.scb) & 0xFFu) << 8) | (((0xFFu << k.scr) & 0xFFu) << 16);
-  k.row0 = row0;
-  k.band_rows = rows;
-  if (n_frames > 0xFFFFFFFFull) return CSIC_EINVAL_ARG;
-  k.n_frames = (uint32_t)n_frames;
-  return CSIC_OK;
-}
-
 int run(csic_ctx* ctx, const csic_params* p, const void* d_rgb, size_t n_frames, void* d_out, int32_t row0,
-        int32_t rows, void* cuda_stream, bool compact = false, const Layout& lay = Layout()) {
+        int32_t rows, void* cuda_stream, bool compact = false, const csic::Layout& lay = csic::Layout()) {
   if (!ctx || !p) return CSIC_EINVAL_ARG;
   int rc = csic_validate(p, nullptr, 0);
   if (rc != CSIC_OK) return rc;
   if (n_frames == 0 || rows == 0) return CSIC_OK;
   if (!d_rgb || !d_out) return CSIC_EINVAL_ARG;
-  csic::KPlan k;
-  rc = build_plan(*p, d_rgb, d_out, n_frames, row0, rows, compact, lay, k);
+  csic::KPlan base;
+  rc = csic::build_plan(*p, d_rgb, d_out, n_frames, row0, rows, compact, lay, base);
   if (rc != CSIC_OK) return rc;
-  if (row0 < 0 || rows < 0 || row0 + rows > k.Ho) return CSIC_EINVAL_ARG;
+  if (row0 < 0 || rows < 0 || row0 + rows > base.Ho) return CSIC_EINVAL_ARG;
   DeviceGuard guard(ctx->device);
   cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : ctx->stream;
-  k.block_threads = ctx->opt_block_threads;
+  const csic::KernelChoice c = csic::select_kernel(base, ctx->dev, ctx->opt);
   int err;
-  if (ctx->opt_family == 0 && csic::plan_rows_kernel(k, ctx->sm_count, ctx->max_smem_optin, ctx->opt_stages, ctx->opt_tile_bytes)) {
-    err = csic::launch_rows(k, ctx->sm_count, ctx->opt_ctas_per_sm, st);
-    ctx->last_family = 2;
-  } else if (ctx->opt_family == 0 && csic::plan_pool_kernel(k, ctx->sm_count, ctx->max_smem_optin)) {
-    err = csic::launch_pool(k, ctx->sm_count, ctx->opt_ctas_per_sm, st);
-    ctx->last_family = 3;
-  } else if (ctx->opt_family != 1 && csic::plan_flex_kernel(k, ctx->sm_count, ctx->max_smem_optin, ctx->opt_stages, ctx->opt_tile_bytes)) {
-    err = csic::launch_flex(k, ctx->sm_count, ctx->opt_ctas_per_sm, st);
-    ctx->last_family = 4;
-  } else {
-    err = csic::launch_generic(k, ctx->sm_count, st);
-    ctx->last_family = 1;
+  switch (c.family) {
+    case csic::FAM_ROWS: err = csic::launch_rows(c.k, c.grid, st); break;
+    case csic::FAM_POOL: err = csic::launch_pool(c.k, c.grid, st); break;
+    case csic::FAM_FLEX: err = csic::launch_flex(c.k, c.grid, st); break;
+    default: err = csic::launch_generic(c.k, c.grid, st); break;
   }
+  ctx->last_family = c.family;
   ctx->launches += 1;
   if (err != (int)cudaSuccess) return cuda_fail((cudaError_t)err, "kernel launch");
   return CSIC_OK;
@@ -275,8 +180,7 @@ int csic_create(int device, csic_ctx** out) {
     g_last_error = "device is not sm_100 (Blackwell B200); this library is built for sm_100a only";
     return CSIC_ENODEVICE;
   }
-  c->sm_count = prop.multiProcessorCount;
-  c->max_smem_optin = prop.sharedMemPerBlockOptin;
+  c->dev = {prop.multiProcessorCount, prop.sharedMemPerBlockOptin};
   // keep the FIRST failing call's own error code (cudaGetLastError may already read cudaSuccess again), and tear down
   // whatever was created before it
   cudaError_t err = cudaSuccess;
@@ -288,7 +192,7 @@ int csic_create(int device, csic_ctx** out) {
     step(cudaEventCreateWithFlags(&c->ev_h2d[i], cudaEventDisableTiming)) &&
         step(cudaEventCreateWithFlags(&c->ev_k[i], cudaEventDisableTiming)) &&
         step(cudaEventCreateWithFlags(&c->ev_d2h[i], cudaEventDisableTiming));
-  if (err == cudaSuccess) step((cudaError_t)csic::rows_kernel_set_attributes(c->max_smem_optin));
+  if (err == cudaSuccess) step((cudaError_t)csic::rows_kernel_set_attributes(c->dev.max_smem_optin));
   if (err != cudaSuccess) {
     const int rc = cuda_fail(err, "csic_create");
     const std::string keep = g_last_error;
@@ -326,7 +230,7 @@ int csic_set_option(csic_ctx* ctx, int option, int64_t value) {
   switch (option) {
     case CSIC_OPT_KERNEL_FAMILY:
       if (value < 0 || value > 2) return CSIC_EINVAL_ARG;
-      ctx->opt_family = (int)value;
+      ctx->opt.family = (int)value;
       return CSIC_OK;
     case CSIC_OPT_HOST_CHUNK_BYTES:
       if (value < 0) return CSIC_EINVAL_ARG;
@@ -334,15 +238,15 @@ int csic_set_option(csic_ctx* ctx, int option, int64_t value) {
       return CSIC_OK;
     case CSIC_OPT_GRID_CTAS_PER_SM:
       if (value < 0 || value > 32) return CSIC_EINVAL_ARG;
-      ctx->opt_ctas_per_sm = (int)value;
+      ctx->opt.ctas_per_sm = (int)value;
       return CSIC_OK;
     case CSIC_OPT_STAGES:
       if (value < 0 || value > 16 || value == 1) return CSIC_EINVAL_ARG;
-      ctx->opt_stages = (int)value;
+      ctx->opt.stages = (int)value;
       return CSIC_OK;
     case CSIC_OPT_BLOCK_THREADS:
       if (value < 0 || value > 512 || (value % 32) != 0) return CSIC_EINVAL_ARG;
-      ctx->opt_block_threads = (int)value;
+      ctx->opt.block_threads = (int)value;
       return CSIC_OK;
     case CSIC_OPT_HOST_FULL_FRAMES:
       ctx->opt_no_compact = value != 0;
@@ -352,7 +256,7 @@ int csic_set_option(csic_ctx* ctx, int option, int64_t value) {
       return CSIC_OK;
     case CSIC_OPT_TILE_BYTES:
       if (value < 0 || value > (200 << 10)) return CSIC_EINVAL_ARG;
-      ctx->opt_tile_bytes = (uint32_t)value;
+      ctx->opt.tile_bytes = (uint32_t)value;
       return CSIC_OK;
     default:
       return CSIC_EINVAL_ARG;
@@ -375,7 +279,7 @@ int csic_process_device_pitched(csic_ctx* ctx, const csic_params* p, const void*
   int rc = csic_validate(p, nullptr, 0);
   if (rc != CSIC_OK) return rc;
   const csic::Geometry g = csic::geometry(*p);
-  Layout lay;
+  csic::Layout lay;
   lay.in_pitch = in_pitch_bytes;
   lay.in_frame = in_frame_stride;
   lay.out_pitch = out_pitch_bytes;
@@ -394,12 +298,20 @@ int csic_expand_planar_device(csic_ctx* ctx, const csic_params* p, const void* d
   if (!d_planar || !d_out) return CSIC_EINVAL_ARG;
   const csic::Geometry g = csic::geometry(*p);
   csic::KPlan k;
-  rc = build_plan(*p, d_planar, d_out, n_frames, 0, g.out_h, false, Layout(), k);
+  rc = csic::build_plan(*p, d_planar, d_out, n_frames, 0, g.out_h, false, csic::Layout(), k);
   if (rc != CSIC_OK) return rc;
   DeviceGuard guard(ctx->device);
   cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : ctx->stream;
-  int err = csic::launch_expand_planar(k, static_cast<const uint8_t*>(d_planar), static_cast<uint8_t*>(d_out),
-                                       expand_format == CSIC_OUT_RGB888, ctx->sm_count, ctx->max_smem_optin, st);
+  const int to_rgb = expand_format == CSIC_OUT_RGB888;
+  // test switches, read per call: the LDG decoder instead of the TMA-staged one; pixels per tile
+  const bool no_tma = std::getenv("CSIC_DEC_NO_TMA") != nullptr;
+  const char* tile = std::getenv("CSIC_DEC_TILE");
+  const long tile_px = tile ? std::strtol(tile, nullptr, 10) : 0;
+  // what the TMA-staged decoder declines (rows narrower than a granule, chroma rows too wide for a stage) runs on LDG
+  csic::DecodeLaunch d;
+  const int err = !no_tma && csic::plan_decode(k, to_rgb, ctx->dev, tile_px > 0 ? (uint32_t)tile_px : 0u, d)
+                      ? csic::launch_decode_tma(d, st)
+                      : csic::launch_expand_planar(k, to_rgb, ctx->dev.sm_count, st);
   ctx->launches += 1;
   if (err != (int)cudaSuccess) return cuda_fail((cudaError_t)err, "expand kernel launch");
   return CSIC_OK;
@@ -534,24 +446,21 @@ static int host_pipeline_run(csic_ctx* ctx, const csic_params* p, const uint8_t*
   // Staging layout.  Dense when the dense layout already satisfies a TMA kernel's 16-byte rules; otherwise the
   // rows are re-pitched on the way in and out (the copies are 2-D anyway), so odd widths also avoid the
   // generic kernel.
-  Layout lay;
-  if (ctx->opt_family == 0) {
-    auto eligible = [&](const Layout& l) {
-      csic::KPlan probe;
-      if (build_plan(*p, reinterpret_cast<const void*>(uintptr_t(4096)), reinterpret_cast<void*>(uintptr_t(4096)), 1, 0,
-                     g.out_h, compact, l, probe) != CSIC_OK)
-        return false;
-      probe.block_threads = ctx->opt_block_threads;
-      return csic::plan_rows_kernel(probe, ctx->sm_count, ctx->max_smem_optin, ctx->opt_stages, ctx->opt_tile_bytes) ||
-             csic::plan_pool_kernel(probe, ctx->sm_count, ctx->max_smem_optin);
-    };
-    if (!eligible(Layout()) && p->out_format != CSIC_OUT_PLANAR) {
-      const size_t wp = ((size_t)g.out_w + 15) & ~(size_t)15;
-      Layout cand;
-      cand.in_pitch = (std::max(g.in_row_bytes, wp * (size_t)p->factor * (size_t)g.in_px_bytes) + 15) & ~(size_t)15;
-      cand.out_pitch = (std::max(g.out_row_bytes, wp * (size_t)g.out_px_bytes) + 15) & ~(size_t)15;
-      if (eligible(cand)) lay = cand;
-    }
+  auto eligible = [&](const csic::Layout& l) {
+    csic::KPlan probe;
+    if (csic::build_plan(*p, reinterpret_cast<const void*>(uintptr_t(4096)), reinterpret_cast<void*>(uintptr_t(4096)), 1, 0,
+                         g.out_h, compact, l, probe) != CSIC_OK)
+      return false;
+    const int family = csic::select_kernel(probe, ctx->dev, ctx->opt).family;
+    return family == csic::FAM_ROWS || family == csic::FAM_POOL;
+  };
+  csic::Layout lay;
+  if (!eligible(csic::Layout()) && p->out_format != CSIC_OUT_PLANAR) {
+    const size_t wp = ((size_t)g.out_w + 15) & ~(size_t)15;
+    csic::Layout cand;
+    cand.in_pitch = (std::max(g.in_row_bytes, wp * (size_t)p->factor * (size_t)g.in_px_bytes) + 15) & ~(size_t)15;
+    cand.out_pitch = (std::max(g.out_row_bytes, wp * (size_t)g.out_px_bytes) + 15) & ~(size_t)15;
+    if (eligible(cand)) lay = cand;
   }
   const size_t in_pitch = lay.in_pitch ? lay.in_pitch : g.in_row_bytes;
   const size_t out_pitch = lay.out_pitch ? lay.out_pitch : g.out_row_bytes;

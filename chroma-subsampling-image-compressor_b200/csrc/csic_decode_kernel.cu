@@ -28,9 +28,7 @@
 // Algorithmic bytes per output pixel: 1 (Y) + 2 / (hs * vs) (chroma) read, 3 written.
 #include <cuda_runtime.h>
 
-#include <algorithm>
 #include <cstdint>
-#include <cstdlib>
 
 #include "csic_internal.h"
 #include "csic_device_math.cuh"
@@ -39,23 +37,6 @@
 namespace csic {
 
 namespace {
-
-constexpr int kDecConsumers = 256;        // default consumer threads (+ the producer warp)
-constexpr int kDecMaxConsumers = 512;
-constexpr uint32_t kDecDescBytes = 48u;
-
-struct DecPlan {
-  const uint8_t* planar;
-  uint8_t* out;
-  uint64_t frame_bytes, cb_off, cr_off;   // PLANAR frame layout: Y at 0, Cb / Cr planes at these offsets
-  uint64_t lim_lo, lim_hi;                // byte range of the planar buffer (hull fetches are clipped to it)
-  uint32_t Wo, Ho, A;                     // A = Wo * Ho pixels per frame
-  uint32_t cw;                            // bytes per chroma plane row
-  uint32_t hs_sh, vhold, last_c;          // log2 of the horizontal hold; odd lines replay sample last_c of the line above
-  uint32_t tile_px, tiles_per_frame, n_tiles;
-  uint32_t stages, y_slot, c_slot, stage_stride, out_off, out_stride, desc_off, bar_off;
-  uint32_t to_rgb;
-};
 
 // Written by the producer before it arms the stage, read by the consumers after the phase flips.
 struct DecDesc {
@@ -351,88 +332,22 @@ cudaError_t attr_hv(int bytes) {
   return cudaFuncSetAttribute(csic_decode_kernel<HS, VHOLD, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
 }
 
-uint32_t env_u32(const char* name, uint32_t dflt) {
-  const char* e = std::getenv(name);
-  if (!e || !*e) return dflt;
-  const long v = std::strtol(e, nullptr, 10);
-  return v > 0 ? (uint32_t)v : dflt;
-}
-
 }  // namespace
 
-// Returns a cudaError_t as int, or -1 when the configuration is outside this kernel (the LDG decoder runs instead):
-// rows narrower than a granule, 2^30 or more pixels per frame, 2^32 or more tiles per launch, or chroma rows so wide
-// that a stage does not fit.
-int launch_decode_tma(const KPlan& k, const uint8_t* planar, uint8_t* out, int to_rgb, int sm_count, size_t max_smem_optin, void* stream) {
-  if (k.Wo < 4 || k.Ho < 1) return -1;
-  const uint64_t A = (uint64_t)k.Wo * (uint64_t)k.Ho;
-  if (A >= (1ull << 30)) return -1;
-  if (std::getenv("CSIC_DEC_NO_TMA")) return -1;
-  DecPlan P{};
-  P.planar = planar; P.out = out;
-  P.frame_bytes = k.out_frame_bytes; P.cb_off = k.planar_cb_off; P.cr_off = k.planar_cr_off;
-  P.lim_lo = reinterpret_cast<uintptr_t>(planar);
-  P.lim_hi = P.lim_lo + (uint64_t)k.n_frames * k.out_frame_bytes;
-  P.Wo = (uint32_t)k.Wo; P.Ho = (uint32_t)k.Ho; P.A = (uint32_t)A;
-  P.cw = (uint32_t)k.planar_cw;
-  P.hs_sh = k.planar_hs == 4 ? 2u : (k.planar_hs == 2 ? 1u : 0u);
-  P.vhold = k.planar_vs == 2 ? 1u : 0u;                           // planar_vs == 2 <=> vf == 2 at f == 1: odd lines are held
-  P.last_c = (uint32_t)((k.last_sample_col / k.f) / k.planar_hs);
-  P.to_rgb = to_rgb ? 1u : 0u;
-  const uint32_t vs = (uint32_t)k.planar_vs;
-  // B200 sweeps (profiles/r2/decode_sweep.txt): 8192-pixel tiles; a frame of up to 12288 pixels is one tile.  A third
-  // stage pays for the RGB reconstruction and on the 4-pixel paths (1080p 4:2:0 to RGB 0.83 -> 0.90, 333-pixel rows to
-  // YCC 0.86 -> 0.93: the consumers otherwise wait for the next tile's loads) where it still leaves two CTAs per SM
-  // their shared memory; where it does not (full-size chroma planes) two stages of 8192 pixels beat three of 4096, and
-  // the 16-pixel path to YCC888 is fastest with two (0.945 vs 0.92).
-  const bool w16 = (k.Wo & 15) == 0;
-  uint32_t T = env_u32("CSIC_DEC_TILE", A <= 12288u ? (uint32_t)((A + 15u) & ~(uint64_t)15) : 8192u) & ~15u;
-  if (T < 64u) T = 64u;
-  const uint32_t S_env = env_u32("CSIC_DEC_STAGES", 0u);
-  auto layout = [&](uint32_t t, uint32_t S) {
-    P.tile_px = (uint32_t)std::min<uint64_t>(t, (A + 15u) & ~(uint64_t)15);
-    const uint32_t nr = std::min<uint32_t>(P.Ho, (P.tile_px + P.Wo - 2u) / P.Wo + 1u);       // rows a tile can touch
-    const uint32_t ncr = vs == 2u ? nr / 2u + 1u : nr;
-    P.stages = S;
-    P.y_slot = (P.tile_px + 32u + 15u) & ~15u;
-    P.c_slot = (ncr * P.cw + 48u + 15u) & ~15u;
-    P.stage_stride = P.y_slot + 2u * P.c_slot;
-    P.out_off = S * P.stage_stride;
-    P.out_stride = (P.tile_px * 3u + 32u + 15u) & ~15u;
-    P.desc_off = P.out_off + 2u * P.out_stride;
-    P.bar_off = P.desc_off + S * kDecDescBytes;
-    return (size_t)P.bar_off + 2u * S * 8u;
-  };
-  uint32_t S = S_env ? std::min(8u, std::max(2u, S_env)) : ((to_rgb || !w16) ? 3u : 2u);
-  size_t smem = layout(T, S);
-  if (!S_env && S == 3u && smem > max_smem_optin / 2) { S = 2u; smem = layout(T, S); }
-  while (smem > max_smem_optin / 2 && T > 256u) { T = (T / 2u) & ~15u; smem = layout(T, S); }   // keep two CTAs per SM
-  if (smem > max_smem_optin) return -1;
-  P.tiles_per_frame = (uint32_t)((A + P.tile_px - 1u) / P.tile_px);
-  P.tile_px = (uint32_t)((((A + P.tiles_per_frame - 1u) / P.tiles_per_frame) + 15u) & ~(uint64_t)15);   // equal tiles (never larger than planned)
-  P.tiles_per_frame = (uint32_t)((A + P.tile_px - 1u) / P.tile_px);
-  const uint64_t n_tiles = (uint64_t)k.n_frames * P.tiles_per_frame;
-  if (n_tiles >= (1ull << 32)) return -1;
-  P.n_tiles = (uint32_t)n_tiles;
-  // one consumer thread per 16-pixel group / 4-pixel granule of a tile, at most 256 (small frames: fewer idle warps)
-  const uint32_t units = w16 ? P.tile_px >> 4 : P.tile_px >> 2;
-  const uint32_t nc_auto = std::min<uint32_t>((uint32_t)kDecConsumers, (units + 31u) & ~31u);
-  const uint32_t nc = std::min<uint32_t>((uint32_t)kDecMaxConsumers, std::max(64u, env_u32("CSIC_DEC_THREADS", nc_auto) & ~31u));
-  const uint32_t threads = nc + 32u;
-  const uint32_t per_sm = (uint32_t)std::max<size_t>(1, std::min<size_t>({(size_t)8, (size_t)(2048u / threads), (size_t)(228u * 1024u) / (smem + 1024u)}));
-  const unsigned grid = (unsigned)std::min<uint64_t>(n_tiles, (uint64_t)sm_count * per_sm);
+int launch_decode_tma(const DecodeLaunch& d, void* stream) {
+  const DecPlan& P = d.P;
   cudaStream_t st = (cudaStream_t)stream;
   if (P.vhold) {
     switch (P.hs_sh) {
-      case 0: return launch_hv<0, true>(P, grid, threads, smem, st);
-      case 1: return launch_hv<1, true>(P, grid, threads, smem, st);
-      default: return launch_hv<2, true>(P, grid, threads, smem, st);
+      case 0: return launch_hv<0, true>(P, d.grid, d.threads, d.smem, st);
+      case 1: return launch_hv<1, true>(P, d.grid, d.threads, d.smem, st);
+      default: return launch_hv<2, true>(P, d.grid, d.threads, d.smem, st);
     }
   }
   switch (P.hs_sh) {
-    case 0: return launch_hv<0, false>(P, grid, threads, smem, st);
-    case 1: return launch_hv<1, false>(P, grid, threads, smem, st);
-    default: return launch_hv<2, false>(P, grid, threads, smem, st);
+    case 0: return launch_hv<0, false>(P, d.grid, d.threads, d.smem, st);
+    case 1: return launch_hv<1, false>(P, d.grid, d.threads, d.smem, st);
+    default: return launch_hv<2, false>(P, d.grid, d.threads, d.smem, st);
   }
 }
 

@@ -24,9 +24,7 @@
 // SpatialDownsampler.scala:17-55, ColorQuantizer.scala:29-44, RGB2YCbCr.scala:123-132, ImageCompressorTop.scala:43-58).
 #include <cuda_runtime.h>
 
-#include <algorithm>
 #include <cstdint>
-#include <cstdlib>
 #include <type_traits>
 
 #include "csic_internal.h"
@@ -37,11 +35,7 @@ namespace csic {
 
 namespace {
 
-constexpr int kFlexConsumers = 256;                  // default: 8 consumer warps (+ 1 producer warp)
-constexpr int kFlexMaxThreads = 288;                 // 8 consumer warps + the producer warp
-constexpr uint32_t kFlexTileBytes = 24u * 1024u;     // input bytes of one tile (B200 sweep: profiles/r1/sweep_flex.txt)
 constexpr uint32_t kCtaWideSpan = 2048u;             // row spans at least this long are stored by the whole CTA
-constexpr uint32_t kDescBytes = 80u;
 constexpr uint32_t kDirectRowBytes = 257u;           // output rows shorter than this that cannot be packed leave from registers (B200 map:
                                                      // 75-250-byte rows 1.3x faster direct, 375-1000-byte rows up to 2x faster staged)
 
@@ -128,7 +122,7 @@ struct FlexDesc {
   uint32_t row_out, out_one, ncols, direct; // output bytes per row, "whole dense rows: one packed span", slots (pad slots incl.),
                                            // "narrow rows: granules go straight to global memory" (direct_store)
 };
-static_assert(sizeof(FlexDesc) == kDescBytes, "kDescBytes out of sync");
+static_assert(sizeof(FlexDesc) == kFlexDescBytes, "kFlexDescBytes out of sync");
 
 }  // namespace
 
@@ -162,7 +156,7 @@ __device__ __forceinline__ void flex_consume(const KPlan& P, uint8_t* smem, uint
   uint32_t s = 0, ph = 0;
   for (uint32_t it = 0; it < n_my; ++it) {
     mbar_wait(full0 + s * 8u, ph);
-    const uint32_t da = desc0 + s * kDescBytes;
+    const uint32_t da = desc0 + s * kFlexDescBytes;
     const uint4 d0 = lds128(da), d1 = lds128(da + 16u), d2 = lds128(da + 32u), d3 = lds128(da + 48u);
     const uint4 d4 = lds128(da + 64u);   // row_out, out_one, ncols, direct
     const uint32_t Dk = d0.x, Dro0 = d0.y, Dnrows = d0.z, Dcol0 = d0.w, Dnpx = d1.x, Da0 = d1.y;
@@ -508,139 +502,7 @@ __global__ void __launch_bounds__(kFlexMaxThreads, 4) csic_flex_kernel(const __g
   else run(std::integral_constant<uint32_t, 4u>{});
 }
 
-// ---- planning and dispatch ---------------------------------------------------------------------------------
-bool plan_flex_kernel(KPlan& k, int sm_count, size_t max_smem_optin, int force_stages, uint32_t force_tile_bytes) {
-  if (k.average && k.f > 1) return false;                       // AVERAGE extension: csic_pool_kernel / generic
-  if (k.band_rows <= 0 || k.n_frames == 0) return false;
-  const uint32_t ipb = (uint32_t)k.in_px_bytes, f = (uint32_t)k.f, pxb = f * ipb;
-  if (k.case_b) {
-    // spatial before chroma: a counter line must be exactly f output rows, each starting on a sample column
-    if (k.W % k.f != 0 || k.Wo % k.hf != 0) return false;
-    k.caseb_row_add = (uint32_t)k.last_sample_col / (uint32_t)k.Wo;
-    k.caseb_col_bytes = ((uint32_t)k.last_sample_col % (uint32_t)k.Wo) * pxb;
-    k.hfe = k.hf;
-  } else {
-    k.hfe = std::max(1, k.hf / k.f);
-  }
-  const bool planar = k.kformat == KF_PLANAR;
-  const uint32_t unit = (k.kformat <= KF_RGB888) ? 12u : (planar ? 4u : 4u * (uint32_t)k.slot_bytes);
-  const uint32_t S = (uint32_t)k.slots_per_row, Wo = (uint32_t)k.Wo;
-  const uint32_t tile_bytes = force_tile_bytes ? std::max(1024u, force_tile_bytes) : kFlexTileBytes;
-  const uint32_t tile_px_max = std::max(16u, (tile_bytes / pxb) & ~15u);
-  k.tile_px = (int32_t)std::min(tile_px_max, (S + 15u) & ~15u);
-  k.nsplit = (int32_t)((S + (uint32_t)k.tile_px - 1u) / (uint32_t)k.tile_px);
-  const uint32_t len_in_max = ((std::min((uint32_t)k.tile_px, Wo) - 1u) * f + 1u) * ipb;
-  // consecutive processed rows contiguous in memory?  (dense rows, every stored row is read)
-  const bool contiguous = k.nsplit == 1 && k.row_step == 1 && k.in_row_bytes == (uint32_t)k.W * ipb;
-  if (k.block_threads <= 0) k.block_threads = kFlexConsumers;
-  k.block_threads = std::min(k.block_threads, kFlexMaxThreads - 32);
-  const uint32_t stages = (uint32_t)std::min(std::max(force_stages, 2), 8);
-  auto up16 = [](uint32_t v) { return (v + 15u) & ~15u; };
-  auto up128 = [](uint32_t v) { return (v + 127u) & ~127u; };
-
-  // "Tall image": when every launch row is a whole frame row and frames lie back to back with the same row stride
-  // inside and across frames (input AND output), the batch IS one image of n_frames * Ho rows -- a tile may then span
-  // frames, which is what batches of small frames need (a 96x96 frame at f = 8 is twelve 288-byte rows: one tile per
-  // frame left the SMs waiting on 3 KB copies).  Only the held-line rule still looks at the row index inside its frame.
-  const uint64_t stored_rows = (uint64_t)(uint32_t)k.Ho * (uint32_t)k.row_step;   // input rows from one frame's first row to the next frame's
-  static const bool no_tall = std::getenv("CSIC_FLEX_NO_TALL") != nullptr;      // experiment switches (tools/): never change results
-  static const int env_rows = std::getenv("CSIC_FLEX_ROWS") ? std::atoi(std::getenv("CSIC_FLEX_ROWS")) : 0;
-  const bool tall = !no_tall && k.nsplit == 1 && !planar && k.n_frames > 1 && k.row0 == 0 && k.band_rows == k.Ho &&
-                    k.in_frame_bytes == stored_rows * k.in_row_bytes && k.out_frame_bytes == (uint64_t)(uint32_t)k.Ho * k.out_row_bytes &&
-                    (uint64_t)k.n_frames * (uint32_t)k.Ho < (1ull << 30) && (uint64_t)k.n_frames * (uint32_t)k.H < (1ull << 31);
-  const uint32_t frames = tall ? 1u : k.n_frames;
-  const uint32_t band_rows = tall ? k.n_frames * (uint32_t)k.Ho : (uint32_t)k.band_rows;
-
-  // Rows per tile (whole rows only).  What the B200 sweeps after the round-2 restructure show (profiles/r2/sweep_flex*.txt,
-  // flex_rows_*.txt): throughput follows (a) the consumer warps that have work, summed over the resident CTAs -- it
-  // saturates near 20 for the light formats and keeps growing to 32 for the fused RGB reconstruction, which is
-  // issue-bound -- and (b) the granules per tile, over which ~110 warp-instructions of per-tile work and two CTA
-  // barriers are spread; two resident CTAs instead of three or four cost another ~15 %.  The candidate that maximises
-  // that product wins: 1366x768 f = 1 RGB888 -> 4 rows, 1080x1920 -> 7, 1918x1078 -> 4, 3838x2158 f = 2 -> 2.
-  const uint32_t NW = (uint32_t)k.block_threads / 32u, gpr = (std::min((uint32_t)k.tile_px, S) + 3u) / 4u;
-  const uint32_t row_in = up16((contiguous ? std::max(len_in_max, k.in_row_bytes) : len_in_max) + 15u) + 16u;
-  uint32_t row_out = ((uint32_t)k.tile_px / 4u) * unit + 16u;
-  if (planar) row_out += 2u * (uint32_t)k.tile_px;
-  // resident CTAs: shared memory, threads, and the 56 registers per thread __launch_bounds__(288, 4) grants
-  const uint32_t cta_cap = std::min<uint32_t>(std::min<uint32_t>(8u, 2048u / ((uint32_t)k.block_threads + 32u)),
-                                              65536u / (56u * ((uint32_t)k.block_threads + 32u)));
-  auto ctas_for = [&](uint32_t r) {
-    const uint32_t smem = stages * (r * row_in + 32u) + r * row_out + 2048u;
-    return std::min<uint32_t>(cta_cap, 227u * 1024u / (smem + 1024u));
-  };
-  int rows = 1;
-  if (k.nsplit == 1) {
-    const uint32_t rmax = std::min<uint32_t>((uint32_t)kFlexMaxRows, band_rows);
-    auto tiles_for = [&](uint32_t r) { return (uint64_t)frames * (uint64_t)((band_rows + r - 1u) / r); };
-    if (force_tile_bytes) {
-      const uint32_t per_row = contiguous ? k.in_row_bytes : len_in_max;
-      rows = (int)std::min<uint32_t>(rmax, std::max<uint32_t>(1u, tile_bytes / std::max(1u, per_row)));
-    } else {
-      // fraction of a CTA's consumer warps that get granules (flex_consume's modes 0 and 2); rows that deal unevenly
-      // or are narrower than a warp run the flat loop: every thread busy, ~15 % more instructions per granule
-      auto busy_frac = [&](uint32_t r) {
-        const bool lanes_ok = gpr * 5u >= ((gpr + 31u) / 32u) * 32u * 4u;
-        if (r <= NW) {
-          const uint32_t parts = NW / r;
-          const uint32_t lanes = parts * 32u, it = (gpr + lanes - 1u) / lanes;
-          if ((parts & (parts - 1u)) == 0u && gpr * 5u >= it * lanes * 4u) return (double)(r * parts) / NW;
-          return 0.85;
-        }
-        const uint32_t rounds = (r + NW - 1u) / NW;
-        if (lanes_ok && r * 5u >= rounds * NW * 4u) return (double)r / (rounds * NW);
-        return 0.85;
-      };
-      const double busy_cap = k.kformat == KF_RGB888 ? 32.0 : 20.0;
-      double best_score = -1.0;
-      for (uint32_t r = 1; r <= rmax; ++r) {
-        const uint32_t c = ctas_for(r);
-        if (c == 0u) break;
-        if (r > 1u && tiles_for(r) < (uint64_t)sm_count * 8u) break;        // keep every SM supplied with several tiles
-        const double gran = (double)r * gpr;
-        // a short last tile per frame recurs with the frame's period under round-robin tile assignment: weigh by its fill
-        const double fill = (double)band_rows / (double)(((band_rows + r - 1u) / r) * r);
-        const double score = std::min(busy_cap, c * NW * busy_frac(r)) * gran / (gran + 400.0) * (c >= 3u ? 1.0 : 0.85) * fill;
-        if (score >= best_score * 1.0001) { best_score = score; rows = (int)r; }
-      }
-    }
-    if (env_rows > 0) rows = (int)std::min<uint32_t>((uint32_t)env_rows, rmax);
-  }
-  k.tile_rows = rows;
-  k.in_dense = (contiguous && rows > 1) ? 1 : 0;
-  const uint64_t tiles_per_band = ((uint64_t)band_rows + (uint32_t)rows - 1u) / (uint32_t)rows;
-  const uint64_t n_tiles = (uint64_t)frames * tiles_per_band * (uint64_t)k.nsplit;
-  if (n_tiles >= (1ull << 31)) return false;
-  const uint32_t dense_out_row = planar ? Wo : S * (unit / 4u);
-  k.out_dense = k.out_row_bytes == dense_out_row ? 1 : 0;
-
-  k.stage_stride = row_in;
-  const uint32_t in_bytes = stages * ((uint32_t)rows * k.stage_stride + 32u);   // + slack: pixel loads read one word ahead
-  uint32_t stage_bytes = (uint32_t)rows * (((uint32_t)k.tile_px / 4u) * unit + 16u) + 16u;   // rows at their own offset mod 16
-  if (planar) stage_bytes += 2u * (uint32_t)(rows / std::max(1, k.planar_vs) + 1) * (uint32_t)k.tile_px;
-  k.out_buf_off = up128(in_bytes);
-  k.out_buf_stride = up16(stage_bytes + 32u);                               // + slack: span_store reads one word ahead
-  k.meta_off = k.out_buf_off + k.out_buf_stride;                            // held words of every stage
-  k.bar_off = up128(k.meta_off + stages * (uint32_t)kFlexMaxRows * 4u);     // full[S], empty[S] mbarriers, then S descriptors
-  k.smem_bytes = k.bar_off + stages * (16u + kDescBytes);
-  if (k.smem_bytes > max_smem_optin) return false;
-  // nothing can fail from here on: commit the tall-image view of the batch
-  k.tiles_per_band = (uint32_t)tiles_per_band;
-  k.n_tiles = (uint32_t)n_tiles;
-  k.tall_ho = 0;
-  if (tall) {
-    k.tall_ho = k.Ho;
-    k.in_frame_bytes *= k.n_frames; k.out_frame_bytes *= k.n_frames;
-    k.H *= (int32_t)k.n_frames; k.Ho = (int32_t)band_rows; k.band_rows = (int32_t)band_rows;
-    k.n_frames = 1;
-  }
-  k.stages = (int32_t)stages;
-  // the grid is a whole number of RESIDENT CTAs per SM: a CTA that has to wait for a slot would run its share of the
-  // tiles after everybody else (round 1 ignored the register limit here: small tiles launched 5-7 CTAs per SM where 4
-  // fit, and the second wave doubled the run time -- 1080x1920 with 4-row tiles: 0.69 instead of 0.9)
-  k.ctas_per_sm = (int32_t)std::max<uint32_t>(1u, std::min<uint32_t>(cta_cap, 227u * 1024u / (k.smem_bytes + 1024u)));
-  return true;
-}
-
+// ---- dispatch ------------------------------------------------------------------------------------------------
 namespace {
 template <int FMT>
 int launch_flex_fmt(const KPlan& k, unsigned grid, cudaStream_t st) {
@@ -657,9 +519,7 @@ cudaError_t flex_attr(size_t b) {
 }
 }  // namespace
 
-int launch_flex(const KPlan& k, int sm_count, int force_ctas_per_sm, void* stream) {
-  const int per_sm = force_ctas_per_sm > 0 ? force_ctas_per_sm : std::max(1, k.ctas_per_sm);
-  const unsigned grid = (unsigned)std::min<uint64_t>((uint64_t)k.n_tiles, (uint64_t)sm_count * (uint64_t)per_sm);
+int launch_flex(const KPlan& k, unsigned grid, void* stream) {
   cudaStream_t st = (cudaStream_t)stream;
   switch (k.kformat) {
     case KF_YCC888: return launch_flex_fmt<KF_YCC888>(k, grid, st);

@@ -1,4 +1,4 @@
-// Internal declarations shared by the host half (csic_params.cpp, csic_api.cu) and the kernels.
+// Internal declarations shared by the host half (csic_params.cpp, csic_plan.cpp, csic_api.cu) and the kernels.
 #ifndef CSIC_INTERNAL_H_
 #define CSIC_INTERNAL_H_
 
@@ -67,41 +67,84 @@ struct KPlan {
   int32_t tall_ho;                       // flex kernel: != 0 -> the batch is addressed as ONE image of n * Ho rows; rows per original frame
 };
 
-// Fills the TMA-row-kernel fields of `k`; returns false when the configuration is not eligible
-// (then the generic kernel runs).  `sm_count`/`max_smem` come from the device.
-bool plan_rows_kernel(KPlan& k, int sm_count, size_t max_smem_optin, int force_stages, uint32_t force_tile_bytes);
-
-// Both return a cudaError_t as int.
-int launch_generic(const KPlan& k, int sm_count, void* stream);
-int launch_expand_planar(const KPlan& k, const uint8_t* planar, uint8_t* out, int to_rgb, int sm_count, size_t max_smem_optin, void* stream);
-// TMA-staged decoder for any width / alignment (csic_decode_kernel.cu); -1 = not eligible, else a cudaError_t
-int launch_decode_tma(const KPlan& k, const uint8_t* planar, uint8_t* out, int to_rgb, int sm_count, size_t max_smem_optin, void* stream);
-int decode_set_attributes(size_t max_smem_optin);
-int launch_rows(const KPlan& k, int sm_count, int force_ctas_per_sm, void* stream);
-constexpr int kDefaultBlockThreads = 256;   // consumer threads; one producer warp is added at launch
+// Constants shared by the planners (csic_plan.cpp) and the kernels.
+constexpr int kDefaultBlockThreads = 256;   // row kernel: consumer threads; one producer warp is added at launch
 constexpr int kMaxConsumerThreads = 512;
-int rows_kernel_set_attributes(size_t max_smem_optin);
-
-// AVERAGE extension: TMA-staged pooling kernel (csic_pool_kernel.cu), chroma-first orders only.
-bool plan_pool_kernel(KPlan& k, int sm_count, size_t max_smem_optin);
-int launch_pool(const KPlan& k, int sm_count, int force_ctas_per_sm, void* stream);
-template <int F> int launch_pool_factor(const KPlan& k, unsigned grid, void* stream);
-template <int F> int pool_set_attributes_factor(size_t max_smem_optin);
-
-// Any width / pitch / base alignment (csic_flex_kernel.cu): DECIMATE pipelines the TMA kernels' 16-byte rules exclude.
-bool plan_flex_kernel(KPlan& k, int sm_count, size_t max_smem_optin, int force_stages, uint32_t force_tile_bytes);
-int launch_flex(const KPlan& k, int sm_count, int force_ctas_per_sm, void* stream);
-int flex_set_attributes(size_t max_smem_optin);
-
-// Implemented once per spatial factor in csic_rows_kernel.cu (explicit specialisations for F = 1, 2, 4, 8).
-template <int F> int launch_rows_factor(const KPlan& k, unsigned grid, void* stream);
-template <int F> int rows_set_attributes_factor(size_t max_smem_optin);
 constexpr int kMaxTileRows = 64;        // rows per tile of the row kernel (small frames: 64 rows x 384 B still make a 24 KB tile; 256 rows
                                         // measured worse on 32x32 and 64x64 frames: the producer's per-row work, profiles/r2/rows_tall.txt)
 constexpr uint32_t kTileMetaBytes = 32 + 4 * kMaxTileRows;   // sizeof(TileMeta) in csic_rows_kernel.cu
 constexpr int kPoolMaxRows = 16;        // output rows per tile of the pooling kernel (each carries f input rows)
 constexpr uint32_t kPoolMetaBytes = 32 + 4 * kPoolMaxRows;   // sizeof(PoolMeta) in csic_pool_kernel.cu
 constexpr int kFlexMaxRows = 64;        // rows per tile of the flex kernel: the producer's lanes take two rows each
+constexpr int kFlexConsumers = 256;                  // flex kernel default: 8 consumer warps (+ 1 producer warp)
+constexpr int kFlexMaxThreads = 288;                 // 8 consumer warps + the producer warp
+constexpr uint32_t kFlexTileBytes = 24u * 1024u;     // input bytes of one flex tile (B200 sweep: profiles/r1/sweep_flex.txt)
+constexpr uint32_t kFlexDescBytes = 80u;             // sizeof(FlexDesc) in csic_flex_kernel.cu
+constexpr int kDecConsumers = 256;        // PLANAR decoder: default consumer threads (+ the producer warp)
+constexpr int kDecMaxConsumers = 512;
+constexpr uint32_t kDecDescBytes = 48u;   // sizeof(DecDesc) in csic_decode_kernel.cu
+
+// Parameters of the TMA-staged PLANAR decoder, passed by value (lives in the constant bank).
+struct DecPlan {
+  const uint8_t* planar;
+  uint8_t* out;
+  uint64_t frame_bytes, cb_off, cr_off;   // PLANAR frame layout: Y at 0, Cb / Cr planes at these offsets
+  uint64_t lim_lo, lim_hi;                // byte range of the planar buffer (hull fetches are clipped to it)
+  uint32_t Wo, Ho, A;                     // A = Wo * Ho pixels per frame
+  uint32_t cw;                            // bytes per chroma plane row
+  uint32_t hs_sh, vhold, last_c;          // log2 of the horizontal hold; odd lines replay sample last_c of the line above
+  uint32_t tile_px, tiles_per_frame, n_tiles;
+  uint32_t stages, y_slot, c_slot, stage_stride, out_off, out_stride, desc_off, bar_off;
+  uint32_t to_rgb;
+};
+
+// ---- planning (csic_plan.cpp, host C++ only): every result depends on the arguments alone -------------------------
+// Optional non-dense device layout: row pitches and frame strides in bytes (0 = dense).
+struct Layout {
+  size_t in_pitch = 0, in_frame = 0, out_pitch = 0, out_frame = 0;
+  bool short_frames = false;   // the buffers hold only one row band of each frame (host band path)
+};
+// The kernel-independent part of a plan (geometry, layout, colour and quantiser constants) of output rows
+// [row0, row0 + rows) of n_frames frames; returns a CSIC_* code.
+int build_plan(const csic_params& p, const void* d_rgb, void* d_out, size_t n_frames, int32_t row0, int32_t rows,
+               bool compact, const Layout& lay, KPlan& k);
+
+struct DeviceLimits { int sm_count; size_t max_smem_optin; };
+// csic_set_option's planner knobs; 0 = the planner's choice.  family: 0 automatic, 1 generic kernel only, 2 no TMA
+// row / pooling kernel (CSIC_OPT_KERNEL_FAMILY).
+struct PlanOptions { int family = 0, stages = 0; uint32_t tile_bytes = 0; int block_threads = 0, ctas_per_sm = 0; };
+enum Family : int32_t { FAM_GENERIC = 1, FAM_ROWS = 2, FAM_POOL = 3, FAM_FLEX = 4 };   // as csic_last_kernel reports them
+struct KernelChoice { int32_t family; KPlan k; unsigned grid; };   // grid = CTAs to launch, 0: nothing to do
+// The first family whose planner takes `base`: TMA row kernel, pooling kernel, flex kernel, else the generic kernel, as
+// opt.family allows.  Every candidate plans on its own copy of `base`.
+KernelChoice select_kernel(const KPlan& base, const DeviceLimits& dev, const PlanOptions& opt);
+
+struct DecodeLaunch { DecPlan P; unsigned grid, threads; size_t smem; };
+// The TMA-staged decoder of the PLANAR batch k.in -> k.out (tile_px: pixels per tile, 0 = the planner's choice).  False
+// when the batch is outside that kernel (the LDG decoder runs instead): rows narrower than a granule, 2^30 or more
+// pixels per frame, 2^32 or more tiles per launch, or chroma rows so wide that a stage does not fit.
+bool plan_decode(const KPlan& k, int to_rgb, const DeviceLimits& dev, uint32_t tile_px, DecodeLaunch& d);
+
+// ---- launch shims and attribute setters (kernel files); each returns a cudaError_t as int ---------------------------
+int launch_generic(const KPlan& k, unsigned grid, void* stream);
+int launch_expand_planar(const KPlan& k, int to_rgb, int sm_count, void* stream);   // LDG decoder of k.in -> k.out
+int launch_decode_tma(const DecodeLaunch& d, void* stream);
+int decode_set_attributes(size_t max_smem_optin);
+int launch_rows(const KPlan& k, unsigned grid, void* stream);
+int rows_kernel_set_attributes(size_t max_smem_optin);
+
+// AVERAGE extension: TMA-staged pooling kernel (csic_pool_kernel.cu), chroma-first orders only.
+int launch_pool(const KPlan& k, unsigned grid, void* stream);
+template <int F> int launch_pool_factor(const KPlan& k, unsigned grid, void* stream);
+template <int F> int pool_set_attributes_factor(size_t max_smem_optin);
+
+// Any width / pitch / base alignment (csic_flex_kernel.cu): DECIMATE pipelines the TMA kernels' 16-byte rules exclude.
+int launch_flex(const KPlan& k, unsigned grid, void* stream);
+int flex_set_attributes(size_t max_smem_optin);
+
+// Implemented once per spatial factor in csic_rows_kernel.cu (explicit specialisations for F = 1, 2, 4, 8).
+template <int F> int launch_rows_factor(const KPlan& k, unsigned grid, void* stream);
+template <int F> int rows_set_attributes_factor(size_t max_smem_optin);
 
 }  // namespace csic
 

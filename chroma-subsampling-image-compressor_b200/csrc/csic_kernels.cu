@@ -1,9 +1,9 @@
-// Planning and dispatch of the pixel pipeline's kernels, written for sm_100a (B200), and the two kernels that are not
-// TMA-staged.  The staged kernels live in their own files:
+// Dispatch of the pixel pipeline's kernels, written for sm_100a (B200), and the two kernels that are not TMA-staged.
+// Every kernel is planned in csic_plan.cpp.  The staged kernels live in their own files:
 //   csic_rows_kernel.cu    the hot path: packed RGB24 row segments through a shared-memory ring filled by the TMA engine
 //                          (cp.async.bulk + mbarrier complete_tx), dp4a colour matrix, chroma hold inside the granule (or
-//                          from one held pixel per row), quantise, pack, TMA bulk store.  Planned here (plan_rows_kernel).
-//   csic_pool_kernel.cu    the AVERAGE extension, same machinery (plan_pool_kernel).
+//                          from one held pixel per row), quantise, pack, TMA bulk store.
+//   csic_pool_kernel.cu    the AVERAGE extension, same machinery.
 //   csic_flex_kernel.cu    DECIMATE for any width / pitch / alignment (hull fetch, staged span stores).
 //   csic_decode_kernel.cu  the PLANAR decoder as flat tiles, any width.
 // In this file:
@@ -22,7 +22,6 @@
 
 #include <algorithm>
 #include <cstdint>
-#include <cstdlib>
 
 #include "csic_internal.h"
 #include "csic_device_math.cuh"
@@ -420,18 +419,14 @@ __global__ void __launch_bounds__(128) csic_expand_planar_any_kernel(const __gri
   }
 }
 
-int launch_expand_planar(const KPlan& k, const uint8_t* planar, uint8_t* out, int to_rgb, int sm_count, size_t max_smem_optin, void* stream) {
+int launch_expand_planar(const KPlan& k, int to_rgb, int sm_count, void* stream) {
   const uint64_t total = (uint64_t)k.n_frames * (uint64_t)k.Ho * (uint64_t)k.Wo;
   if (total == 0) return (int)cudaSuccess;
-  // the TMA-staged decoder (csic_decode_kernel.cu) takes every realistic shape; what it declines -- rows narrower than a
-  // granule, chroma rows too wide for a stage -- runs on the LDG kernel above
-  const int tma = launch_decode_tma(k, planar, out, to_rgb, sm_count, max_smem_optin, stream);
-  if (tma >= 0) return tma;
   const uint64_t n_rows = (uint64_t)k.n_frames * (uint64_t)k.Ho;
   if (n_rows >= (1ull << 32)) return (int)cudaErrorInvalidValue;
   const unsigned threads = (unsigned)std::min<uint32_t>(128u, ((((uint32_t)k.Wo + 3u) >> 2) + 31u) & ~31u);
   const unsigned blocks = (unsigned)std::min<uint64_t>(n_rows, (uint64_t)sm_count * (2048u / threads));
-  csic_expand_planar_any_kernel<<<blocks, threads, 0, (cudaStream_t)stream>>>(k, planar, out, to_rgb);
+  csic_expand_planar_any_kernel<<<blocks, threads, 0, (cudaStream_t)stream>>>(k, k.in, k.out, to_rgb);
   return (int)cudaGetLastError();
 }
 
@@ -451,15 +446,10 @@ int launch_generic_fmt(const KPlan& k, unsigned blocks, unsigned threads, cudaSt
 }
 }  // namespace
 
-int launch_generic(const KPlan& k, int sm_count, void* stream) {
-  const uint64_t n_rows = (uint64_t)k.n_frames * (uint64_t)k.band_rows;
-  if (n_rows == 0 || k.slots_per_row == 0) return (int)cudaSuccess;
-  if (n_rows >= (1ull << 32)) return (int)cudaErrorInvalidValue;
-  // one warp per row, or per 32 / gpr rows when a row has fewer than 32 granules; four warps per CTA
-  const uint32_t gpr = ((uint32_t)k.slots_per_row + 3u) >> 2;
-  const uint64_t groups = gpr < 32u ? (n_rows + 32u / gpr - 1u) / (32u / gpr) : n_rows;
-  const unsigned threads = 128u;
-  const unsigned blocks = (unsigned)std::min<uint64_t>((groups + 3u) / 4u, (uint64_t)sm_count * 16u);
+int launch_generic(const KPlan& k, unsigned blocks, void* stream) {
+  if (blocks == 0) return (int)cudaSuccess;
+  if ((uint64_t)k.n_frames * (uint64_t)k.band_rows >= (1ull << 32)) return (int)cudaErrorInvalidValue;
+  const unsigned threads = 128u;   // four warps per CTA
   cudaStream_t st = (cudaStream_t)stream;
   switch (k.kformat) {
     case KF_YCC888: return launch_generic_fmt<KF_YCC888>(k, blocks, threads, st);
@@ -469,152 +459,6 @@ int launch_generic(const KPlan& k, int sm_count, void* stream) {
     case KF_PLANAR: return launch_generic_fmt<KF_PLANAR>(k, blocks, threads, st);
     default: return launch_generic_fmt<KF_SLOT32>(k, blocks, threads, st);
   }
-}
-
-// ================================================================================================
-// TMA-staged row kernel: planning and dispatch (the kernel itself lives in csic_rows_kernel.cu)
-// ================================================================================================
-bool plan_rows_kernel(KPlan& k, int sm_count, size_t max_smem_optin, int force_stages, uint32_t force_tile_bytes) {
-  if (k.average && k.f > 1) return false;                       // AVERAGE extension: csic_pool_kernel / generic
-  if (k.band_rows <= 0 || k.n_frames == 0) return false;
-  const bool auto_threads = k.block_threads <= 0;
-  if (auto_threads) k.block_threads = kDefaultBlockThreads;
-  if (k.block_threads > kMaxConsumerThreads) return false;
-  // The kernel processes Wp = Wo rounded up to 16 output pixels per row; columns >= Wo are read from / written to
-  // the row padding, so both pitches must cover Wp (dense buffers qualify when Wo % 16 == 0).
-  k.Wp = (k.Wo + 15) & ~15;
-  const bool planar = k.kformat == KF_PLANAR;
-  const uint32_t opx0 = planar ? 1u : (k.kformat <= KF_RGB888 ? 3u : (uint32_t)k.slot_bytes);
-  const uint64_t need_in = (uint64_t)k.Wp * (uint32_t)k.f * (uint32_t)k.in_px_bytes, need_out = (uint64_t)k.Wp * opx0;
-  if (k.in_row_bytes < need_in || k.out_row_bytes < need_out) return false;
-  if ((k.in_row_bytes | k.out_row_bytes) & 15u) return false;    // 16-byte TMA granularity of every row start
-  if ((reinterpret_cast<uintptr_t>(k.in) | reinterpret_cast<uintptr_t>(k.out)) & 15u) return false;
-  if ((k.in_frame_bytes | k.out_frame_bytes) & 15u) return false;
-  if (k.case_b) {
-    // spatial before chroma: a counter line must be exactly f output rows, each starting on a sample column
-    if (k.W % k.f != 0 || k.Wo % 4 != 0) return false;
-    k.caseb_row_add = (uint32_t)k.last_sample_col / (uint32_t)k.Wo;
-    k.caseb_col_bytes = ((uint32_t)k.last_sample_col % (uint32_t)k.Wo) * (uint32_t)k.in_px_bytes * (uint32_t)k.f;
-  }
-  k.ragged = k.Wp != k.Wo;
-  k.in_dense = k.in_row_bytes == need_in;
-  k.out_dense = k.out_row_bytes == need_out;
-  // PLANAR: three dense planes; chroma rows (Wo / hs bytes) must be 16-byte multiples too; bands start on a
-  // chroma row
-  if (planar && (k.ragged || !k.out_dense || k.Wo % (16 * k.planar_hs) != 0 || k.row0 % k.planar_vs != 0)) return false;
-
-  // hold width inside a granule, in output pixels
-  if (!k.case_b) k.hfe = std::max(1, k.hf / k.f);
-  else k.hfe = k.hf;
-
-  // 32-bit bundle slots at f == 1 leave through shared memory + TMA bulk stores like the 3-byte formats: there the
-  // output is larger than the input (4 B per 3 B pixel) and per-warp 512-byte st.global bursts held the kernel at 0.90
-  // of the copy peak (ncu: warps waiting on the store path, DRAM 70 % busy) -- 0.98 staged.  Narrower slots and f >= 2
-  // keep the direct stores (16-bit slots at f == 1: 0.94 direct, 0.83 staged; cfg4: 1.03).  Must match kStaged in
-  // csic_rows_kernel.cu.
-  const bool staged = k.kformat <= KF_RGB888 || planar || (k.f == 1 && k.kformat == KF_SLOT32);
-  const uint32_t opx = planar ? 1u : (k.kformat <= KF_RGB888 ? 3u : (uint32_t)k.slot_bytes);
-  // Tile budget: input bytes of one tile.  Staged formats also hold two output buffers per CTA.
-  const uint32_t tile_budget = force_tile_bytes ? force_tile_bytes : 24u * 1024u;
-  const uint32_t ipb = (uint32_t)k.in_px_bytes;
-  const uint32_t row_in = (uint32_t)k.Wp * ipb * (uint32_t)k.f;  // bytes of one processed input row
-  int nsplit = 0;
-  const uint32_t tile_max = tile_budget + tile_budget / 3;        // a tile may overshoot the budget by a third
-  for (int n = (int)((row_in + tile_max - 1) / tile_max); n <= 64; ++n) {
-    if (n >= 1 && k.Wp % (16 * (planar ? k.planar_hs : 1) * n) == 0) { nsplit = n; break; }
-  }
-  if (nsplit == 0) return false;
-  k.nsplit = nsplit;
-  k.tile_px = k.Wp / nsplit;
-  k.tile_in_bytes = (uint32_t)k.tile_px * ipb * (uint32_t)k.f;    // one row segment
-  k.tile_out_bytes = (uint32_t)k.tile_px * opx;
-  // "Tall image" (as in the flex kernel): when every launch row is a whole frame row and frames lie back to back with the
-  // same row stride inside and across frames, on the input AND the output side, the batch IS one image of n_frames * Ho
-  // rows, and a tile may span frames -- 32x32 frames make 64-row tiles of two frames instead of one 3 KB tile per frame
-  // (0.74 -> 0.95 of the copy peak).  The kernel does not change: the only rule that looks at a row index, "odd lines
-  // replay the line above" (f == 1, 4:2:0 / 4:1:0), reads the same parity when frames have an even number of rows.
-  const uint64_t stored_rows = (uint64_t)(uint32_t)k.Ho * (uint32_t)k.row_step;   // input rows from one frame's first row to the next frame's
-  static const bool no_tall = std::getenv("CSIC_ROWS_NO_TALL") != nullptr;        // experiment switch (tools/): never changes results
-  const bool tall = !no_tall && nsplit == 1 && !planar && !k.case_b && k.n_frames > 1 && k.row0 == 0 && k.band_rows == k.Ho &&
-                    k.in_frame_bytes == stored_rows * k.in_row_bytes && k.out_frame_bytes == (uint64_t)(uint32_t)k.Ho * k.out_row_bytes &&
-                    !(k.vf == 2 && k.f == 1 && (k.Ho & 1)) &&
-                    (uint64_t)k.n_frames * (uint32_t)k.Ho < (1ull << 30) && (uint64_t)k.n_frames * (uint32_t)k.H < (1ull << 31);
-  const uint32_t frames = tall ? 1u : k.n_frames;
-  const int band_rows = tall ? (int)(k.n_frames * (uint32_t)k.Ho) : k.band_rows;
-  // Rows per tile: whole rows only (so the tile's output is contiguous), as many as fit the budget,
-  // but keep at least ~4 tiles per SM so small batches still spread over the chip.
-  int rows = 1;
-  if (nsplit == 1) {
-    rows = (int)std::min<uint32_t>((uint32_t)kMaxTileRows, std::max<uint32_t>(1u, tile_budget / k.tile_in_bytes));
-    // e.g. 15 KB RGBA 4K rows: one row leaves the ring too shallow, two rows (30 KB) are within the slack
-    if ((uint32_t)rows * k.tile_in_bytes < tile_budget * 7u / 10u && (uint32_t)(rows + 1) * k.tile_in_bytes <= tile_max &&
-        rows < kMaxTileRows)
-      ++rows;
-    rows = std::min(rows, band_rows);
-    auto tiles_for = [&](int r) { return (uint64_t)frames * (uint64_t)((band_rows + r - 1) / r); };
-    while (rows > 1 && tiles_for(rows) < (uint64_t)sm_count * 4u) rows = (rows + 1) / 2;
-    // staged 32-bit slots: a tile's two output buffers are larger than its input stages; keep two CTAs resident
-    // (4096-pixel rows: two rows per tile left room for one CTA only -- 0.81 of the copy peak instead of 0.98)
-    if (staged && !planar && k.kformat > KF_RGB888)
-      while (rows > 1 && 2u * ((uint32_t)rows * (k.tile_in_bytes + 32u)) + 2u * ((uint32_t)rows * k.tile_out_bytes) + 2048u > 227u * 1024u / 2u - 1024u)
-        --rows;
-    // Equal tiles: CTAs take tiles round robin, so a short last tile per frame recurs with the period of the frame
-    // (96 rows as 64 + 32: every other CTA got the 32-row tiles only and the kernel ran at 0.71 of the copy peak
-    // where 64x64 and 128x128 frames reach 0.98 - 1.01).  Even row counts keep a held line and its sample in one tile.
-    if (rows > 1) {
-      const int t = (band_rows + rows - 1) / rows;
-      int bal = (band_rows + t - 1) / t;
-      if ((k.vf == 2 || planar) && (bal & 1) && bal < rows) ++bal;
-      rows = std::min(rows, bal);
-    }
-    if (planar && rows > 1) rows &= ~(k.planar_vs - 1);          // tiles start on a chroma row
-    if (rows < 1) rows = 1;
-  }
-  k.tile_rows = rows;
-  k.tiles_per_band = (uint32_t)((band_rows + rows - 1) / rows);
-  const uint64_t n_tiles = (uint64_t)frames * (uint64_t)k.tiles_per_band * (uint64_t)nsplit;
-  if (n_tiles >= (1ull << 31)) return false;
-  k.n_tiles = (uint32_t)n_tiles;
-  // Tiny tiles (whole frames of a few KB: a tile never spans two frames): a granule per thread is all there is, so the
-  // per-tile costs dominate -- half-size CTAs, as many as fit (32x32 frames: 0.74 of the copy peak vs 0.51;
-  // profiles/r1/sweep_rows_v8.txt)
-  const bool tiny = (uint32_t)rows * ((uint32_t)k.tile_px >> 2) <= 512u && n_tiles > (uint64_t)sm_count * 8u;
-  if (tiny && auto_threads) k.block_threads = 128;
-
-  auto up128 = [](uint32_t v) { return (v + 127u) & ~127u; };
-  k.stage_stride = up128((uint32_t)rows * (k.tile_in_bytes + 32u));
-  k.out_buf_stride = staged ? up128((uint32_t)rows * k.tile_out_bytes) : 0u;
-  if (planar)   // [Y rows][Cb rows][Cr rows]
-    k.out_buf_stride = up128((uint32_t)rows * (uint32_t)k.tile_px +
-                             2u * (uint32_t)((rows + k.planar_vs - 1) / k.planar_vs) * ((uint32_t)k.tile_px / (uint32_t)k.planar_hs));
-  // Ring depth and residency, fitted to B200 sweeps (profiles/r1/exp_ctas_v4.txt): the kernel is fastest with
-  // about four ~24 KB tiles in flight per SM -- 2 resident CTAs x 2 stages (cfg4 0.996 of the measured copy peak
-  // vs 0.953 with 4 CTAs; cfg2 0.97 vs 0.94 with 6 tiles in flight).  Only when a tile carries little compute
-  // per byte (f >= 4: one pixel in 16 is converted) does a third stage pay (cfg5 0.98 vs 0.92).
-  auto need = [&](int s) {
-    return (uint32_t)s * k.stage_stride + 2u * k.out_buf_stride + (uint32_t)s * kTileMetaBytes + (uint32_t)s * 16u + 384u;
-  };
-  auto ctas_for = [&](int s) {
-    const uint32_t by_smem = (uint32_t)(227u * 1024u / (need(s) + 1024u));
-    return std::min<uint32_t>(std::min<uint32_t>(by_smem, 2048u / ((uint32_t)k.block_threads + 32u)), 8u);
-  };
-  int stages = force_stages >= 2 ? force_stages : (k.f >= 4 ? 3 : 2);
-  while (force_stages < 2 && stages > 2 && ctas_for(stages) < 2) --stages;
-  if (need(stages) > max_smem_optin || ctas_for(stages) < 1) return false;
-  // f == 1 converts every byte it loads (issue slots 64 % busy with 16 warps): there more resident warps win
-  // (PLANAR 1080p: 0.97 of the copy peak with 3 CTAs vs 0.84 with 2; 16-bit bundles: 0.93 with 4).
-  k.ctas_per_sm = (int32_t)std::min<uint32_t>(ctas_for(stages), tiny ? 8u : (k.f == 1 ? 4u : 2u));
-  k.stages = stages;
-  if (tall) {                                      // nothing can fail from here on: commit the tall-image view of the batch
-    k.in_frame_bytes *= k.n_frames; k.out_frame_bytes *= k.n_frames;
-    k.H *= (int32_t)k.n_frames; k.Ho = band_rows; k.band_rows = band_rows;
-    k.n_frames = 1;
-  }
-  k.out_buf_off = (uint32_t)stages * k.stage_stride;
-  k.meta_off = up128(k.out_buf_off + 2u * k.out_buf_stride);
-  k.bar_off = up128(k.meta_off + (uint32_t)stages * (uint32_t)kTileMetaBytes);
-  k.smem_bytes = k.bar_off + (uint32_t)stages * 16u;     // full[] and empty[] mbarriers
-  return true;
 }
 
 int rows_kernel_set_attributes(size_t max_smem_optin) {
@@ -631,96 +475,7 @@ int rows_kernel_set_attributes(size_t max_smem_optin) {
   return 0;
 }
 
-// ---- AVERAGE extension: planning and dispatch of csic_pool_kernel --------------------------------
-bool plan_pool_kernel(KPlan& k, int sm_count, size_t max_smem_optin) {
-  if (!(k.average && k.f > 1)) return false;
-  if (k.case_b) {
-    // pooling before chroma: a counter line (W == f * Wo stream elements) must be whole output rows that start on a
-    // sample column; the held block of an odd line is the stream element (line-1) * W + lastSampleCol
-    if (k.W % k.f != 0 || k.Wo % k.hf != 0) return false;
-    k.caseb_row_add = (uint32_t)k.last_sample_col / (uint32_t)k.Wo;
-    k.caseb_col_bytes = ((uint32_t)k.last_sample_col % (uint32_t)k.Wo) * (uint32_t)k.in_px_bytes * (uint32_t)k.f;
-  }
-  // Like the row kernel, the kernel processes Wp = Wo rounded up to 16 output pixels per row: columns >= Wo are read
-  // from / written into the row padding, so both pitches must cover Wp (dense buffers qualify when Wo % 16 == 0;
-  // csic_process_host re-pitches other widths in its staging buffers, csic_process_device_pitched takes them as given).
-  k.Wp = (k.Wo + 15) & ~15;
-  const uint32_t opx_p = k.kformat <= KF_RGB888 ? 3u : (uint32_t)k.slot_bytes;
-  if (k.in_row_bytes % 16 != 0 || (uint64_t)k.in_row_bytes < (uint64_t)k.Wp * (uint32_t)k.f * (uint32_t)k.in_px_bytes) return false;
-  if ((uint64_t)k.out_row_bytes < (uint64_t)k.Wp * opx_p) return false;
-  if ((reinterpret_cast<uintptr_t>(k.in) | reinterpret_cast<uintptr_t>(k.out)) & 15u) return false;
-  if ((k.in_frame_bytes | k.out_frame_bytes | k.out_row_bytes) & 15u) return false;
-  k.ragged = k.Wp != k.Wo;
-  k.in_dense = (uint64_t)k.in_row_bytes == (uint64_t)k.Wp * (uint32_t)k.f * (uint32_t)k.in_px_bytes;    // the f rows of a block row are contiguous
-  k.out_dense = (uint64_t)k.out_row_bytes == (uint64_t)k.Wp * opx_p;                                     // output rows are back to back
-  if (k.band_rows <= 0 || k.n_frames == 0) return false;
-  // 4x4 / 8x8 pooling keeps more live registers per thread: 6 consumer warps leave room for one more CTA per SM
-  // (B200 sweep, profiles/r1/sweep_pool_v8.txt: 8K 4x4 0.97 of the copy peak vs 0.92 with 8 warps)
-  const bool auto_threads = k.block_threads <= 0;
-  if (auto_threads) k.block_threads = k.f >= 4 ? 192 : kDefaultBlockThreads;
-  if (k.block_threads > kMaxConsumerThreads) return false;
-
-  const bool staged = k.kformat <= KF_RGB888;
-  const uint32_t opx = staged ? 3u : (uint32_t)k.slot_bytes;
-  const uint32_t f = (uint32_t)k.f, ipb = (uint32_t)k.in_px_bytes;
-  const uint32_t budget = 24u * 1024u, tile_max = budget + budget / 3;   // (48 KB tiles for 8x8 pooling: 1080p +5 %, 4K / 8K -12 %)
-  const uint32_t block_row_bytes = (uint32_t)k.Wp * f * f * ipb;          // the f input rows of one output row
-  int nsplit = 0;
-  for (int n = (int)((block_row_bytes + tile_max - 1) / tile_max); n <= 256; ++n)
-    if (n >= 1 && k.Wp % (16 * n) == 0) { nsplit = n; break; }
-  if (nsplit == 0) return false;
-  k.nsplit = nsplit;
-  k.tile_px = k.Wp / nsplit;
-  k.tile_in_bytes = (uint32_t)k.tile_px * f * f * ipb;                   // per output-row segment: f row parts
-  k.tile_out_bytes = (uint32_t)k.tile_px * opx;
-  int rows = 1;
-  if (nsplit == 1) {
-    rows = (int)std::max<uint32_t>(1u, budget / k.tile_in_bytes);
-    // e.g. 2560x1440 2x2 or 640x480 8x8: an output row carries 15 KB of input -- one row leaves the ring too shallow, two
-    // rows (30 KB) are within the slack (the row kernel's rule)
-    if ((uint32_t)rows * k.tile_in_bytes < budget * 7u / 10u && (uint32_t)(rows + 1) * k.tile_in_bytes <= tile_max) ++rows;
-    rows = std::min(rows, (int)(2u * (uint32_t)kPoolMaxRows / f));      // held_addr[] holds rows * f/2 entries
-    rows = std::min(rows, k.band_rows);
-    if (!k.out_dense) rows = 1;                                           // a tile's output must be one contiguous range
-    auto tiles_for = [&](int r) { return (uint64_t)k.n_frames * (uint64_t)((k.band_rows + r - 1) / r); };
-    while (rows > 1 && tiles_for(rows) < (uint64_t)sm_count * 4u) rows = (rows + 1) / 2;
-    if (rows > 1) {                                                       // equal tiles (see plan_rows_kernel)
-      const int t = (k.band_rows + rows - 1) / rows;
-      rows = std::min(rows, (k.band_rows + t - 1) / t);
-    }
-  }
-  k.tile_rows = rows;
-  k.tiles_per_band = (uint32_t)((k.band_rows + rows - 1) / rows);
-  const uint64_t n_tiles = (uint64_t)k.n_frames * (uint64_t)k.tiles_per_band * (uint64_t)nsplit;
-  if (n_tiles >= (1ull << 31)) return false;
-  k.n_tiles = (uint32_t)n_tiles;
-  // 8x8 pooling is bound by the integer pipes, and a granule is 256 input pixels: a 15 KB tile has twenty of them, four
-  // threads each -- 80 busy threads of 192 (1080p: 240 output pixels per row, split three ways).  Size the CTA to the
-  // tile and let more of them be resident instead (1080p 8x8: 0.69-0.81 -> 0.78-0.91 of the copy peak).
-  const uint32_t units = (uint32_t)rows * ((uint32_t)k.tile_px >> 2) * 4u;
-  const bool small_cta = auto_threads && k.f == 8 && 2u * units <= (uint32_t)k.block_threads;   // (tiles that fill 2/3 of the CTA or more: 3-4 % slower this way)
-  if (small_cta) k.block_threads = (int32_t)std::max(64u, (units + 31u) & ~31u);
-  auto up128 = [](uint32_t v) { return (v + 127u) & ~127u; };
-  k.stage_stride = up128((uint32_t)rows * k.tile_in_bytes + (uint32_t)kPoolMaxRows * 32u);
-  k.out_buf_stride = staged ? (uint32_t)(kMaxConsumerThreads / 32) * 384u / 2u : 0u;   // 2 x stride = one 384-byte slot per warp
-  k.stages = 2;
-  const uint32_t need = 2u * k.stage_stride + 2u * k.out_buf_stride + 2u * kPoolMetaBytes + 32u + 384u;
-  if (need > max_smem_optin) return false;
-  // pooling converts every input pixel: the kernel is issue-bound, so take all the warps that fit (measured:
-  // 4 CTAs 0.79 of the copy peak on the 4K 2x2 case vs 0.73 with 2)
-  const uint32_t threads = (uint32_t)k.block_threads + 32u;
-  const uint32_t by_regs = 65536u / ((k.f == 2 ? 56u : 72u) * threads);     // __maxnreg__ of csic_pool_kernel
-  k.ctas_per_sm = (int32_t)std::max<uint32_t>(1u, std::min<uint32_t>(std::min<uint32_t>(small_cta ? 8u : 4u, by_regs), 227u * 1024u / (need + 1024u)));
-  k.out_buf_off = 2u * k.stage_stride;
-  k.meta_off = up128(k.out_buf_off + 2u * k.out_buf_stride);
-  k.bar_off = up128(k.meta_off + 2u * kPoolMetaBytes);
-  k.smem_bytes = k.bar_off + 2u * 16u;
-  return true;
-}
-
-int launch_pool(const KPlan& k, int sm_count, int force_ctas_per_sm, void* stream) {
-  const int per_sm = force_ctas_per_sm > 0 ? force_ctas_per_sm : std::max(1, k.ctas_per_sm);
-  const unsigned grid = (unsigned)std::min<uint64_t>((uint64_t)k.n_tiles, (uint64_t)sm_count * (uint64_t)per_sm);
+int launch_pool(const KPlan& k, unsigned grid, void* stream) {
   switch (k.f) {
     case 2: return launch_pool_factor<2>(k, grid, stream);
     case 4: return launch_pool_factor<4>(k, grid, stream);
@@ -728,11 +483,7 @@ int launch_pool(const KPlan& k, int sm_count, int force_ctas_per_sm, void* strea
   }
 }
 
-int launch_rows(const KPlan& k, int sm_count, int force_ctas_per_sm, void* stream) {
-  // Persistent grid: a whole number of CTAs per SM, as many as the shared-memory footprint allows.
-  uint32_t per_sm = (uint32_t)std::max(1, k.ctas_per_sm);
-  if (force_ctas_per_sm > 0) per_sm = (uint32_t)force_ctas_per_sm;   // tuning knob; the hardware caps residency
-  const unsigned grid = (unsigned)std::min<uint64_t>((uint64_t)k.n_tiles, (uint64_t)sm_count * per_sm);
+int launch_rows(const KPlan& k, unsigned grid, void* stream) {
   switch (k.f) {
     case 1: return launch_rows_factor<1>(k, grid, stream);
     case 2: return launch_rows_factor<2>(k, grid, stream);
