@@ -31,7 +31,7 @@ int cuda_fail(cudaError_t e, const char* what) {
     if (e__ != cudaSuccess) return cuda_fail(e__, #call); \
   } while (0)
 
-constexpr int kPipe = 3;   // chunks in flight in csic_process_host
+using csic::kPipe;
 // Input bytes per pipelined chunk.  B200 + PCIe 5 x16, 4K batches (profiles/r2/e2e_chunk_sweep.txt): 16 MB 32.6 k MP/s,
 // 32 MB 32.3 k, 64 MB (round 1) 31.9 k, 128 MB 31.3 k -- the pipeline's fill and drain cost one chunk each per call.
 constexpr size_t kDefaultChunkBytes = 16u << 20;
@@ -61,13 +61,9 @@ struct csic_ctx {
   csic::DeviceLimits dev = {};
   cudaStream_t stream = nullptr;             // default compute stream
   cudaStream_t s_h2d = nullptr, s_d2h = nullptr;
-  void* d_in[kPipe] = {nullptr, nullptr, nullptr};
-  void* d_out[kPipe] = {nullptr, nullptr, nullptr};
-  size_t d_in_cap = 0, d_out_cap = 0;
+  struct Ring { void* buf[kPipe] = {}; size_t cap = 0; } d_in, d_out;   // device staging: kPipe buffers of cap bytes
+  Ring h_in, h_out;                          // pinned bounce buffers for pageable callers
   cudaEvent_t ev_h2d[kPipe] = {}, ev_k[kPipe] = {}, ev_d2h[kPipe] = {};
-  void* h_in[kPipe] = {nullptr, nullptr, nullptr};    // pinned bounce buffers for pageable callers
-  void* h_out[kPipe] = {nullptr, nullptr, nullptr};
-  size_t h_in_cap = 0, h_out_cap = 0;
   int opt_no_bounce = 0;
   int last_family = 0;
   int64_t launches = 0;
@@ -90,12 +86,6 @@ struct DeviceGuard {
     if (prev >= 0) cudaSetDevice(prev);
   }
 };
-
-// True when a DECIMATE pipeline reads only every f-th input row and those rows sit at a uniform pitch
-// across the frames of a batch: then csic_process_host ships just those rows over PCIe.
-bool can_compact(const csic_params& p) {
-  return p.pool_mode == CSIC_POOL_DECIMATE && p.factor > 1 && p.height % p.factor == 0;
-}
 
 int run(csic_ctx* ctx, const csic_params* p, const void* d_rgb, size_t n_frames, void* d_out, int32_t row0,
         int32_t rows, void* cuda_stream, bool compact = false, const csic::Layout& lay = csic::Layout()) {
@@ -124,25 +114,14 @@ int run(csic_ctx* ctx, const csic_params* p, const void* d_rgb, size_t n_frames,
   return CSIC_OK;
 }
 
-int ensure_staging(csic_ctx* ctx, size_t in_bytes, size_t out_bytes) {
-  if (in_bytes > ctx->d_in_cap) {
-    for (int i = 0; i < kPipe; ++i) {
-      if (ctx->d_in[i]) cudaFree(ctx->d_in[i]);
-      ctx->d_in[i] = nullptr;
-    }
-    ctx->d_in_cap = 0;
-    for (int i = 0; i < kPipe; ++i) CSIC_CUDA(cudaMalloc(&ctx->d_in[i], in_bytes));
-    ctx->d_in_cap = in_bytes;
-  }
-  if (out_bytes > ctx->d_out_cap) {
-    for (int i = 0; i < kPipe; ++i) {
-      if (ctx->d_out[i]) cudaFree(ctx->d_out[i]);
-      ctx->d_out[i] = nullptr;
-    }
-    ctx->d_out_cap = 0;
-    for (int i = 0; i < kPipe; ++i) CSIC_CUDA(cudaMalloc(&ctx->d_out[i], out_bytes));
-    ctx->d_out_cap = out_bytes;
-  }
+// Grows one ring of staging buffers (device or pinned: alloc / release) to at least `bytes` each.
+template <typename Alloc, typename Release>
+int grow_ring(csic_ctx::Ring& r, size_t bytes, Alloc alloc, Release release) {
+  if (bytes <= r.cap) return CSIC_OK;
+  for (void*& b : r.buf) { if (b) release(b); b = nullptr; }
+  r.cap = 0;
+  for (void*& b : r.buf) CSIC_CUDA(alloc(&b, bytes));
+  r.cap = bytes;
   return CSIC_OK;
 }
 
@@ -211,10 +190,10 @@ int csic_destroy(csic_ctx* ctx) {
   for (cudaStream_t st : {ctx->stream, ctx->s_h2d, ctx->s_d2h})
     if (st) cudaStreamSynchronize(st);
   for (int i = 0; i < kPipe; ++i) {
-    if (ctx->d_in[i]) cudaFree(ctx->d_in[i]);
-    if (ctx->d_out[i]) cudaFree(ctx->d_out[i]);
-    if (ctx->h_in[i]) cudaFreeHost(ctx->h_in[i]);
-    if (ctx->h_out[i]) cudaFreeHost(ctx->h_out[i]);
+    if (ctx->d_in.buf[i]) cudaFree(ctx->d_in.buf[i]);
+    if (ctx->d_out.buf[i]) cudaFree(ctx->d_out.buf[i]);
+    if (ctx->h_in.buf[i]) cudaFreeHost(ctx->h_in.buf[i]);
+    if (ctx->h_out.buf[i]) cudaFreeHost(ctx->h_out.buf[i]);
     if (ctx->ev_h2d[i]) cudaEventDestroy(ctx->ev_h2d[i]);
     if (ctx->ev_k[i]) cudaEventDestroy(ctx->ev_k[i]);
     if (ctx->ev_d2h[i]) cudaEventDestroy(ctx->ev_d2h[i]);
@@ -279,11 +258,7 @@ int csic_process_device_pitched(csic_ctx* ctx, const csic_params* p, const void*
   int rc = csic_validate(p, nullptr, 0);
   if (rc != CSIC_OK) return rc;
   const csic::Geometry g = csic::geometry(*p);
-  csic::Layout lay;
-  lay.in_pitch = in_pitch_bytes;
-  lay.in_frame = in_frame_stride;
-  lay.out_pitch = out_pitch_bytes;
-  lay.out_frame = out_frame_stride;
+  const csic::Layout lay{in_pitch_bytes, in_frame_stride, out_pitch_bytes, out_frame_stride};
   return run(ctx, p, d_rgb, n_frames, d_out, 0, g.out_h, cuda_stream, false, lay);
 }
 
@@ -322,40 +297,6 @@ int csic_process_band(csic_ctx* ctx, const csic_params* p, const void* d_rgb, si
   return run(ctx, p, d_rgb, n_frames, d_out, out_row0, out_rows, cuda_stream);
 }
 
-// Input rows a band of output rows reads: the rows it decimates / pools from, plus -- when the band
-// starts on a line whose chroma is held from the line above -- the row holding that sample.
-int csic_band_input_rows(const csic_params* p, int32_t out_row0, int32_t out_rows, int32_t* in_row0,
-                         int32_t* in_rows) {
-  int rc = csic_validate(p, nullptr, 0);
-  if (rc != CSIC_OK) return rc;
-  const csic::Geometry g = csic::geometry(*p);
-  if (out_row0 < 0 || out_rows <= 0 || out_row0 + out_rows > g.out_h) return CSIC_EINVAL_ARG;
-  const int f = p->factor;
-  const bool avg = p->pool_mode == CSIC_POOL_AVERAGE && f > 1;
-  int64_t lo = (int64_t)out_row0 * f;
-  int64_t hi = (int64_t)(out_row0 + out_rows - 1) * f + (avg ? f - 1 : 0);   // inclusive
-  const bool case_b = !g.chroma_first && f > 1;
-  if (!case_b) {
-    if (g.vf == 2 && (lo & 1)) lo -= 1;   // only possible for f == 1
-  } else {
-    // chroma runs on the decimated stream with full-size counters: walk the band's first and last
-    // stream elements back to their sources (ImageCompressorTop.scala:52-58).
-    const int64_t W = p->width, Wo = g.out_w;
-    const int64_t last = ((W - 1) / g.hf) * g.hf;
-    auto src_row = [&](int64_t m) {
-      const int64_t col = m % W, line = (m / W) % p->height;
-      const int64_t s = (g.vf == 2 && (line & 1)) ? (line - 1) * W + last : m - col % g.hf;
-      return (s / Wo) * f;
-    };
-    lo = std::min(lo, src_row((int64_t)out_row0 * Wo));
-    lo = std::min(lo, src_row((int64_t)out_row0 * Wo + Wo - 1));
-  }
-  hi = std::min<int64_t>(hi, p->height - 1);
-  if (in_row0) *in_row0 = (int32_t)lo;
-  if (in_rows) *in_rows = (int32_t)(hi - lo + 1);
-  return CSIC_OK;
-}
-
 namespace {
 
 bool is_pageable(const void* p) {
@@ -367,43 +308,20 @@ bool is_pageable(const void* p) {
   return at.type == cudaMemoryTypeUnregistered;
 }
 
-int ensure_bounce(csic_ctx* ctx, size_t in_bytes, size_t out_bytes) {
-  if (in_bytes > ctx->h_in_cap) {
-    for (int i = 0; i < kPipe; ++i) {
-      if (ctx->h_in[i]) cudaFreeHost(ctx->h_in[i]);
-      ctx->h_in[i] = nullptr;
-    }
-    ctx->h_in_cap = 0;
-    for (int i = 0; i < kPipe; ++i) CSIC_CUDA(cudaHostAlloc(&ctx->h_in[i], in_bytes, cudaHostAllocDefault));
-    ctx->h_in_cap = in_bytes;
-  }
-  if (out_bytes > ctx->h_out_cap) {
-    for (int i = 0; i < kPipe; ++i) {
-      if (ctx->h_out[i]) cudaFreeHost(ctx->h_out[i]);
-      ctx->h_out[i] = nullptr;
-    }
-    ctx->h_out_cap = 0;
-    for (int i = 0; i < kPipe; ++i) CSIC_CUDA(cudaHostAlloc(&ctx->h_out[i], out_bytes, cudaHostAllocDefault));
-    ctx->h_out_cap = out_bytes;
-  }
-  return CSIC_OK;
-}
-
-// Copies `n_rows` rows of `row_bytes` from src (row stride src_step) to dst (row stride dst_step) on several
-// host threads: a pageable caller's rows are gathered into / scattered from the pinned bounce buffers at host
-// memory speed instead of the driver's single-threaded staging.
-void parallel_rows_copy(uint8_t* dst, size_t dst_step, const uint8_t* src, size_t src_step, size_t row_bytes, size_t n_rows) {
-  const size_t total = row_bytes * n_rows;
+// One copy of csic::frame_copies between host buffers, on several host threads: a pageable caller's rows are gathered
+// into / scattered from the pinned bounce buffers at host memory speed instead of the driver's single-threaded staging.
+void host_copy(uint8_t* dst, const uint8_t* src, const csic::Copy& c) {
+  const size_t total = c.width * c.height;
   unsigned T = std::min<unsigned>(8u, std::max(1u, std::thread::hardware_concurrency() / 2));
   if (total < (4u << 20)) T = 1;
-  const bool contiguous = dst_step == row_bytes && src_step == row_bytes;
+  const bool contiguous = !c.dst_pitch || (c.dst_pitch == c.width && c.src_pitch == c.width);
   // contiguous ranges are cut by bytes (a "row" may be a whole frame), strided ones by rows
-  const size_t units = contiguous ? total : n_rows;
+  const size_t units = contiguous ? total : c.height;
   auto work = [=](size_t u0, size_t u1) {
     if (contiguous) {
-      std::memcpy(dst + u0, src + u0, u1 - u0);
+      std::memcpy(dst + c.dst + u0, src + c.src + u0, u1 - u0);
     } else {
-      for (size_t r = u0; r < u1; ++r) std::memcpy(dst + r * dst_step, src + r * src_step, row_bytes);
+      for (size_t r = u0; r < u1; ++r) std::memcpy(dst + c.dst + r * c.dst_pitch, src + c.src + r * c.src_pitch, c.width);
     }
   };
   if (T == 1) { work(0, units); return; }
@@ -411,6 +329,15 @@ void parallel_rows_copy(uint8_t* dst, size_t dst_step, const uint8_t* src, size_
   for (unsigned t = 1; t < T; ++t) th.emplace_back(work, units * t / T, units * (t + 1) / T);
   work(0, units / T);
   for (std::thread& x : th) x.join();
+}
+
+// Issues the copies of csic::frame_copies between host and device buffers (or back) on `st`.
+int device_copies(uint8_t* dst, const uint8_t* src, const std::vector<csic::Copy>& cs, cudaMemcpyKind dir,
+                  cudaStream_t st) {
+  for (const csic::Copy& c : cs)
+    CSIC_CUDA(c.dst_pitch ? cudaMemcpy2DAsync(dst + c.dst, c.dst_pitch, src + c.src, c.src_pitch, c.width, c.height, dir, st)
+                          : cudaMemcpyAsync(dst + c.dst, src + c.src, c.width, dir, st));
+  return CSIC_OK;
 }
 
 }  // namespace
@@ -428,58 +355,15 @@ struct ChunkShare {
 
 static int host_pipeline_run(csic_ctx* ctx, const csic_params* p, const uint8_t* rgb, size_t n_frames, uint8_t* out,
                              int32_t row0, int32_t rows, ChunkShare* share) {
-  const csic::Geometry g = csic::geometry(*p);
   DeviceGuard guard(ctx->device);
-  const bool band = !(row0 == 0 && rows == g.out_h);
-
-  // DECIMATE with f > 1 reads only every f-th row: ship only those (a strided 2-D copy), 1/f of the H2D bytes.
-  const bool compact = can_compact(*p) && !ctx->opt_no_compact;
-  int32_t in_row0 = 0, in_rows = p->height;
-  if (band) {
-    int rc = csic_band_input_rows(p, row0, rows, &in_row0, &in_rows);
-    if (rc != CSIC_OK) return rc;
-  }
-  // rows kept on the device, in stored-row units (a stored row is an input row, or every f-th one when compact)
-  const size_t first_stored = compact ? (size_t)(in_row0 / p->factor) : (size_t)in_row0;
-  const size_t rows_stored = compact ? (size_t)(row0 + rows) - first_stored : (size_t)in_rows;
-
-  // Staging layout.  Dense when the dense layout already satisfies a TMA kernel's 16-byte rules; otherwise the
-  // rows are re-pitched on the way in and out (the copies are 2-D anyway), so odd widths also avoid the
-  // generic kernel.
-  auto eligible = [&](const csic::Layout& l) {
-    csic::KPlan probe;
-    if (csic::build_plan(*p, reinterpret_cast<const void*>(uintptr_t(4096)), reinterpret_cast<void*>(uintptr_t(4096)), 1, 0,
-                         g.out_h, compact, l, probe) != CSIC_OK)
-      return false;
-    const int family = csic::select_kernel(probe, ctx->dev, ctx->opt).family;
-    return family == csic::FAM_ROWS || family == csic::FAM_POOL;
-  };
-  csic::Layout lay;
-  if (!eligible(csic::Layout()) && p->out_format != CSIC_OUT_PLANAR) {
-    const size_t wp = ((size_t)g.out_w + 15) & ~(size_t)15;
-    csic::Layout cand;
-    cand.in_pitch = (std::max(g.in_row_bytes, wp * (size_t)p->factor * (size_t)g.in_px_bytes) + 15) & ~(size_t)15;
-    cand.out_pitch = (std::max(g.out_row_bytes, wp * (size_t)g.out_px_bytes) + 15) & ~(size_t)15;
-    if (eligible(cand)) lay = cand;
-  }
-  const size_t in_pitch = lay.in_pitch ? lay.in_pitch : g.in_row_bytes;
-  const size_t out_pitch = lay.out_pitch ? lay.out_pitch : g.out_row_bytes;
-  const size_t dev_frame_bytes = in_pitch * rows_stored;
-  if (band && p->out_format == CSIC_OUT_PLANAR) return CSIC_EINVAL_MODE;   // planes are not row bands
-  const size_t dev_out_frame_bytes = band ? out_pitch * (size_t)rows : std::max(out_pitch * (size_t)rows, g.out_frame_bytes);
-  const size_t host_row_step = g.in_row_bytes * (size_t)(compact ? p->factor : 1);
-  if (band) {   // the device holds only the band's rows: frames are dev_*_frame_bytes apart
-    lay.in_pitch = in_pitch;
-    lay.out_pitch = out_pitch;
-    lay.in_frame = dev_frame_bytes;
-    lay.out_frame = dev_out_frame_bytes;
-    lay.short_frames = true;
-  }
-  // Frames per chunk: ~opt_chunk_bytes of input, at least one frame, at most what is there.
-  size_t per = std::max<size_t>(1, ctx->opt_chunk_bytes / std::max<size_t>(1, dev_frame_bytes));
-  per = std::min(per, n_frames);
-  if (share) per = std::min(per, std::max<size_t>(1, n_frames / (share->gpus * (size_t)kPipe)));   // several chunks per GPU
-  int rc = ensure_staging(ctx, per * dev_frame_bytes, per * dev_out_frame_bytes);
+  csic::HostPlan h;
+  int rc = csic::plan_host(*p, row0, rows, n_frames, ctx->dev, ctx->opt, ctx->opt_chunk_bytes, ctx->opt_no_compact,
+                           share ? share->gpus : 0, h);
+  if (rc != CSIC_OK) return rc;
+  const size_t per = h.frames_per_chunk;
+  auto dev_alloc = [](void** b, size_t n) { return cudaMalloc(b, n); };
+  rc = grow_ring(ctx->d_in, per * h.in.staging.frame, dev_alloc, cudaFree);
+  if (rc == CSIC_OK) rc = grow_ring(ctx->d_out, per * h.out.staging.frame, dev_alloc, cudaFree);
   if (rc != CSIC_OK) return rc;
 
   // The chunks this context processes, in order: consecutive ones when it owns the whole batch, otherwise whatever
@@ -496,29 +380,24 @@ static int host_pipeline_run(csic_ctx* ctx, const csic_params* p, const uint8_t*
   // Pageable caller buffers (a JVM heap, malloc): cudaMemcpyAsync would fall back to the driver's synchronous,
   // single-threaded staging (measured 5 k MP/s vs 31 k MP/s pinned on cfg4).  Gather the needed rows into pinned
   // bounce buffers on several host threads instead, overlapped with the DMA of the neighbouring chunks.
-  const bool bounce = !ctx->opt_no_bounce && n_frames * dev_frame_bytes >= (8u << 20) && (is_pageable(rgb) || is_pageable(out));
-  const size_t bounce_in_frame = g.in_row_bytes * rows_stored, bounce_out_frame = band ? g.out_row_bytes * (size_t)rows : g.out_frame_bytes;
+  const bool bounce =
+      !ctx->opt_no_bounce && n_frames * h.in.staging.frame >= (8u << 20) && (is_pageable(rgb) || is_pageable(out));
   if (bounce) {
-    rc = ensure_bounce(ctx, per * bounce_in_frame, per * bounce_out_frame);
+    auto pinned = [](void** b, size_t n) { return cudaHostAlloc(b, n, cudaHostAllocDefault); };
+    rc = grow_ring(ctx->h_in, per * h.in.bounce.frame, pinned, cudaFreeHost);
+    if (rc == CSIC_OK) rc = grow_ring(ctx->h_out, per * h.out.bounce.frame, pinned, cudaFreeHost);
     if (rc != CSIC_OK) return rc;
   }
   // scatters chunk j's result from its bounce buffer to the caller once its D2H has landed
   auto drain = [&](size_t j) -> int {
     const int bj = (int)(j % kPipe);
-    const size_t jf0 = mine[j].first, jnf = mine[j].second;
     CSIC_CUDA(cudaEventSynchronize(ctx->ev_d2h[bj]));
-    const uint8_t* hb = static_cast<const uint8_t*>(ctx->h_out[bj]);
-    if (band) {
-      for (size_t k = 0; k < jnf; ++k)
-        parallel_rows_copy(out + (jf0 + k) * g.out_frame_bytes + (size_t)row0 * g.out_row_bytes, g.out_row_bytes,
-                           hb + k * bounce_out_frame, g.out_row_bytes, g.out_row_bytes, (size_t)rows);
-    } else {
-      parallel_rows_copy(out + jf0 * g.out_frame_bytes, bounce_out_frame, hb, bounce_out_frame, bounce_out_frame, jnf);
-    }
+    for (const csic::Copy& x : csic::frame_copies(h.out, h.out.caller.at(mine[j].first), h.out.bounce, mine[j].second))
+      host_copy(out, static_cast<const uint8_t*>(ctx->h_out.buf[bj]), x);
     return CSIC_OK;
   };
   // The scatter of chunk j runs on its own host thread, so that it overlaps the gather of chunk j + kPipe - 1 on this
-  // one (each side fans out over parallel_rows_copy's workers).  Joined before its bounce buffer is refilled.
+  // one (each side fans out over host_copy's workers).  Joined before its bounce buffer is refilled.
   struct AsyncDrain {
     std::thread th;
     int rc = CSIC_OK;
@@ -552,46 +431,26 @@ static int host_pipeline_run(csic_ctx* ctx, const csic_params* p, const uint8_t*
       CSIC_CUDA(cudaStreamWaitEvent(ctx->s_h2d, ctx->ev_k[b], 0));
       CSIC_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_d2h[b], 0));
     }
-    uint8_t* d_in = static_cast<uint8_t*>(ctx->d_in[b]);
-    uint8_t* d_out = static_cast<uint8_t*>(ctx->d_out[b]);
+    uint8_t* d_in = static_cast<uint8_t*>(ctx->d_in.buf[b]);
+    uint8_t* d_out = static_cast<uint8_t*>(ctx->d_out.buf[b]);
     if (bounce) {
       if (c >= (size_t)kPipe) CSIC_CUDA(cudaEventSynchronize(ctx->ev_h2d[b]));   // bounce_in[b] has been shipped
-      uint8_t* hb = static_cast<uint8_t*>(ctx->h_in[b]);
-      if (!band) {                          // only the rows that are read, densely; uniform stride across frames
-        parallel_rows_copy(hb, g.in_row_bytes, rgb + f0 * g.in_frame_bytes, host_row_step, g.in_row_bytes, nf * rows_stored);
-      } else {
-        for (size_t k = 0; k < nf; ++k)
-          parallel_rows_copy(hb + k * bounce_in_frame, g.in_row_bytes,
-                             rgb + (f0 + k) * g.in_frame_bytes + first_stored * host_row_step, host_row_step,
-                             g.in_row_bytes, rows_stored);
-      }
-      if (in_pitch != g.in_row_bytes) {
-        CSIC_CUDA(cudaMemcpy2DAsync(d_in, in_pitch, hb, g.in_row_bytes, g.in_row_bytes, nf * rows_stored,
-                                    cudaMemcpyHostToDevice, s_in));
-      } else {
-        CSIC_CUDA(cudaMemcpyAsync(d_in, hb, nf * bounce_in_frame, cudaMemcpyHostToDevice, s_in));
-      }
-    } else if (band) {
-      // one strided copy per frame: rows [first_stored, first_stored + rows_stored) of that frame
-      for (size_t k = 0; k < nf; ++k)
-        CSIC_CUDA(cudaMemcpy2DAsync(d_in + k * dev_frame_bytes, in_pitch,
-                                    rgb + (f0 + k) * g.in_frame_bytes + first_stored * host_row_step, host_row_step,
-                                    g.in_row_bytes, rows_stored, cudaMemcpyHostToDevice, s_in));
-    } else if (compact || lay.in_pitch) {
-      CSIC_CUDA(cudaMemcpy2DAsync(d_in, in_pitch, rgb + f0 * g.in_frame_bytes, host_row_step, g.in_row_bytes,
-                                  nf * rows_stored, cudaMemcpyHostToDevice, s_in));
+      uint8_t* hb = static_cast<uint8_t*>(ctx->h_in.buf[b]);
+      for (const csic::Copy& x : csic::frame_copies(h.in, h.in.bounce, h.in.caller.at(f0), nf)) host_copy(hb, rgb, x);
+      rc = device_copies(d_in, hb, csic::frame_copies(h.in, h.in.staging, h.in.bounce, nf), cudaMemcpyHostToDevice, s_in);
     } else {
-      CSIC_CUDA(cudaMemcpyAsync(d_in, rgb + f0 * g.in_frame_bytes, nf * g.in_frame_bytes, cudaMemcpyHostToDevice,
-                                s_in));
+      rc = device_copies(d_in, rgb, csic::frame_copies(h.in, h.in.staging, h.in.caller.at(f0), nf),
+                         cudaMemcpyHostToDevice, s_in);
     }
-    ctx->h2d_bytes += nf * rows_stored * g.in_row_bytes;
+    if (rc != CSIC_OK) return rc;
+    ctx->h2d_bytes += nf * h.in.rows * h.in.width;
     if (!single) {
       CSIC_CUDA(cudaEventRecord(ctx->ev_h2d[b], s_in));
       CSIC_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_h2d[b], 0));
     }
     // virtual frame bases: row r of the frame sits at base + r * pitch; only the band's rows are ever touched
-    rc = run(ctx, p, d_in - first_stored * in_pitch, nf, d_out - (size_t)row0 * out_pitch, row0, rows, ctx->stream,
-             compact, lay);
+    rc = run(ctx, p, d_in - h.first_stored * h.in_pitch, nf, d_out - (size_t)row0 * h.out_pitch, row0, rows, ctx->stream,
+             h.compact, h.lay);
     if (rc != CSIC_OK) return rc;
     if (!single) {
       CSIC_CUDA(cudaEventRecord(ctx->ev_k[b], ctx->stream));
@@ -599,26 +458,14 @@ static int host_pipeline_run(csic_ctx* ctx, const csic_params* p, const uint8_t*
     }
     if (bounce) {
       rc = adrain.join();                  // chunk c - kPipe has left h_out[b]
-      if (rc != CSIC_OK) return rc;
-      uint8_t* hb = static_cast<uint8_t*>(ctx->h_out[b]);
-      if (band || lay.out_pitch) {
-        CSIC_CUDA(cudaMemcpy2DAsync(hb, g.out_row_bytes, d_out, out_pitch, g.out_row_bytes, nf * (size_t)rows,
-                                    cudaMemcpyDeviceToHost, s_out));
-      } else {
-        CSIC_CUDA(cudaMemcpyAsync(hb, d_out, nf * g.out_frame_bytes, cudaMemcpyDeviceToHost, s_out));
-      }
-    } else if (band) {
-      for (size_t k = 0; k < nf; ++k)
-        CSIC_CUDA(cudaMemcpy2DAsync(out + (f0 + k) * g.out_frame_bytes + (size_t)row0 * g.out_row_bytes, g.out_row_bytes,
-                                    d_out + k * dev_out_frame_bytes, out_pitch, g.out_row_bytes, (size_t)rows,
-                                    cudaMemcpyDeviceToHost, s_out));
-    } else if (lay.out_pitch) {
-      CSIC_CUDA(cudaMemcpy2DAsync(out + f0 * g.out_frame_bytes, g.out_row_bytes, d_out, out_pitch, g.out_row_bytes,
-                                  nf * (size_t)g.out_h, cudaMemcpyDeviceToHost, s_out));
+      if (rc == CSIC_OK)
+        rc = device_copies(static_cast<uint8_t*>(ctx->h_out.buf[b]), d_out,
+                           csic::frame_copies(h.out, h.out.bounce, h.out.staging, nf), cudaMemcpyDeviceToHost, s_out);
     } else {
-      CSIC_CUDA(cudaMemcpyAsync(out + f0 * g.out_frame_bytes, d_out, nf * g.out_frame_bytes, cudaMemcpyDeviceToHost,
-                                s_out));
+      rc = device_copies(out, d_out, csic::frame_copies(h.out, h.out.caller.at(f0), h.out.staging, nf),
+                         cudaMemcpyDeviceToHost, s_out);
     }
+    if (rc != CSIC_OK) return rc;
     if (!single) CSIC_CUDA(cudaEventRecord(ctx->ev_d2h[b], s_out));
     if (bounce && c + 1 >= (size_t)kPipe) start_drain(c + 1 - (size_t)kPipe);   // the chunk issued kPipe-1 iterations ago
   }
@@ -774,11 +621,9 @@ static int multi_process_host_impl(csic_multi* m, const csic_params* p, const ui
     }
   } else {
     // fewer frames than GPUs: aligned row bands of every frame (zero halo; SURVEY.md section 8(e) E2)
-    const bool case_b = !g.chroma_first && p->factor > 1;
-    const int unit = case_b ? p->factor * g.vf : std::max(1, (p->factor % g.vf == 0 ? p->factor : p->factor * g.vf) / p->factor);
-    const int units = (g.out_h + unit - 1) / unit;
     for (size_t i = 0; i < G; ++i) {
-      const int r0 = std::min(g.out_h, (int)(units * i / G) * unit), r1 = std::min(g.out_h, (int)(units * (i + 1) / G) * unit);
+      int32_t r0, r1;
+      csic::band_split(*p, i, G, r0, r1);
       if (r1 <= r0) continue;
       th.emplace_back([=, &rcs, &errs] {
         cudaSetDevice(m->ctx[i]->device);

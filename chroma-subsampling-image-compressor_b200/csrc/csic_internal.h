@@ -4,6 +4,7 @@
 
 #include <cstddef>
 #include <cstdint>
+#include <vector>
 
 #include "../../include/csic.h"
 
@@ -118,6 +119,35 @@ struct KernelChoice { int32_t family; KPlan k; unsigned grid; };   // grid = CTA
 // The first family whose planner takes `base`: TMA row kernel, pooling kernel, flex kernel, else the generic kernel, as
 // opt.family allows.  Every candidate plans on its own copy of `base`.
 KernelChoice select_kernel(const KPlan& base, const DeviceLimits& dev, const PlanOptions& opt);
+
+// ---- host staging (csic_process_host / _band / csic_multi_process_host) --------------------------------------------
+constexpr int kPipe = 3;   // chunks in flight, each with its own staging (and bounce) buffers
+// Where row r of frame k of one buffer sits: byte off + k * frame + r * pitch; at(k): the same buffer from frame k on.
+struct CopySide { size_t off, pitch, frame; CopySide at(size_t k) const { return {off + k * frame, pitch, frame}; } };
+// One direction of the host pipeline: `rows` rows of `width` bytes per frame, as laid out in the caller's buffer, the
+// pinned bounce buffer (pageable callers) and the device staging buffer (frame 0 = the chunk's first frame).
+struct CopyShape { size_t width, rows; CopySide caller, bounce, staging; };
+struct HostPlan {
+  bool compact;                        // only every f-th input row is shipped (DECIMATE, f > 1)
+  size_t first_stored;                 // the band's first stored row (an input row, or every f-th one when compact)
+  Layout lay;                          // the staging layout run() is handed
+  size_t in_pitch, out_pitch;          // staging row pitches the kernel sees
+  size_t frames_per_chunk;
+  CopyShape in, out;                   // in.rows: stored rows per frame; a PLANAR output frame is one row
+};
+// The host pipeline of output rows [row0, row0 + rows) of n_frames frames: ~chunk_bytes of staged input per chunk;
+// full_frames ships whole frames even where compact rows would do; share_gpus: how many GPUs pull chunks from one
+// shared cursor (0: none).  Returns a CSIC_* code.
+int plan_host(const csic_params& p, int32_t row0, int32_t rows, size_t n_frames, const DeviceLimits& dev,
+              const PlanOptions& opt, size_t chunk_bytes, bool full_frames, size_t share_gpus, HostPlan& h);
+// One copy between two buffers, offsets from their bases; dst_pitch == 0: a 1-D copy of `width` bytes.
+struct Copy { size_t dst, dst_pitch, src, src_pitch, width, height; };
+// The copies that move nf frames of s: both sides dense, one 1-D copy; both sides' frames whole rows apart
+// (frame == rows * pitch), one 2-D copy over all rows; otherwise one 2-D copy per frame.
+std::vector<Copy> frame_copies(const CopyShape& s, const CopySide& dst, const CopySide& src, size_t nf);
+// Output rows [r0, r1) of GPU i of G when every frame is cut into bands that start on an alignment unit, so that no
+// band needs a row above it (sharding.band_plan); empty when r1 <= r0.
+void band_split(const csic_params& p, size_t i, size_t G, int32_t& r0, int32_t& r1);
 
 struct DecodeLaunch { DecPlan P; unsigned grid, threads; size_t smem; };
 // The TMA-staged decoder of the PLANAR batch k.in -> k.out (tile_px: pixels per tile, 0 = the planner's choice).  False

@@ -74,16 +74,22 @@ int budget_rows(uint32_t row_bytes, uint32_t budget, uint32_t tile_max, int max_
 
 // Row and pooling kernels process Wp = Wo rounded up to 16 output pixels (of opx bytes) per row, in the row padding past
 // Wo: both pitches must cover Wp (dense buffers: Wo % 16 == 0); rows, frames and bases keep 16-byte TMA granularity.
+struct PaddedRows { int32_t Wp; uint64_t in, out; };   // Wp and the least input / output row bytes that cover it
+PaddedRows padded_rows(int32_t Wo, int32_t f, int32_t ipb, uint32_t opx) {
+  const int32_t Wp = (Wo + 15) & ~15;
+  return {Wp, (uint64_t)Wp * (uint32_t)f * (uint32_t)ipb, (uint64_t)Wp * opx};
+}
+
 bool plan_padded_rows(KPlan& k, uint32_t opx) {
-  k.Wp = (k.Wo + 15) & ~15;
-  const uint64_t need_in = (uint64_t)k.Wp * (uint32_t)k.f * (uint32_t)k.in_px_bytes, need_out = (uint64_t)k.Wp * opx;
-  if (k.in_row_bytes < need_in || k.out_row_bytes < need_out) return false;
+  const PaddedRows need = padded_rows(k.Wo, k.f, k.in_px_bytes, opx);
+  k.Wp = need.Wp;
+  if (k.in_row_bytes < need.in || k.out_row_bytes < need.out) return false;
   if ((k.in_row_bytes | k.out_row_bytes) & 15u) return false;
   if ((reinterpret_cast<uintptr_t>(k.in) | reinterpret_cast<uintptr_t>(k.out)) & 15u) return false;
   if ((k.in_frame_bytes | k.out_frame_bytes) & 15u) return false;
   k.ragged = k.Wp != k.Wo;
-  k.in_dense = k.in_row_bytes == need_in;      // pooling: the f rows of a block row are contiguous
-  k.out_dense = k.out_row_bytes == need_out;
+  k.in_dense = k.in_row_bytes == need.in;      // pooling: the f rows of a block row are contiguous
+  k.out_dense = k.out_row_bytes == need.out;
   return true;
 }
 
@@ -516,4 +522,121 @@ bool plan_decode(const KPlan& k, int to_rgb, const DeviceLimits& dev, uint32_t t
   return true;
 }
 
+// ---- host staging (csic_api.cu's host pipeline) -------------------------------------------------------------------
+namespace {
+
+// Dense when the dense layout already satisfies a TMA kernel's 16-byte rules; otherwise the rows are re-pitched on the
+// way in and out (the copies are 2-D anyway), so odd widths also avoid the generic kernel.
+Layout staging_layout(const csic_params& p, const Geometry& g, bool compact, const DeviceLimits& dev,
+                      const PlanOptions& opt) {
+  auto eligible = [&](const Layout& l) {   // one frame at 4 KiB aligned bases
+    KPlan k;
+    if (build_plan(p, (void*)uintptr_t(4096), (void*)uintptr_t(4096), 1, 0, g.out_h, compact, l, k) != CSIC_OK) return false;
+    const int family = select_kernel(k, dev, opt).family;
+    return family == FAM_ROWS || family == FAM_POOL;
+  };
+  if (eligible(Layout()) || p.out_format == CSIC_OUT_PLANAR) return Layout();
+  const PaddedRows need = padded_rows(g.out_w, p.factor, g.in_px_bytes, (uint32_t)g.out_px_bytes);
+  Layout cand;
+  cand.in_pitch = (std::max<size_t>(g.in_row_bytes, need.in) + 15) & ~(size_t)15;
+  cand.out_pitch = (std::max<size_t>(g.out_row_bytes, need.out) + 15) & ~(size_t)15;
+  return eligible(cand) ? cand : Layout();
+}
+
+}  // namespace
+
+int plan_host(const csic_params& p, int32_t row0, int32_t rows, size_t n_frames, const DeviceLimits& dev,
+              const PlanOptions& opt, size_t chunk_bytes, bool full_frames, size_t share_gpus, HostPlan& h) {
+  const Geometry g = geometry(p);
+  const bool band = !(row0 == 0 && rows == g.out_h);
+  // A DECIMATE pipeline with f > 1 reads only every f-th input row, and when they sit at a uniform pitch across the
+  // frames of a batch only those rows are shipped: 1/f of the H2D bytes.
+  h.compact = p.pool_mode == CSIC_POOL_DECIMATE && p.factor > 1 && p.height % p.factor == 0 && !full_frames;
+  int32_t in_row0 = 0, in_rows = p.height;
+  if (band) {
+    const int rc = csic_band_input_rows(&p, row0, rows, &in_row0, &in_rows);
+    if (rc != CSIC_OK) return rc;
+    if (p.out_format == CSIC_OUT_PLANAR) return CSIC_EINVAL_MODE;   // planes are not row bands
+  }
+  const size_t step = h.compact ? (size_t)p.factor : 1u;            // input rows per stored row
+  h.first_stored = (size_t)in_row0 / step;
+  const size_t rows_stored = h.compact ? (size_t)(row0 + rows) - h.first_stored : (size_t)in_rows;
+  h.lay = staging_layout(p, g, h.compact, dev, opt);
+  h.in_pitch = h.lay.in_pitch ? h.lay.in_pitch : g.in_row_bytes;
+  h.out_pitch = h.lay.out_pitch ? h.lay.out_pitch : g.out_row_bytes;
+  const size_t dev_in_frame = h.in_pitch * rows_stored;
+  const size_t dev_out_frame = band ? h.out_pitch * (size_t)rows : std::max(h.out_pitch * (size_t)rows, g.out_frame_bytes);
+  if (band) h.lay = {h.in_pitch, dev_in_frame, h.out_pitch, dev_out_frame, true};   // the device holds the band's rows only
+  // Frames per chunk: ~chunk_bytes of input, at least one, at most all; several chunks per GPU that shares the cursor.
+  h.frames_per_chunk = std::min(n_frames, std::max<size_t>(1, chunk_bytes / std::max<size_t>(1, dev_in_frame)));
+  if (share_gpus)
+    h.frames_per_chunk = std::min(h.frames_per_chunk, std::max<size_t>(1, n_frames / (share_gpus * (size_t)kPipe)));
+  const size_t irb = g.in_row_bytes;
+  h.in = {irb, rows_stored, {h.first_stored * step * irb, step * irb, g.in_frame_bytes}, {0, irb, irb * rows_stored},
+          {0, h.in_pitch, dev_in_frame}};
+  const bool planar = p.out_format == CSIC_OUT_PLANAR;
+  const size_t orow = planar ? g.out_frame_bytes : g.out_row_bytes, orows = planar ? 1u : (size_t)rows;
+  h.out = {orow, orows, {(size_t)row0 * orow, orow, g.out_frame_bytes}, {0, orow, orow * orows},
+           {0, planar ? orow : h.out_pitch, dev_out_frame}};
+  return CSIC_OK;
+}
+
+std::vector<Copy> frame_copies(const CopyShape& s, const CopySide& dst, const CopySide& src, size_t nf) {
+  const size_t w = s.width, r = s.rows;
+  auto dense = [&](const CopySide& x) { return x.pitch == w && x.frame == r * w; };
+  auto whole_rows = [&](const CopySide& x) { return x.frame == r * x.pitch; };
+  if (dense(dst) && dense(src)) return {{dst.off, 0, src.off, 0, nf * r * w, 1}};
+  if (whole_rows(dst) && whole_rows(src)) return {{dst.off, dst.pitch, src.off, src.pitch, w, nf * r}};
+  std::vector<Copy> v;
+  for (size_t k = 0; k < nf; ++k) v.push_back({dst.off + k * dst.frame, dst.pitch, src.off + k * src.frame, src.pitch, w, r});
+  return v;
+}
+
+void band_split(const csic_params& p, size_t i, size_t G, int32_t& r0, int32_t& r1) {
+  const Geometry g = geometry(p);
+  const bool case_b = !g.chroma_first && p.factor > 1;
+  const int unit = case_b ? p.factor * g.vf : std::max(1, (p.factor % g.vf == 0 ? p.factor : p.factor * g.vf) / p.factor);
+  const int units = (g.out_h + unit - 1) / unit;
+  r0 = std::min(g.out_h, (int)(units * i / G) * unit);
+  r1 = std::min(g.out_h, (int)(units * (i + 1) / G) * unit);
+}
+
 }  // namespace csic
+
+extern "C" {
+
+// Input rows a band of output rows reads: the rows it decimates / pools from, plus -- when the band
+// starts on a line whose chroma is held from the line above -- the row holding that sample.
+int csic_band_input_rows(const csic_params* p, int32_t out_row0, int32_t out_rows, int32_t* in_row0,
+                         int32_t* in_rows) {
+  int rc = csic_validate(p, nullptr, 0);
+  if (rc != CSIC_OK) return rc;
+  const csic::Geometry g = csic::geometry(*p);
+  if (out_row0 < 0 || out_rows <= 0 || out_row0 + out_rows > g.out_h) return CSIC_EINVAL_ARG;
+  const int f = p->factor;
+  const bool avg = p->pool_mode == CSIC_POOL_AVERAGE && f > 1;
+  int64_t lo = (int64_t)out_row0 * f;
+  int64_t hi = (int64_t)(out_row0 + out_rows - 1) * f + (avg ? f - 1 : 0);   // inclusive
+  const bool case_b = !g.chroma_first && f > 1;
+  if (!case_b) {
+    if (g.vf == 2 && (lo & 1)) lo -= 1;   // only possible for f == 1
+  } else {
+    // chroma runs on the decimated stream with full-size counters: walk the band's first and last
+    // stream elements back to their sources (ImageCompressorTop.scala:52-58).
+    const int64_t W = p->width, Wo = g.out_w;
+    const int64_t last = ((W - 1) / g.hf) * g.hf;
+    auto src_row = [&](int64_t m) {
+      const int64_t col = m % W, line = (m / W) % p->height;
+      const int64_t s = (g.vf == 2 && (line & 1)) ? (line - 1) * W + last : m - col % g.hf;
+      return (s / Wo) * f;
+    };
+    lo = std::min(lo, src_row((int64_t)out_row0 * Wo));
+    lo = std::min(lo, src_row((int64_t)out_row0 * Wo + Wo - 1));
+  }
+  hi = std::min<int64_t>(hi, p->height - 1);
+  if (in_row0) *in_row0 = (int32_t)lo;
+  if (in_rows) *in_rows = (int32_t)(hi - lo + 1);
+  return CSIC_OK;
+}
+
+}  // extern "C"

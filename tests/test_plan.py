@@ -3,9 +3,11 @@ the parameter sources, prints the kernel family and the key fields of each plan.
 tuned rules of DESIGN.md section 5 give on a B200 (148 SMs, 232448 bytes of opt-in shared memory per block): a change
 to a tuned rule shows up here before any benchmark runs."""
 import itertools
+import json
 import os
 import subprocess
 
+import numpy as np
 import pytest
 
 from conftest import ROOT
@@ -152,3 +154,148 @@ def test_plan_depends_only_on_arguments(driver):
     env = dict(os.environ, CSIC_ROWS_NO_TALL="1", CSIC_FLEX_NO_TALL="1", CSIC_FLEX_ROWS="3", CSIC_DEC_STAGES="4",
                CSIC_DEC_THREADS="64", CSIC_DEC_TILE="1000", CSIC_DEC_NO_TMA="1")
     assert run(driver, lines[::-1], env=env)[::-1] == base
+
+
+# ---- host staging (plan_host, frame_copies, band_split) ----------------------------------------------------------------
+MIB = 1 << 20
+
+
+def host(W, H, a, b, f, ops=312, fmt=0, in_fmt=0, pool=0, n=1, row0=0, rows=-1, full=0, chunk=16 * MIB, gpus=0):
+    return f"H {W} {H} {a} {b} {f} {ops} {fmt} {in_fmt} {pool} {n} {row0} {rows} {full} {chunk} {gpus}"
+
+
+def host_plans(driver, lines):
+    return [None if r.startswith("error") else json.loads(r) for r in run(driver, lines)]
+
+
+def copy_kind(copies):
+    """one 1-D copy, one 2-D copy over all frames, or one 2-D copy per frame"""
+    if len(copies) == 1:
+        return "1d" if copies[0][1] == 0 else "2d"
+    return "frame"
+
+
+# (case, line, compact, first stored, rows stored, in pitch, out pitch, device in / out frame, frames per chunk, H2D, D2H)
+# 148 SMs, 16 MiB chunks, pinned buffers.  The last case's H2D was one 2-D copy per frame before the copy rule; its band
+# input is the whole frame.
+HOST_CASES = [
+    ("4k_bundle128", host(3840, 2160, 2, 0, 2, fmt=3, n=128), 1, 0, 1080, 11520, 7680, 12441600, 8294400, 1, "2d", "1d"),
+    ("w1000_f4", host(1000, 16, 2, 0, 4, n=2), 1, 0, 4, 3072, 768, 12288, 3072, 2, "2d", "2d"),
+    ("band_5_20", host(256, 64, 2, 0, 2, n=3, row0=5, rows=15), 1, 5, 15, 768, 384, 11520, 5760, 3, "frame", "frame"),
+    ("band_case_b", host(128, 48, 2, 0, 2, ops=123, n=2, row0=3, rows=10), 1, 1, 12, 384, 192, 4608, 1920, 2, "frame",
+     "frame"),
+    ("planar1080p", host(1920, 1080, 2, 0, 1, fmt=4, n=8), 0, 0, 1080, 5760, 1920, 6220800, 3110400, 2, "1d", "1d"),
+    ("rgb1366", host(1366, 768, 2, 0, 1, fmt=1, n=4), 0, 0, 768, 4128, 4128, 3170304, 3170304, 4, "2d", "2d"),
+    ("avg4k", host(3840, 2160, 2, 0, 2, fmt=3, pool=1, n=16), 0, 0, 2160, 11520, 7680, 24883200, 8294400, 1, "1d", "1d"),
+    ("band_whole_input", host(64, 32, 2, 0, 1, n=3, row0=1, rows=31), 0, 0, 32, 192, 192, 6144, 5952, 3, "1d", "frame"),
+]
+
+
+@pytest.mark.parametrize("case", HOST_CASES, ids=[c[0] for c in HOST_CASES])
+def test_host_plan_pins_cases(driver, case):
+    _, line, compact, first, rows_stored, in_pitch, out_pitch, in_frame, out_frame, per, h2d, d2h = case
+    h = host_plans(driver, [line])[0]
+    assert h is not None
+    got = (h["compact"], h["first_stored"], h["in_shape"][1], h["in_pitch"], h["out_pitch"], h["in_staging"][2],
+           h["out_staging"][2], h["per"])
+    assert got == (compact, first, rows_stored, in_pitch, out_pitch, in_frame, out_frame, per), h
+    c0 = h["chunks"][0]
+    assert (copy_kind(c0["h2d"]), copy_kind(c0["d2h"])) == (h2d, d2h), c0
+
+
+def covered(copies, side, size, frame_bytes=None):
+    """Bytes each copy touches on one side ("dst" or "src") as a count per byte of a buffer of `size` bytes; every range
+    must lie inside the buffer."""
+    off, pitch = (0, 1) if side == "dst" else (2, 3)
+    diff = np.zeros(size + 1, dtype=np.int64)
+    for c in copies:
+        width, height = (c[4], 1) if c[1] == 0 else (c[4], c[5])
+        starts = c[off] + np.arange(height, dtype=np.int64) * (c[pitch] if c[1] else 0)
+        assert starts.min() >= 0 and starts.max() + width <= size, (c, size)
+        np.add.at(diff, starts, 1)
+        np.add.at(diff, starts + width, -1)
+    return np.cumsum(diff[:-1])
+
+
+def host_grid_lines():
+    lines = []
+    sizes = [(3, 5), (6, 4), (17, 16), (64, 32), (96, 64), (128, 48), (333, 120)]
+    for (W, H), (a, b), f, fmt, pool, ops in itertools.product(sizes, [(4, 4), (2, 0), (1, 0)], [1, 2, 4],
+                                                                 [0, 1, 3, 4], [0, 1], [312, 123]):
+        Ho = -(-H // f)
+        bands = [(0, -1), (1, Ho - 1), (Ho // 3, max(1, Ho // 3))]
+        for (row0, rows), (chunk, gpus) in itertools.product(bands, [(64 << 10, 0), (96 << 10, 2), (16 * MIB, 3),
+                                                                     (64 << 10, 1)]):
+            if rows == 0 or (row0, rows) == (0, Ho):
+                continue
+            lines.append(host(W, H, a, b, f, ops=ops, fmt=fmt, pool=pool, n=7, row0=row0, rows=rows, chunk=chunk,
+                              gpus=gpus, full=int(W == 17)))
+    return lines
+
+
+def test_host_copies_over_grid(driver):
+    """The copies of every chunk: D2H writes exactly the band's output rows of every frame, each byte once; H2D reads
+    exactly the rows csic_band_input_rows names (every f-th when compact), each once, and ships what csic_host_bytes
+    counts; staging and bounce sides stay inside their buffers.  Direct and bounce paths alike."""
+    lines = host_grid_lines()
+    planned = 0
+    for line, h in zip(lines, host_plans(driver, lines)):
+        if h is None:
+            continue
+        planned += 1
+        t = line.split()
+        H, f, n, row0, rows = int(t[2]), int(t[5]), int(t[10]), int(t[11]), int(t[12])
+        irb, in_frame = h["in_shape"][0], h["in_caller"][2]
+        out_frame, (ow, orows) = h["out_caller"][2], h["out_shape"]
+        per, compact = h["per"], h["compact"]
+        if rows < 0:
+            row0, rows, lo, n_in = 0, orows, 0, H
+        else:
+            lo, n_in = h["in_rows"]
+        # expected caller bytes: output rows [row0, row0 + rows) of every frame (a PLANAR frame is one row)
+        want_out = np.zeros(n * out_frame, dtype=np.int64)
+        want_in = np.zeros(n * in_frame, dtype=np.int64)
+        for k in range(n):
+            want_out[k * out_frame + row0 * ow: k * out_frame + (row0 + orows) * ow] = 1
+            for r in range(lo, lo + n_in):
+                if not compact or r % f == 0:
+                    want_in[k * in_frame + r * irb: k * in_frame + (r + 1) * irb] = 1
+        for path in (("h2d", "d2h"), ("gather", "scatter")):
+            reads, writes = [], []
+            for c in h["chunks"]:
+                reads += c[path[0]]
+                writes += c[path[1]]
+            assert np.array_equal(covered(writes, "dst", n * out_frame), want_out), (line, path)
+            assert np.array_equal(covered(reads, "src", n * in_frame), want_in), (line, path)
+            shipped = sum(c[4] * (1 if c[1] == 0 else c[5]) for c in reads)
+            assert shipped == n * h["in_shape"][1] * irb == int(want_in.sum()), line
+        for c in h["chunks"]:
+            assert c["nf"] <= per
+            for name, side, buf in (("h2d", "dst", "in_staging"), ("d2h", "src", "out_staging"),
+                                    ("gather", "dst", "in_bounce"), ("scatter", "src", "out_bounce"),
+                                    ("b2d", "dst", "in_staging"), ("b2d", "src", "in_bounce"),
+                                    ("d2b", "dst", "out_bounce"), ("d2b", "src", "out_staging")):
+                width, nrows = h["in_shape"] if buf.startswith("in") else h["out_shape"]
+                cov = covered(c[name], side, per * h[buf][2])
+                assert cov.max() <= 1 and cov.sum() == c["nf"] * width * nrows, (line, name, side)
+    assert planned > 3000
+
+
+def test_band_split_matches_sharding(driver):
+    import csic_b200 as csic
+    cases = []
+    for (a, b), f, ops, H, G in itertools.product([(4, 4), (4, 2), (2, 2), (2, 0), (1, 1), (1, 0)], [1, 2, 4, 8],
+                                                  [312, 123, 231, 132], [1, 7, 16, 33, 100, 1080], [1, 2, 3, 5, 8]):
+        cases.append((f"B {8 * f} {H} {a} {b} {f} {ops} {G}", (a, b, f, ops, H, G)))
+    out = run(driver, [c[0] for c in cases])
+    checked = 0
+    for (line, (a, b, f, ops, H, G)), res in zip(cases, out):
+        if res.startswith("error"):
+            continue
+        digits = [ops // 100, ops // 10 % 10, ops % 10]
+        chroma_first = digits.index(3) < digits.index(1)   # csic_step: 3 chroma, 1 spatial
+        v = list(map(int, res.split()))
+        got = [(v[2 * i], v[2 * i + 1] - v[2 * i]) for i in range(G)]
+        assert got == csic.sharding.band_plan(-(-H // f), G, f, a, b, chroma_first), line
+        checked += 1
+    assert checked > 1000
