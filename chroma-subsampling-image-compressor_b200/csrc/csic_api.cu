@@ -101,13 +101,7 @@ int run(csic_ctx* ctx, const csic_params* p, const void* d_rgb, size_t n_frames,
   DeviceGuard guard(ctx->device);
   cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : ctx->stream;
   const csic::KernelChoice c = csic::select_kernel(base, ctx->dev, ctx->opt);
-  int err;
-  switch (c.family) {
-    case csic::FAM_ROWS: err = csic::launch_rows(c.k, c.grid, st); break;
-    case csic::FAM_POOL: err = csic::launch_pool(c.k, c.grid, st); break;
-    case csic::FAM_FLEX: err = csic::launch_flex(c.k, c.grid, st); break;
-    default: err = csic::launch_generic(c.k, c.grid, st); break;
-  }
+  const int err = csic::launch(c, st);
   ctx->last_family = c.family;
   ctx->launches += 1;
   if (err != (int)cudaSuccess) return cuda_fail((cudaError_t)err, "kernel launch");
@@ -171,7 +165,7 @@ int csic_create(int device, csic_ctx** out) {
     step(cudaEventCreateWithFlags(&c->ev_h2d[i], cudaEventDisableTiming)) &&
         step(cudaEventCreateWithFlags(&c->ev_k[i], cudaEventDisableTiming)) &&
         step(cudaEventCreateWithFlags(&c->ev_d2h[i], cudaEventDisableTiming));
-  if (err == cudaSuccess) step((cudaError_t)csic::rows_kernel_set_attributes(c->dev.max_smem_optin));
+  if (err == cudaSuccess) step((cudaError_t)csic::set_kernel_attributes(c->dev.max_smem_optin));
   if (err != cudaSuccess) {
     const int rc = cuda_fail(err, "csic_create");
     const std::string keep = g_last_error;

@@ -214,33 +214,24 @@ __global__ void __launch_bounds__(kDecMaxConsumers + 32) csic_decode_kernel(cons
   const uint32_t tid = threadIdx.x;
   const uint32_t NC = blockDim.x - 32u;          // consumer threads; the last warp is the producer
   const uint32_t sbase = smem_u32(smem);
-  const uint32_t S = P.stages;
-  const uint32_t n_my = (P.n_tiles > blockIdx.x) ? (P.n_tiles - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
   const uint64_t pol = policy_evict_first();
-  const uint32_t full_bar = sbase + P.bar_off, empty_bar = full_bar + S * 8u;
-
-  if (tid == 0) {
-    for (uint32_t s = 0; s < S; ++s) {
-      mbar_init(full_bar + s * 8u, 1);
-      mbar_init(empty_bar + s * 8u, NC / 32u);
-    }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  __syncthreads();
+  const Ring ring(sbase + P.bar_off, P.stages, P.n_tiles);
+  ring.init(NC / 32u);                           // one arrive per consumer warp
 
   // ============================== producer warp ==============================================
   if (tid >= NC) {
     const uint32_t lane = tid - NC;
-    uint32_t s = 0, par = 1;                      // parity of the empty barrier's PREVIOUS phase: first pass falls through
-    for (uint32_t i = 0; i < n_my; ++i) {
-      if (i >= S) mbar_wait(empty_bar + s * 8u, par);
+    Ring::Pos pos;
+    for (uint32_t i = 0; i < ring.n_my; ++i, pos.next(ring.S)) {
+      const uint32_t s = pos.s;
+      ring.wait_empty(pos, i);
       if (lane < 3u) {
         const uint32_t tile = blockIdx.x + i * gridDim.x;
         const uint32_t k = tile / P.tiles_per_frame, tt = tile - k * P.tiles_per_frame;
         const uint32_t p0 = tt * P.tile_px, npx = min(P.tile_px, P.A - p0), p1 = p0 + npx - 1u;
         const uint32_t r0 = p0 / P.Wo, col0 = p0 - r0 * P.Wo, r1 = p1 / P.Wo, col1 = p1 - r1 * P.Wo;
         const uint8_t* frame = P.planar + (uint64_t)k * P.frame_bytes;
-        const uint32_t bar = full_bar + s * 8u;
+        const uint32_t bar = ring.full(s);
         const uint32_t slot = sbase + s * P.stage_stride;
         DecDesc* d = reinterpret_cast<DecDesc*>(smem + P.desc_off) + s;
         if (lane == 0) {
@@ -266,8 +257,7 @@ __global__ void __launch_bounds__(kDecMaxConsumers + 32) csic_decode_kernel(cons
         }
       }
       __syncwarp();
-      if (lane == 0) mbar_arrive(full_bar + s * 8u);
-      if (++s == S) { s = 0; par ^= 1u; }
+      if (lane == 0) mbar_arrive(ring.full(s));
     }
     return;
   }
@@ -276,9 +266,10 @@ __global__ void __launch_bounds__(kDecMaxConsumers + 32) csic_decode_kernel(cons
   const uint32_t Wo = P.Wo, cw = P.cw, last_c = P.last_c;
   const bool w16 = (Wo & 15u) == 0u, w4 = (Wo & 3u) == 0u;
   const DecWalk walk16 = make_walk(16u, tid, NC, Wo), walk4 = make_walk(4u, tid, NC, Wo);
-  uint32_t s = 0, par = 0;
-  for (uint32_t i = 0; i < n_my; ++i) {
-    mbar_wait(full_bar + s * 8u, par);
+  Ring::Pos pos;
+  for (uint32_t i = 0; i < ring.n_my; ++i, pos.next(ring.S)) {
+    const uint32_t s = pos.s;
+    ring.wait_full(pos);
     const DecDesc* d = reinterpret_cast<const DecDesc*>(smem + P.desc_off) + s;
     DecTile T;
     T.npx = d->npx; T.y_s = d->y_s; T.cb_s = d->cb_s; T.cr_s = d->cr_s; T.r0 = d->r0; T.col0 = d->col0; T.nrows = d->nrows;
@@ -293,7 +284,7 @@ __global__ void __launch_bounds__(kDecMaxConsumers + 32) csic_decode_kernel(cons
     else tile_granules<HS, VHOLD, RGB, false>(T, walk4, Wo, cw, last_c, tid, NC);
     // inputs consumed: the stage goes back to the producer
     __syncwarp();
-    if ((tid & 31u) == 0) mbar_arrive(empty_bar + s * 8u);
+    if ((tid & 31u) == 0) mbar_arrive(ring.empty(s));
 
     const uint32_t len = T.npx * 3u;
     if ((galign & 3u) == 0u) {
@@ -314,50 +305,26 @@ __global__ void __launch_bounds__(kDecMaxConsumers + 32) csic_decode_kernel(cons
       consumer_barrier(NC);
       span_store(out_g, T.out_s, len, tid, NC);
     }
-    if (++s == S) { s = 0; par ^= 1u; }
   }
   if (tid == 0) tma_store_wait_all();
 }
 
 template <int HS, bool VHOLD>
-int launch_hv(const DecPlan& P, unsigned grid, unsigned threads, size_t smem, cudaStream_t st) {
-  if (P.to_rgb) csic_decode_kernel<HS, VHOLD, true><<<grid, threads, smem, st>>>(P);
-  else csic_decode_kernel<HS, VHOLD, false><<<grid, threads, smem, st>>>(P);
-  return (int)cudaGetLastError();
-}
-template <int HS, bool VHOLD>
-cudaError_t attr_hv(int bytes) {
-  cudaError_t e = cudaFuncSetAttribute(csic_decode_kernel<HS, VHOLD, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
-  if (e != cudaSuccess) return e;
-  return cudaFuncSetAttribute(csic_decode_kernel<HS, VHOLD, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+DecodeFn by_rgb(bool to_rgb) { return to_rgb ? csic_decode_kernel<HS, VHOLD, true> : csic_decode_kernel<HS, VHOLD, false>; }
+template <bool VHOLD>
+DecodeFn by_hs(uint32_t hs_sh, bool to_rgb) {
+  return hs_sh == 0 ? by_rgb<0, VHOLD>(to_rgb) : (hs_sh == 1 ? by_rgb<1, VHOLD>(to_rgb) : by_rgb<2, VHOLD>(to_rgb));
 }
 
 }  // namespace
 
-int launch_decode_tma(const DecodeLaunch& d, void* stream) {
-  const DecPlan& P = d.P;
-  cudaStream_t st = (cudaStream_t)stream;
-  if (P.vhold) {
-    switch (P.hs_sh) {
-      case 0: return launch_hv<0, true>(P, d.grid, d.threads, d.smem, st);
-      case 1: return launch_hv<1, true>(P, d.grid, d.threads, d.smem, st);
-      default: return launch_hv<2, true>(P, d.grid, d.threads, d.smem, st);
-    }
-  }
-  switch (P.hs_sh) {
-    case 0: return launch_hv<0, false>(P, d.grid, d.threads, d.smem, st);
-    case 1: return launch_hv<1, false>(P, d.grid, d.threads, d.smem, st);
-    default: return launch_hv<2, false>(P, d.grid, d.threads, d.smem, st);
-  }
+DecodeFn decode_kernel(uint32_t hs_sh, bool vhold, bool to_rgb) {
+  return vhold ? by_hs<true>(hs_sh, to_rgb) : by_hs<false>(hs_sh, to_rgb);
 }
 
-int decode_set_attributes(size_t max_smem_optin) {
-  cudaError_t e;
-  const int b = (int)max_smem_optin;
-  if ((e = attr_hv<0, true>(b)) != cudaSuccess || (e = attr_hv<1, true>(b)) != cudaSuccess || (e = attr_hv<2, true>(b)) != cudaSuccess ||
-      (e = attr_hv<0, false>(b)) != cudaSuccess || (e = attr_hv<1, false>(b)) != cudaSuccess || (e = attr_hv<2, false>(b)) != cudaSuccess)
-    return (int)e;
-  return (int)cudaSuccess;
+int launch_decode_tma(const DecodeLaunch& d, void* stream) {
+  decode_kernel(d.P.hs_sh, d.P.vhold, d.P.to_rgb)<<<d.grid, d.threads, d.smem, (cudaStream_t)stream>>>(d.P);
+  return (int)cudaGetLastError();
 }
 
 }  // namespace csic

@@ -128,11 +128,11 @@ static_assert(sizeof(FlexDesc) == kFlexDescBytes, "kFlexDescBytes out of sync");
 
 // The consumer warps' loop over this CTA's tiles.
 template <int FMT, bool TRUNC, uint32_t HFE, uint32_t PXB, bool DIRECT>
-__device__ __forceinline__ void flex_consume(const KPlan& P, uint8_t* smem, uint32_t n_my) {
+__device__ __forceinline__ void flex_consume(const KPlan& P, uint8_t* smem, const Ring& ring) {
   constexpr uint32_t kUnit = FlexFmt<FMT>::kUnit;
   const uint32_t tid = threadIdx.x, NC = blockDim.x - 32u, NW = NC >> 5;
   const uint32_t sbase = smem_u32(smem), out_s = sbase + P.out_buf_off, held_base = sbase + P.meta_off;
-  const uint32_t S = (uint32_t)P.stages, full0 = sbase + P.bar_off, empty0 = full0 + 8u * S, desc0 = full0 + 16u * S;
+  const uint32_t desc0 = sbase + P.bar_off + kRingBarBytes * ring.S;
   const uint32_t in_stage = P.stage_stride * (uint32_t)P.tile_rows + 32u;     // bytes of one input stage
   const uint32_t ipb = (uint32_t)P.in_px_bytes, pxb = (uint32_t)P.f * ipb;
   const uint32_t nsplit = (uint32_t)P.nsplit;
@@ -153,9 +153,10 @@ __device__ __forceinline__ void flex_consume(const KPlan& P, uint8_t* smem, uint
   //      row-dependent set up once per warp -- taken when at least 4/5 of the lanes of a row's warps get a granule
   //   1  very wide rows: row by row with the whole CTA          2  more rows than warps: one row per warp and round
   //   3  one flat loop over the tile's granules (rows that deal unevenly)
-  uint32_t s = 0, ph = 0;
-  for (uint32_t it = 0; it < n_my; ++it) {
-    mbar_wait(full0 + s * 8u, ph);
+  Ring::Pos pos;
+  for (uint32_t it = 0; it < ring.n_my; ++it, pos.next(ring.S)) {
+    const uint32_t s = pos.s;
+    ring.wait_full(pos);
     const uint32_t da = desc0 + s * kFlexDescBytes;
     const uint4 d0 = lds128(da), d1 = lds128(da + 16u), d2 = lds128(da + 32u), d3 = lds128(da + 48u);
     const uint4 d4 = lds128(da + 64u);   // row_out, out_one, ncols, direct
@@ -313,7 +314,7 @@ __device__ __forceinline__ void flex_consume(const KPlan& P, uint8_t* smem, uint
       }
     }
     consumer_barrier(NC);          // staging complete; every read of input stage s, its held words and descriptor is done
-    if (tid == 0) mbar_arrive(empty0 + s * 8u);
+    if (tid == 0) mbar_arrive(ring.empty(s));
 
     // ---- store ---------------------------------------------------------------------------------------------
     if (direct) {
@@ -339,7 +340,6 @@ __device__ __forceinline__ void flex_consume(const KPlan& P, uint8_t* smem, uint
         });
       }
     }
-    if (++s == S) { s = 0u; ph ^= 1u; }
   }
 }
 
@@ -349,28 +349,18 @@ __global__ void __launch_bounds__(kFlexMaxThreads, 4) csic_flex_kernel(const __g
   constexpr uint32_t kUnit = FlexFmt<FMT>::kUnit, kOpx = kUnit / 4u;
   const uint32_t tid = threadIdx.x, NT = blockDim.x;
   const uint32_t sbase = smem_u32(smem), held_base = sbase + P.meta_off;
-  const uint32_t bar0 = sbase + P.bar_off;
-  const uint32_t S = (uint32_t)P.stages;
   const uint32_t in_stage = P.stage_stride * (uint32_t)P.tile_rows + 32u;     // bytes of one input stage
   const uint32_t ipb = (uint32_t)P.in_px_bytes, f = (uint32_t)P.f, pxb = f * ipb;
   const uint32_t nsplit = (uint32_t)P.nsplit;
   const uint32_t hfe = (uint32_t)P.hfe;
   const bool vhold = P.vf == 2;
   const uint64_t rstep = (uint64_t)(uint32_t)P.row_step * P.in_row_bytes;
-  const uint32_t n_my = (P.n_tiles > blockIdx.x) ? (P.n_tiles - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
-  if (n_my == 0) return;
+  const Ring ring(sbase + P.bar_off, (uint32_t)P.stages, P.n_tiles);
+  if (ring.n_my == 0) return;
   // Input rows of a tile land in stage s at  in(s) + j * rs_mul + ((a0 + j * rs_add) & 15),  a0 = src0 & 15.
   const uint32_t rs_mul = P.in_dense ? P.in_row_bytes : P.stage_stride;
   const uint32_t NC = NT - 32u;    // consumer threads; the last warp is the producer
-  const uint32_t full0 = bar0, empty0 = bar0 + 8u * S;
-  if (tid == 0) {
-    for (uint32_t s = 0; s < S; ++s) {
-      mbar_init(full0 + s * 8u, 1);        // the producer's arrive (+ the TMA byte count)
-      mbar_init(empty0 + s * 8u, 1);       // one consumer's arrive, behind the consumers' barrier
-    }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  __syncthreads();
+  ring.init(1);                    // one consumer's arrive, behind the consumers' barrier
 
   // ============================== producer warp ==============================================================
   // Walks this CTA's tiles up to S stages ahead of the consumers.  All lanes track the geometry; lane 0 describes the
@@ -386,11 +376,11 @@ __global__ void __launch_bounds__(kFlexMaxThreads, 4) csic_flex_kernel(const __g
     const uintptr_t lim_hi = reinterpret_cast<uintptr_t>(P.in) + (uint64_t)(P.n_frames - 1u) * P.in_frame_bytes +
                              (uint64_t)((uint32_t)(P.row0 + P.band_rows - 1) * (uint32_t)P.row_step) * P.in_row_bytes +
                              ((uint32_t)P.Wo - 1u) * pxb + ipb;
-    uint32_t s = 0, ph = 1;                 // stage and the parity of the empty-barrier phase to wait for (from the second lap)
-    for (uint32_t j = 0; j < n_my; ++j, s = (s + 1u == S) ? 0u : s + 1u, ph ^= (s == 0u) ? 1u : 0u) {
-      const uint32_t bar = full0 + s * 8u, in_s = sbase + s * in_stage;
-      if (j >= S) mbar_wait(empty0 + s * 8u, ph);                          // the consumers drained the previous use
-      FlexDesc* d = reinterpret_cast<FlexDesc*>(smem + P.bar_off + 16u * S) + s;
+    Ring::Pos pos;
+    for (uint32_t j = 0; j < ring.n_my; ++j, pos.next(ring.S)) {
+      const uint32_t s = pos.s, bar = ring.full(s), in_s = sbase + s * in_stage;
+      ring.wait_empty(pos, j);
+      FlexDesc* d = reinterpret_cast<FlexDesc*>(smem + P.bar_off + kRingBarBytes * ring.S) + s;
       const uint32_t ro0 = (uint32_t)P.row0 + ptb * (uint32_t)P.tile_rows;
       const uint32_t nrows = min((uint32_t)P.tile_rows, (uint32_t)(P.row0 + P.band_rows) - ro0);
       const uint32_t col0 = pseg * (uint32_t)P.tile_px;
@@ -490,56 +480,27 @@ __global__ void __launch_bounds__(kFlexMaxThreads, 4) csic_flex_kernel(const __g
   auto run = [&](auto hfe_tag) {
     constexpr uint32_t H = decltype(hfe_tag)::value;
     if (direct) {
-      if (pxb == 3u) flex_consume<FMT, TRUNC, H, 3u, true>(P, smem, n_my);
-      else if (pxb == 6u) flex_consume<FMT, TRUNC, H, 6u, true>(P, smem, n_my);
-      else flex_consume<FMT, TRUNC, H, 0u, true>(P, smem, n_my);
-    } else if (pxb == 3u) flex_consume<FMT, TRUNC, H, 3u, false>(P, smem, n_my);          // RGB24, f = 1
-    else if (pxb == 6u) flex_consume<FMT, TRUNC, H, 6u, false>(P, smem, n_my);     // RGB24, f = 2
-    else flex_consume<FMT, TRUNC, H, 0u, false>(P, smem, n_my);                    // sampled pixels on a common byte phase
+      if (pxb == 3u) flex_consume<FMT, TRUNC, H, 3u, true>(P, smem, ring);
+      else if (pxb == 6u) flex_consume<FMT, TRUNC, H, 6u, true>(P, smem, ring);
+      else flex_consume<FMT, TRUNC, H, 0u, true>(P, smem, ring);
+    } else if (pxb == 3u) flex_consume<FMT, TRUNC, H, 3u, false>(P, smem, ring);          // RGB24, f = 1
+    else if (pxb == 6u) flex_consume<FMT, TRUNC, H, 6u, false>(P, smem, ring);     // RGB24, f = 2
+    else flex_consume<FMT, TRUNC, H, 0u, false>(P, smem, ring);                    // sampled pixels on a common byte phase
   };
   if (hfe == 1u) run(std::integral_constant<uint32_t, 1u>{});
   else if (hfe == 2u) run(std::integral_constant<uint32_t, 2u>{});
   else run(std::integral_constant<uint32_t, 4u>{});
 }
 
-// ---- dispatch ------------------------------------------------------------------------------------------------
-namespace {
-template <int FMT>
-int launch_flex_fmt(const KPlan& k, unsigned grid, cudaStream_t st) {
-  const unsigned threads = (unsigned)k.block_threads + 32u;   // + producer warp
-  if (k.trunc) csic_flex_kernel<FMT, true><<<grid, threads, k.smem_bytes, st>>>(k);
-  else csic_flex_kernel<FMT, false><<<grid, threads, k.smem_bytes, st>>>(k);
-  return (int)cudaGetLastError();
-}
-template <int FMT>
-cudaError_t flex_attr(size_t b) {
-  cudaError_t e = cudaFuncSetAttribute(csic_flex_kernel<FMT, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)b);
-  if (e != cudaSuccess) return e;
-  return cudaFuncSetAttribute(csic_flex_kernel<FMT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)b);
-}
-}  // namespace
-
-int launch_flex(const KPlan& k, unsigned grid, void* stream) {
-  cudaStream_t st = (cudaStream_t)stream;
-  switch (k.kformat) {
-    case KF_YCC888: return launch_flex_fmt<KF_YCC888>(k, grid, st);
-    case KF_RGB888: return launch_flex_fmt<KF_RGB888>(k, grid, st);
-    case KF_SLOT8: return launch_flex_fmt<KF_SLOT8>(k, grid, st);
-    case KF_SLOT16: return launch_flex_fmt<KF_SLOT16>(k, grid, st);
-    case KF_PLANAR: return launch_flex_fmt<KF_PLANAR>(k, grid, st);
-    default: return launch_flex_fmt<KF_SLOT32>(k, grid, st);
+KernelFn flex_kernel(int kformat, bool trunc) {
+  switch (kformat) {
+    case KF_YCC888: return trunc ? csic_flex_kernel<KF_YCC888, true> : csic_flex_kernel<KF_YCC888, false>;
+    case KF_RGB888: return trunc ? csic_flex_kernel<KF_RGB888, true> : csic_flex_kernel<KF_RGB888, false>;
+    case KF_SLOT8: return trunc ? csic_flex_kernel<KF_SLOT8, true> : csic_flex_kernel<KF_SLOT8, false>;
+    case KF_SLOT16: return trunc ? csic_flex_kernel<KF_SLOT16, true> : csic_flex_kernel<KF_SLOT16, false>;
+    case KF_PLANAR: return trunc ? csic_flex_kernel<KF_PLANAR, true> : csic_flex_kernel<KF_PLANAR, false>;
+    default: return trunc ? csic_flex_kernel<KF_SLOT32, true> : csic_flex_kernel<KF_SLOT32, false>;
   }
-}
-
-int flex_set_attributes(size_t max_smem_optin) {
-  cudaError_t e;
-  if ((e = flex_attr<KF_YCC888>(max_smem_optin)) != cudaSuccess) return (int)e;
-  if ((e = flex_attr<KF_RGB888>(max_smem_optin)) != cudaSuccess) return (int)e;
-  if ((e = flex_attr<KF_SLOT8>(max_smem_optin)) != cudaSuccess) return (int)e;
-  if ((e = flex_attr<KF_SLOT16>(max_smem_optin)) != cudaSuccess) return (int)e;
-  if ((e = flex_attr<KF_SLOT32>(max_smem_optin)) != cudaSuccess) return (int)e;
-  if ((e = flex_attr<KF_PLANAR>(max_smem_optin)) != cudaSuccess) return (int)e;
-  return (int)cudaSuccess;
 }
 
 }  // namespace csic

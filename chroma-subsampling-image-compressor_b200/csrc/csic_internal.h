@@ -69,6 +69,7 @@ struct KPlan {
 };
 
 // Constants shared by the planners (csic_plan.cpp) and the kernels.
+constexpr uint32_t kRingBarBytes = 16;      // mbarrier bytes per stage of a TMA-staged kernel's ring (Ring, csic_tma.cuh)
 constexpr int kDefaultBlockThreads = 256;   // row kernel: consumer threads; one producer warp is added at launch
 constexpr int kMaxConsumerThreads = 512;
 constexpr int kMaxTileRows = 64;        // rows per tile of the row kernel (small frames: 64 rows x 384 B still make a 24 KB tile; 256 rows
@@ -155,26 +156,20 @@ struct DecodeLaunch { DecPlan P; unsigned grid, threads; size_t smem; };
 // pixels per frame, 2^32 or more tiles per launch, or chroma rows so wide that a stage does not fit.
 bool plan_decode(const KPlan& k, int to_rgb, const DeviceLimits& dev, uint32_t tile_px, DecodeLaunch& d);
 
-// ---- launch shims and attribute setters (kernel files); each returns a cudaError_t as int ---------------------------
-int launch_generic(const KPlan& k, unsigned grid, void* stream);
+// ---- kernel instances and launches (kernel files); each int result is a cudaError_t --------------------------------
+// One function per family (per factor where the build compiles one file per factor) maps a plan's run-time key to the
+// kernel's template instance.  The launchers and set_kernel_attributes both go through them, and the setter enumerates
+// every key, so no instance a plan can select runs without its dynamic shared-memory limit raised.
+using KernelFn = void (*)(KPlan);
+using DecodeFn = void (*)(DecPlan);
+template <int F> KernelFn rows_kernel(int kformat, bool q8, bool trunc);   // csic_rows_kernel.cu, F = 1, 2, 4, 8
+template <int F> KernelFn pool_kernel(int kformat, bool in4);              // csic_pool_kernel.cu, F = 2, 4, 8 (AVERAGE)
+KernelFn flex_kernel(int kformat, bool trunc);                             // csic_flex_kernel.cu
+DecodeFn decode_kernel(uint32_t hs_sh, bool vhold, bool to_rgb);           // csic_decode_kernel.cu
+int launch(const KernelChoice& c, void* stream);                           // csic_kernels.cu: the chosen kernel
+int set_kernel_attributes(size_t max_smem_optin);
 int launch_expand_planar(const KPlan& k, int to_rgb, int sm_count, void* stream);   // LDG decoder of k.in -> k.out
 int launch_decode_tma(const DecodeLaunch& d, void* stream);
-int decode_set_attributes(size_t max_smem_optin);
-int launch_rows(const KPlan& k, unsigned grid, void* stream);
-int rows_kernel_set_attributes(size_t max_smem_optin);
-
-// AVERAGE extension: TMA-staged pooling kernel (csic_pool_kernel.cu), chroma-first orders only.
-int launch_pool(const KPlan& k, unsigned grid, void* stream);
-template <int F> int launch_pool_factor(const KPlan& k, unsigned grid, void* stream);
-template <int F> int pool_set_attributes_factor(size_t max_smem_optin);
-
-// Any width / pitch / base alignment (csic_flex_kernel.cu): DECIMATE pipelines the TMA kernels' 16-byte rules exclude.
-int launch_flex(const KPlan& k, unsigned grid, void* stream);
-int flex_set_attributes(size_t max_smem_optin);
-
-// Implemented once per spatial factor in csic_rows_kernel.cu (explicit specialisations for F = 1, 2, 4, 8).
-template <int F> int launch_rows_factor(const KPlan& k, unsigned grid, void* stream);
-template <int F> int rows_set_attributes_factor(size_t max_smem_optin);
 
 }  // namespace csic
 

@@ -432,64 +432,85 @@ int launch_expand_planar(const KPlan& k, int to_rgb, int sm_count, void* stream)
 
 namespace {
 template <int FMT, int AF>
-int launch_generic_af(const KPlan& k, unsigned blocks, unsigned threads, cudaStream_t st) {
-  if (k.trunc) csic_generic_kernel<true, FMT, AF><<<blocks, threads, 0, st>>>(k);
-  else csic_generic_kernel<false, FMT, AF><<<blocks, threads, 0, st>>>(k);
-  return (int)cudaGetLastError();
-}
+KernelFn generic_by_trunc(bool trunc) { return trunc ? csic_generic_kernel<true, FMT, AF> : csic_generic_kernel<false, FMT, AF>; }
 template <int FMT>
-int launch_generic_fmt(const KPlan& k, unsigned blocks, unsigned threads, cudaStream_t st) {
-  if (!(k.average && k.f > 1)) return launch_generic_af<FMT, 0>(k, blocks, threads, st);
-  if (k.f == 2) return launch_generic_af<FMT, 2>(k, blocks, threads, st);
-  if (k.f == 4) return launch_generic_af<FMT, 4>(k, blocks, threads, st);
-  return launch_generic_af<FMT, 8>(k, blocks, threads, st);
+KernelFn generic_by_af(int af, bool trunc) {
+  switch (af) {
+    case 2: return generic_by_trunc<FMT, 2>(trunc);
+    case 4: return generic_by_trunc<FMT, 4>(trunc);
+    case 8: return generic_by_trunc<FMT, 8>(trunc);
+    default: return generic_by_trunc<FMT, 0>(trunc);
+  }
+}
+// af: the AVERAGE factor, 0 for DECIMATE (see csic_generic_kernel)
+KernelFn generic_kernel(int kformat, int af, bool trunc) {
+  switch (kformat) {
+    case KF_YCC888: return generic_by_af<KF_YCC888>(af, trunc);
+    case KF_RGB888: return generic_by_af<KF_RGB888>(af, trunc);
+    case KF_SLOT8: return generic_by_af<KF_SLOT8>(af, trunc);
+    case KF_SLOT16: return generic_by_af<KF_SLOT16>(af, trunc);
+    case KF_PLANAR: return generic_by_af<KF_PLANAR>(af, trunc);
+    default: return generic_by_af<KF_SLOT32>(af, trunc);
+  }
+}
+
+// the per-factor instances of the row and pooling kernels (compiled one file per factor)
+KernelFn rows_for(int f, int kformat, bool q8, bool trunc) {
+  switch (f) {
+    case 1: return rows_kernel<1>(kformat, q8, trunc);
+    case 2: return rows_kernel<2>(kformat, q8, trunc);
+    case 4: return rows_kernel<4>(kformat, q8, trunc);
+    default: return rows_kernel<8>(kformat, q8, trunc);
+  }
+}
+
+KernelFn pool_for(int f, int kformat, bool in4) {
+  switch (f) {
+    case 2: return pool_kernel<2>(kformat, in4);
+    case 4: return pool_kernel<4>(kformat, in4);
+    default: return pool_kernel<8>(kformat, in4);
+  }
 }
 }  // namespace
 
-int launch_generic(const KPlan& k, unsigned blocks, void* stream) {
-  if (blocks == 0) return (int)cudaSuccess;
-  if ((uint64_t)k.n_frames * (uint64_t)k.band_rows >= (1ull << 32)) return (int)cudaErrorInvalidValue;
-  const unsigned threads = 128u;   // four warps per CTA
-  cudaStream_t st = (cudaStream_t)stream;
-  switch (k.kformat) {
-    case KF_YCC888: return launch_generic_fmt<KF_YCC888>(k, blocks, threads, st);
-    case KF_RGB888: return launch_generic_fmt<KF_RGB888>(k, blocks, threads, st);
-    case KF_SLOT8: return launch_generic_fmt<KF_SLOT8>(k, blocks, threads, st);
-    case KF_SLOT16: return launch_generic_fmt<KF_SLOT16>(k, blocks, threads, st);
-    case KF_PLANAR: return launch_generic_fmt<KF_PLANAR>(k, blocks, threads, st);
-    default: return launch_generic_fmt<KF_SLOT32>(k, blocks, threads, st);
+int launch(const KernelChoice& c, void* stream) {
+  const KPlan& k = c.k;
+  KernelFn fn;
+  unsigned threads = (unsigned)k.block_threads + 32u;   // + producer warp
+  size_t smem = k.smem_bytes;
+  switch (c.family) {
+    case FAM_ROWS: fn = rows_for(k.f, k.kformat, k.sy == 0 && k.scb == 0 && k.scr == 0, k.trunc != 0); break;
+    case FAM_POOL: fn = pool_for(k.f, k.kformat, k.in_px_bytes == 4); break;
+    case FAM_FLEX: fn = flex_kernel(k.kformat, k.trunc != 0); break;
+    default:
+      if (c.grid == 0) return (int)cudaSuccess;
+      if ((uint64_t)k.n_frames * (uint64_t)k.band_rows >= (1ull << 32)) return (int)cudaErrorInvalidValue;
+      fn = generic_kernel(k.kformat, k.average && k.f > 1 ? k.f : 0, k.trunc != 0);
+      threads = 128u;   // four warps per CTA
+      smem = 0;
   }
+  fn<<<c.grid, threads, smem, (cudaStream_t)stream>>>(k);
+  return (int)cudaGetLastError();
 }
 
-int rows_kernel_set_attributes(size_t max_smem_optin) {
-  int e;
-  if ((e = flex_set_attributes(max_smem_optin)) != 0) return e;
-  if ((e = decode_set_attributes(max_smem_optin)) != 0) return e;
-  if ((e = pool_set_attributes_factor<2>(max_smem_optin)) != 0) return e;
-  if ((e = pool_set_attributes_factor<4>(max_smem_optin)) != 0) return e;
-  if ((e = pool_set_attributes_factor<8>(max_smem_optin)) != 0) return e;
-  if ((e = rows_set_attributes_factor<1>(max_smem_optin)) != 0) return e;
-  if ((e = rows_set_attributes_factor<2>(max_smem_optin)) != 0) return e;
-  if ((e = rows_set_attributes_factor<4>(max_smem_optin)) != 0) return e;
-  if ((e = rows_set_attributes_factor<8>(max_smem_optin)) != 0) return e;
-  return 0;
-}
-
-int launch_pool(const KPlan& k, unsigned grid, void* stream) {
-  switch (k.f) {
-    case 2: return launch_pool_factor<2>(k, grid, stream);
-    case 4: return launch_pool_factor<4>(k, grid, stream);
-    default: return launch_pool_factor<8>(k, grid, stream);
-  }
-}
-
-int launch_rows(const KPlan& k, unsigned grid, void* stream) {
-  switch (k.f) {
-    case 1: return launch_rows_factor<1>(k, grid, stream);
-    case 2: return launch_rows_factor<2>(k, grid, stream);
-    case 4: return launch_rows_factor<4>(k, grid, stream);
-    default: return launch_rows_factor<8>(k, grid, stream);
-  }
+// Raises the dynamic shared-memory limit of every instance of the TMA-staged kernels (the generic and LDG kernels use
+// static shared memory only).  Keys that select the same instance set it twice.
+int set_kernel_attributes(size_t max_smem_optin) {
+  cudaError_t e = cudaSuccess;
+  auto set = [&](auto fn) {
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)max_smem_optin);
+  };
+  for (int fmt = KF_YCC888; fmt <= KF_PLANAR; ++fmt)
+    for (const bool a : {false, true}) {
+      for (const bool b : {false, true})
+        for (const int f : {1, 2, 4, 8}) set(rows_for(f, fmt, a, b));
+      for (const int f : {2, 4, 8}) set(pool_for(f, fmt, a));
+      set(flex_kernel(fmt, a));
+    }
+  for (uint32_t hs_sh = 0; hs_sh < 3; ++hs_sh)
+    for (const bool vhold : {false, true})
+      for (const bool to_rgb : {false, true}) set(decode_kernel(hs_sh, vhold, to_rgb));
+  return (int)e;
 }
 
 }  // namespace csic

@@ -98,7 +98,7 @@ void ring_layout(KPlan& k, uint32_t stages, uint32_t meta_bytes) {
   k.out_buf_off = stages * k.stage_stride;
   k.meta_off = up128(k.out_buf_off + 2u * k.out_buf_stride);
   k.bar_off = up128(k.meta_off + stages * meta_bytes);
-  k.smem_bytes = k.bar_off + stages * 16u;
+  k.smem_bytes = k.bar_off + stages * kRingBarBytes;
 }
 
 // Halves the rows per tile until there are ~4 tiles per SM: small batches still spread over the chip.
@@ -339,8 +339,8 @@ bool plan_flex_kernel(KPlan& k, int sm_count, size_t max_smem_optin, int force_s
   k.out_buf_off = up128(in_bytes);
   k.out_buf_stride = up16(stage_bytes + 32u);                               // + slack: span_store reads one word ahead
   k.meta_off = k.out_buf_off + k.out_buf_stride;                            // held words of every stage
-  k.bar_off = up128(k.meta_off + stages * (uint32_t)kFlexMaxRows * 4u);     // full[S], empty[S] mbarriers, then S descriptors
-  k.smem_bytes = k.bar_off + stages * (16u + kFlexDescBytes);
+  k.bar_off = up128(k.meta_off + stages * (uint32_t)kFlexMaxRows * 4u);     // the ring's mbarriers, then S descriptors
+  k.smem_bytes = k.bar_off + stages * (kRingBarBytes + kFlexDescBytes);
   if (k.smem_bytes > max_smem_optin) return false;
   k.tall_ho = tall ? k.Ho : 0;
   if (tall) commit_tall(k);
@@ -498,7 +498,7 @@ bool plan_decode(const KPlan& k, int to_rgb, const DeviceLimits& dev, uint32_t t
     P.out_stride = (P.tile_px * 3u + 32u + 15u) & ~15u;
     P.desc_off = P.out_off + 2u * P.out_stride;
     P.bar_off = P.desc_off + S * kDecDescBytes;
-    return (size_t)P.bar_off + 2u * S * 8u;
+    return (size_t)P.bar_off + S * kRingBarBytes;
   };
   uint32_t S = (to_rgb || !w16) ? 3u : 2u;
   size_t smem = layout(T, S);

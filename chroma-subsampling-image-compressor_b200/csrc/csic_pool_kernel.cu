@@ -322,20 +322,10 @@ __global__ void __maxnreg__(F == 2 ? 56 : 72) csic_pool_kernel(const __grid_cons
   const uint32_t tid = threadIdx.x;
   const uint32_t NC = blockDim.x - 32u;
   const uint32_t sbase = smem_u32(smem);
-  const uint32_t S = (uint32_t)P.stages;
-  const uint32_t n_my = (P.n_tiles > blockIdx.x) ? (P.n_tiles - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
   const uint64_t pol = policy_evict_first();
-  const uint32_t full_bar = sbase + P.bar_off, empty_bar = full_bar + S * 8u;
   const uint32_t seg_row_bytes = P.tile_in_bytes / F;          // one input row part of a segment
-
-  if (tid == 0) {
-    for (uint32_t s = 0; s < S; ++s) {
-      mbar_init(full_bar + s * 8u, 1);
-      mbar_init(empty_bar + s * 8u, NC / 32u);
-    }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  __syncthreads();
+  const Ring ring(sbase + P.bar_off, (uint32_t)P.stages, P.n_tiles);
+  ring.init(NC / 32u);                                          // one arrive per consumer warp
 
   // ============================== producer warp ==============================================
   if (tid >= NC) {
@@ -344,18 +334,13 @@ __global__ void __maxnreg__(F == 2 ? 56 : 72) csic_pool_kernel(const __grid_cons
     if (lane != 0 && !pool_first) return;        // chroma-first orders: one lane feeds the TMA engine
     const uint32_t ipb = (uint32_t)P.in_px_bytes;
     uint32_t cached_line = 0xFFFFFFFFu, cached_frame = 0xFFFFFFFFu, cached_pair = 0;   // the last block this warp reduced
-    for (uint32_t i = 0; i < n_my; ++i) {
-      const uint32_t s = i % S;
-      if (i >= S) mbar_wait(empty_bar + s * 8u, ((i / S) - 1u) & 1u);
-      const uint32_t tile = blockIdx.x + i * gridDim.x;
-      const uint32_t t2 = tile / (uint32_t)P.nsplit;
-      const uint32_t seg = tile - t2 * (uint32_t)P.nsplit;
-      const uint32_t k = t2 / P.tiles_per_band;
-      const uint32_t tb = t2 - k * P.tiles_per_band;
-      const uint32_t ro0 = (uint32_t)P.row0 + tb * (uint32_t)P.tile_rows;
-      const uint32_t nrows = min((uint32_t)P.tile_rows, (uint32_t)(P.row0 + P.band_rows) - ro0);
+    for (uint32_t i = 0; i < ring.n_my; ++i) {
+      const Ring::Pos pos = ring.at(i);
+      ring.wait_empty(pos, i);
+      const RowTile t = row_tile(P, blockIdx.x + i * gridDim.x);
+      const uint32_t s = pos.s, seg = t.seg, k = t.k, ro0 = t.ro0, nrows = t.nrows;
       const uint8_t* frame = P.in + (uint64_t)k * P.in_frame_bytes;
-      const uint32_t bar = full_bar + s * 8u;
+      const uint32_t bar = ring.full(s);
       const uint32_t dst = sbase + s * P.stage_stride;
       const uint32_t aux = dst + (uint32_t)P.tile_rows * P.tile_in_bytes;    // kPoolMaxRows windows of 32 bytes
       PoolMeta* m = reinterpret_cast<PoolMeta*>(smem + P.meta_off) + s;
@@ -460,9 +445,10 @@ __global__ void __maxnreg__(F == 2 ? 56 : 72) csic_pool_kernel(const __grid_cons
   // which specialisation of pool_tile (see its MODE parameter)
   const int mode = C.trunc ? 4 : ((C.linear && C.pre_y == 0xFFu) ? (C.pool_first ? 3 : (C.vhold ? 1 : 2)) : 0);
 
-  for (uint32_t i = 0; i < n_my; ++i) {
-    const uint32_t s = i % S;
-    mbar_wait(full_bar + s * 8u, (i / S) & 1u);
+  for (uint32_t i = 0; i < ring.n_my; ++i) {
+    const Ring::Pos pos = ring.at(i);
+    const uint32_t s = pos.s;
+    ring.wait_full(pos);
     const uint32_t in_s = sbase + s * P.stage_stride;
     const uint32_t out_s = sbase + P.out_buf_off;     // 12-byte formats: one 384-byte staging slot per consumer warp
     const PoolMeta* m = reinterpret_cast<const PoolMeta*>(smem + P.meta_off) + s;
@@ -482,49 +468,20 @@ __global__ void __maxnreg__(F == 2 ? 56 : 72) csic_pool_kernel(const __grid_cons
     }
 
     __syncwarp();
-    if ((tid & 31u) == 0) mbar_arrive(empty_bar + s * 8u);
-  }
-}
-
-namespace {
-constexpr int kF = CSIC_POOL_F;
-
-template <int FMT, bool IN4>
-int launch_one(const KPlan& k, unsigned grid, cudaStream_t st) {
-  csic_pool_kernel<kF, FMT, IN4><<<grid, (unsigned)k.block_threads + 32u, k.smem_bytes, st>>>(k);
-  return (int)cudaGetLastError();
-}
-template <int FMT>
-int launch_fmt(const KPlan& k, unsigned grid, cudaStream_t st) {
-  return k.in_px_bytes == 4 ? launch_one<FMT, true>(k, grid, st) : launch_one<FMT, false>(k, grid, st);
-}
-template <int FMT, bool IN4>
-cudaError_t attr_one(size_t bytes) {
-  return cudaFuncSetAttribute(csic_pool_kernel<kF, FMT, IN4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-}
-}  // namespace
-
-template <>
-int launch_pool_factor<CSIC_POOL_F>(const KPlan& k, unsigned grid, void* stream) {
-  cudaStream_t st = (cudaStream_t)stream;
-  switch (k.kformat) {
-    case KF_YCC888: return launch_fmt<KF_YCC888>(k, grid, st);
-    case KF_RGB888: return launch_fmt<KF_RGB888>(k, grid, st);
-    case KF_SLOT8: return launch_fmt<KF_SLOT8>(k, grid, st);
-    case KF_SLOT16: return launch_fmt<KF_SLOT16>(k, grid, st);
-    default: return launch_fmt<KF_SLOT32>(k, grid, st);
+    if ((tid & 31u) == 0) mbar_arrive(ring.empty(s));
   }
 }
 
 template <>
-int pool_set_attributes_factor<CSIC_POOL_F>(size_t b) {
-  cudaError_t e;
-#define CSIC_ATTR(FMT)                                                  \
-  if ((e = attr_one<FMT, false>(b)) != cudaSuccess) return (int)e;      \
-  if ((e = attr_one<FMT, true>(b)) != cudaSuccess) return (int)e;
-  CSIC_ATTR(KF_YCC888) CSIC_ATTR(KF_RGB888) CSIC_ATTR(KF_SLOT8) CSIC_ATTR(KF_SLOT16) CSIC_ATTR(KF_SLOT32)
-#undef CSIC_ATTR
-  return (int)cudaSuccess;
+KernelFn pool_kernel<CSIC_POOL_F>(int kformat, bool in4) {
+  constexpr int F = CSIC_POOL_F;
+  switch (kformat) {
+    case KF_YCC888: return in4 ? csic_pool_kernel<F, KF_YCC888, true> : csic_pool_kernel<F, KF_YCC888, false>;
+    case KF_RGB888: return in4 ? csic_pool_kernel<F, KF_RGB888, true> : csic_pool_kernel<F, KF_RGB888, false>;
+    case KF_SLOT8: return in4 ? csic_pool_kernel<F, KF_SLOT8, true> : csic_pool_kernel<F, KF_SLOT8, false>;
+    case KF_SLOT16: return in4 ? csic_pool_kernel<F, KF_SLOT16, true> : csic_pool_kernel<F, KF_SLOT16, false>;
+    default: return in4 ? csic_pool_kernel<F, KF_SLOT32, true> : csic_pool_kernel<F, KF_SLOT32, false>;
+  }
 }
 
 }  // namespace csic

@@ -236,19 +236,9 @@ __global__ void __launch_bounds__(kMaxConsumerThreads + 32) csic_rows_kernel(con
   const uint32_t tid = threadIdx.x;
   const uint32_t NC = blockDim.x - 32u;        // consumer threads; the last warp is the producer
   const uint32_t sbase = smem_u32(smem);
-  const uint32_t S = (uint32_t)P.stages;
-  const uint32_t n_my = (P.n_tiles > blockIdx.x) ? (P.n_tiles - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
   const uint64_t pol = policy_evict_first();   // every byte is touched exactly once: do not keep it in L2
-  const uint32_t full_bar = sbase + P.bar_off, empty_bar = full_bar + S * 8u;
-
-  if (tid == 0) {
-    for (uint32_t s = 0; s < S; ++s) {
-      mbar_init(full_bar + s * 8u, 1);            // the producer's arrive.expect_tx
-      mbar_init(empty_bar + s * 8u, NC / 32u);    // one arrive per consumer warp
-    }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  __syncthreads();
+  const Ring ring(sbase + P.bar_off, (uint32_t)P.stages, P.n_tiles);
+  ring.init(NC / 32u);                          // one arrive per consumer warp
 
   // ============================== producer warp ==============================================
   // Walks this CTA's tiles S deep ahead of the consumers.  All lanes track the geometry; the per-row work of a tile
@@ -259,18 +249,13 @@ __global__ void __launch_bounds__(kMaxConsumerThreads + 32) csic_rows_kernel(con
     const uint32_t lane = tid - NC;
     const uint32_t ipb = (uint32_t)P.in_px_bytes;
     const bool one_copy = P.row_step == 1 && P.nsplit == 1 && P.in_dense;   // consecutive rows are contiguous in memory
-    for (uint32_t i = 0; i < n_my; ++i) {
-      const uint32_t s = i % S;
-      if (i >= S) mbar_wait(empty_bar + s * 8u, ((i / S) - 1u) & 1u);   // consumers drained the previous use
-      const uint32_t tile = blockIdx.x + i * gridDim.x;
-      const uint32_t t2 = tile / (uint32_t)P.nsplit;
-      const uint32_t seg = tile - t2 * (uint32_t)P.nsplit;
-      const uint32_t k = t2 / P.tiles_per_band;
-      const uint32_t tb = t2 - k * P.tiles_per_band;
-      const uint32_t ro0 = (uint32_t)P.row0 + tb * (uint32_t)P.tile_rows;
-      const uint32_t nrows = min((uint32_t)P.tile_rows, (uint32_t)(P.row0 + P.band_rows) - ro0);
+    for (uint32_t i = 0; i < ring.n_my; ++i) {
+      const Ring::Pos pos = ring.at(i);
+      ring.wait_empty(pos, i);
+      const RowTile t = row_tile(P, blockIdx.x + i * gridDim.x);
+      const uint32_t s = pos.s, seg = t.seg, k = t.k, ro0 = t.ro0, nrows = t.nrows;
       const uint8_t* frame = P.in + (uint64_t)k * P.in_frame_bytes;
-      const uint32_t bar = full_bar + s * 8u;
+      const uint32_t bar = ring.full(s);
       const uint32_t dst = sbase + s * P.stage_stride;
       const uint32_t aux = dst + (uint32_t)P.tile_rows * P.tile_in_bytes;    // 32-byte window per row
       TileMeta* m = reinterpret_cast<TileMeta*>(smem + P.meta_off) + s;
@@ -364,9 +349,10 @@ __global__ void __launch_bounds__(kMaxConsumerThreads + 32) csic_rows_kernel(con
   const int hfe = P.hfe;
   const bool in4 = P.in_px_bytes == 4;
 
-  for (uint32_t i = 0; i < n_my; ++i) {
-    const uint32_t s = i % S;
-    mbar_wait(full_bar + s * 8u, (i / S) & 1u);
+  for (uint32_t i = 0; i < ring.n_my; ++i) {
+    const Ring::Pos pos = ring.at(i);
+    const uint32_t s = pos.s;
+    ring.wait_full(pos);
 
     const uint32_t in_s = sbase + s * P.stage_stride;
     const uint32_t out_s = sbase + P.out_buf_off + (i & 1u) * P.out_buf_stride;
@@ -405,7 +391,7 @@ __global__ void __launch_bounds__(kMaxConsumerThreads + 32) csic_rows_kernel(con
     }
     // This warp is done with stage s and its meta: give it back to the producer.
     __syncwarp();
-    if ((tid & 31u) == 0) mbar_arrive(empty_bar + s * 8u);
+    if ((tid & 31u) == 0) mbar_arrive(ring.empty(s));
   }
   if (kStaged && tid == 0) tma_store_wait_all();
 }
@@ -413,47 +399,21 @@ __global__ void __launch_bounds__(kMaxConsumerThreads + 32) csic_rows_kernel(con
 
 namespace {
 constexpr int kF = CSIC_ROWS_F;
-
-template <int FMT, bool Q8, bool TR>
-int launch_one(const KPlan& k, unsigned grid, cudaStream_t st) {
-  csic_rows_kernel<kF, FMT, Q8, TR><<<grid, (unsigned)k.block_threads + 32u, k.smem_bytes, st>>>(k);   // + producer warp
-  return (int)cudaGetLastError();
-}
-template <int FMT>
-int launch_fmt(const KPlan& k, unsigned grid, cudaStream_t st) {
-  const bool q8 = FMT == KF_SLOT32 && k.sy == 0 && k.scb == 0 && k.scr == 0;
-  if (q8) return k.trunc ? launch_one<FMT, (FMT == KF_SLOT32), true>(k, grid, st) : launch_one<FMT, (FMT == KF_SLOT32), false>(k, grid, st);
-  return k.trunc ? launch_one<FMT, false, true>(k, grid, st) : launch_one<FMT, false, false>(k, grid, st);
-}
-template <int FMT, bool Q8, bool TR>
-cudaError_t attr_one(size_t bytes) {
-  return cudaFuncSetAttribute(csic_rows_kernel<kF, FMT, Q8, TR>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-}
+template <int FMT, bool Q8>
+KernelFn by_trunc(bool trunc) { return trunc ? csic_rows_kernel<kF, FMT, Q8, true> : csic_rows_kernel<kF, FMT, Q8, false>; }
 }  // namespace
 
+// q8: the bundle's slots keep all 8 bits of every channel (only KF_SLOT32 has an instance for it)
 template <>
-int launch_rows_factor<CSIC_ROWS_F>(const KPlan& k, unsigned grid, void* stream) {
-  cudaStream_t st = (cudaStream_t)stream;
-  switch (k.kformat) {
-    case KF_YCC888: return launch_fmt<KF_YCC888>(k, grid, st);
-    case KF_RGB888: return launch_fmt<KF_RGB888>(k, grid, st);
-    case KF_SLOT8: return launch_fmt<KF_SLOT8>(k, grid, st);
-    case KF_SLOT16: return launch_fmt<KF_SLOT16>(k, grid, st);
-    case KF_PLANAR: return launch_fmt<KF_PLANAR>(k, grid, st);
-    default: return launch_fmt<KF_SLOT32>(k, grid, st);
+KernelFn rows_kernel<kF>(int kformat, bool q8, bool trunc) {
+  switch (kformat) {
+    case KF_YCC888: return by_trunc<KF_YCC888, false>(trunc);
+    case KF_RGB888: return by_trunc<KF_RGB888, false>(trunc);
+    case KF_SLOT8: return by_trunc<KF_SLOT8, false>(trunc);
+    case KF_SLOT16: return by_trunc<KF_SLOT16, false>(trunc);
+    case KF_PLANAR: return by_trunc<KF_PLANAR, false>(trunc);
+    default: return q8 ? by_trunc<KF_SLOT32, true>(trunc) : by_trunc<KF_SLOT32, false>(trunc);
   }
-}
-
-template <>
-int rows_set_attributes_factor<CSIC_ROWS_F>(size_t b) {
-  cudaError_t e;
-#define CSIC_ATTR(FMT, Q8)                                                   \
-  if ((e = attr_one<FMT, Q8, false>(b)) != cudaSuccess) return (int)e;       \
-  if ((e = attr_one<FMT, Q8, true>(b)) != cudaSuccess) return (int)e;
-  CSIC_ATTR(KF_YCC888, false) CSIC_ATTR(KF_RGB888, false) CSIC_ATTR(KF_SLOT8, false) CSIC_ATTR(KF_SLOT16, false)
-  CSIC_ATTR(KF_SLOT32, false) CSIC_ATTR(KF_SLOT32, true) CSIC_ATTR(KF_PLANAR, false)
-#undef CSIC_ATTR
-  return (int)cudaSuccess;
 }
 
 }  // namespace csic

@@ -1,8 +1,11 @@
-// TMA / mbarrier / shared-memory PTX wrappers shared by the TMA-staged kernels (sm_100a).
+// TMA / mbarrier / shared-memory PTX wrappers shared by the TMA-staged kernels (sm_100a), and their common skeleton: the
+// stage ring and the row tiles.
 #ifndef CSIC_TMA_CUH_
 #define CSIC_TMA_CUH_
 #include <cuda_runtime.h>
 #include <cstdint>
+
+#include "csic_internal.h"
 
 namespace csic {
 
@@ -61,6 +64,68 @@ __device__ __forceinline__ uint64_t policy_evict_first() {
   uint64_t pol;
   asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
   return pol;
+}
+
+// The S-stage ring of a TMA-staged kernel.  The producer warp fills stage s and arrives on full(s) (its bulk copies add
+// their bytes to that phase); the consumers wait on full(s), use the stage and arrive on empty(s), on which the producer
+// waits before it refills the stage.  Barriers at `bar`: full[S], then empty[S] (kRingBarBytes per stage).  A CTA
+// walks tiles blockIdx.x, blockIdx.x + gridDim.x, ... of n_tiles: n_my of them.
+struct Ring {
+  uint32_t bar, ebar, S, n_my;
+  // Stage of a tile and the parity of the barrier phase it waits for, which flips each lap of the ring.
+  struct Pos {
+    uint32_t s = 0, ph = 0;
+    __device__ __forceinline__ void next(uint32_t S) {
+      if (++s == S) { s = 0; ph ^= 1u; }
+    }
+  };
+  __device__ __forceinline__ Ring(uint32_t bar_, uint32_t stages, uint32_t n_tiles)
+      : bar(bar_), ebar(bar_ + stages * 8u), S(stages),
+        n_my(n_tiles > blockIdx.x ? (n_tiles - blockIdx.x + gridDim.x - 1) / gridDim.x : 0) {}
+  // the position of this CTA's i-th tile, for loops that would rather divide than carry a Pos (the row and pooling
+  // kernels: counters there cost registers)
+  __device__ __forceinline__ Pos at(uint32_t i) const {
+    Pos p;
+    p.s = i % S;
+    p.ph = (i / S) & 1u;
+    return p;
+  }
+  __device__ __forceinline__ uint32_t full(uint32_t s) const { return bar + s * 8u; }
+  __device__ __forceinline__ uint32_t empty(uint32_t s) const { return ebar + s * 8u; }
+  // full[] counts the producer's one arrive, empty[] `empty_arrivals` consumer arrives; every thread of the CTA calls it
+  __device__ __forceinline__ void init(uint32_t empty_arrivals) const {
+    if (threadIdx.x == 0) {
+      for (uint32_t s = 0; s < S; ++s) {
+        mbar_init(full(s), 1);
+        mbar_init(empty(s), empty_arrivals);
+      }
+      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    __syncthreads();
+  }
+  // producer, before it fills the i-th tile's stage: from the second lap on, the consumers must have drained its last use
+  __device__ __forceinline__ void wait_empty(const Pos& p, uint32_t i) const {
+    if (i >= S) mbar_wait(empty(p.s), p.ph ^ 1u);
+  }
+  // consumers: the stage's bytes have landed and the producer's shared-memory writes are visible
+  __device__ __forceinline__ void wait_full(const Pos& p) const { mbar_wait(full(p.s), p.ph); }
+};
+static_assert(kRingBarBytes == 2u * 8u, "a ring stage has one 8-byte full and one 8-byte empty mbarrier");
+
+// Tile `tile` of the row and pooling kernels: segment seg of row tile tb of frame k (tile = (k * tiles_per_band + tb) *
+// nsplit + seg), output rows [ro0, ro0 + nrows).
+struct RowTile {
+  uint32_t seg, k, ro0, nrows;
+};
+__device__ __forceinline__ RowTile row_tile(const KPlan& P, uint32_t tile) {
+  RowTile t;
+  const uint32_t t2 = tile / (uint32_t)P.nsplit;
+  t.seg = tile - t2 * (uint32_t)P.nsplit;
+  t.k = t2 / P.tiles_per_band;
+  const uint32_t tb = t2 - t.k * P.tiles_per_band;
+  t.ro0 = (uint32_t)P.row0 + tb * (uint32_t)P.tile_rows;
+  t.nrows = min((uint32_t)P.tile_rows, (uint32_t)(P.row0 + P.band_rows) - t.ro0);
+  return t;
 }
 
 __device__ __forceinline__ uint32_t lds32(uint32_t a) {
