@@ -1,6 +1,8 @@
 // Runs the kernel planners (csic_plan.cpp) without a GPU.  One case per input line, one result line per case:
 //   F W H a b f ops fmt in pool n row0 rows compact family stages tile_bytes block_threads ctas_per_sm
+//     [in_pitch in_frame out_pitch out_frame]
 //     -> family grid stages ctas_per_sm tile_rows nsplit tile_px n_tiles block_threads smem_bytes Ho n_frames tall_ho
+//        slots_per_row in_dense out_dense
 //   D W H a b f n to_rgb tile_px
 //     -> ok tile_px stages threads grid smem
 //   H W H a b f ops fmt in pool n row0 rows full_frames chunk_bytes share_gpus
@@ -10,7 +12,8 @@
 //   B W H a b f ops G
 //     -> r0 r1 of each of G GPUs (band_split)
 // `ops` is the stage order as three digits of csic_step (e.g. 312 = chroma, spatial, colour); rows -1: all.  Buffers
-// are dense and 4 KiB aligned.  Device limits: argv[1] SMs, argv[2] opt-in shared memory per block.  A line that fails
+// are 4 KiB aligned and dense, except that an F line may end in a layout (row pitches and frame strides in bytes, 0 =
+// dense, as csic_process_device_pitched takes them).  Device limits: argv[1] SMs, argv[2] opt-in shared memory per block.  A line that fails
 // parameter validation, build_plan or plan_host prints "error <code>".
 #include <algorithm>
 #include <cstdio>
@@ -70,18 +73,22 @@ int main(int argc, char** argv) {
       csic::PlanOptions opt;
       in >> ops >> fmt >> in_fmt >> pool >> n >> row0 >> rows >> compact >> opt.family >> opt.stages >> opt.tile_bytes >>
           opt.block_threads >> opt.ctas_per_sm;
+      csic::Layout lay;
+      for (size_t* v : {&lay.in_pitch, &lay.in_frame, &lay.out_pitch, &lay.out_frame})
+        if (!(in >> *v)) *v = 0;
       set_ops(p, ops);
       p.out_format = fmt; p.in_format = in_fmt; p.pool_mode = pool;
       if (rc == CSIC_OK) rc = csic_validate(&p, nullptr, 0);
       csic::KPlan base;
       if (rc == CSIC_OK)
         rc = csic::build_plan(p, in_buf, out_buf, n, row0, rows < 0 ? csic::geometry(p).out_h : rows, compact != 0,
-                              csic::Layout(), base);
+                              lay, base);
       if (rc != CSIC_OK) { std::printf("error %d\n", rc); continue; }
       const csic::KernelChoice c = csic::select_kernel(base, dev, opt);
       const csic::KPlan& k = c.k;
-      std::printf("%d %u %d %d %d %d %d %u %d %u %d %u %d\n", c.family, c.grid, k.stages, k.ctas_per_sm, k.tile_rows, k.nsplit,
-                  k.tile_px, k.n_tiles, k.block_threads, k.smem_bytes, k.Ho, k.n_frames, k.tall_ho);
+      std::printf("%d %u %d %d %d %d %d %u %d %u %d %u %d %d %d %d\n", c.family, c.grid, k.stages, k.ctas_per_sm, k.tile_rows,
+                  k.nsplit, k.tile_px, k.n_tiles, k.block_threads, k.smem_bytes, k.Ho, k.n_frames, k.tall_ho, k.slots_per_row,
+                  k.in_dense, k.out_dense);
     } else if (kind == "D") {
       size_t n;
       int to_rgb;

@@ -705,7 +705,9 @@ def test_decoder_full_size_batches(csic, ctx, W, H, ab):
 
 def test_row_segments_and_ring_depths(csic, ctx):
     """Force rows to be split into several tiles (CSIC_OPT_TILE_BYTES small -> nsplit > 1: held chroma comes from
-    TMA-fetched aux windows, per-segment stores) and vary ring depth / block size / CTAs per SM: results never change."""
+    TMA-fetched aux windows, per-segment stores) under other block sizes and CTAs per SM: results never change.  These
+    batches are small: no CTA gets more than one tile, so no stage is reused at the forced depths; ring reuse at every
+    depth is tests/test_tile_walks.py's."""
     rng = np.random.default_rng(5)
     try:
         for tile_bytes, stages, threads, ctas in [(1024, 2, 128, 1), (3072, 3, 256, 3), (6144, 4, 64, 2), (16384, 2, 512, 1)]:
