@@ -1,6 +1,6 @@
 // Runs the kernel planners (csic_plan.cpp) without a GPU.  One case per input line, one result line per case:
 //   F W H a b f ops fmt in pool n row0 rows compact family stages tile_bytes block_threads ctas_per_sm
-//     [in_pitch in_frame out_pitch out_frame]
+//     [in_pitch in_frame out_pitch out_frame [y_bits cb_bits cr_bits]]
 //     -> family grid stages ctas_per_sm tile_rows nsplit tile_px n_tiles block_threads smem_bytes Ho n_frames tall_ho
 //        slots_per_row in_dense out_dense
 //   D W H a b f n to_rgb tile_px
@@ -13,8 +13,9 @@
 //     -> r0 r1 of each of G GPUs (band_split)
 // `ops` is the stage order as three digits of csic_step (e.g. 312 = chroma, spatial, colour); rows -1: all.  Buffers
 // are 4 KiB aligned and dense, except that an F line may end in a layout (row pitches and frame strides in bytes, 0 =
-// dense, as csic_process_device_pitched takes them).  Device limits: argv[1] SMs, argv[2] opt-in shared memory per block.  A line that fails
-// parameter validation, build_plan or plan_host prints "error <code>".
+// dense, as csic_process_device_pitched takes them) and then in the bit depths of Y, Cb and Cr (default 8 each: they
+// set the slot width of the bundle formats).  Device limits: argv[1] SMs, argv[2] opt-in shared memory per block.  A
+// line that fails parameter validation, build_plan or plan_host prints "error <code>".
 #include <algorithm>
 #include <cstdio>
 #include <cstdlib>
@@ -76,6 +77,10 @@ int main(int argc, char** argv) {
       csic::Layout lay;
       for (size_t* v : {&lay.in_pitch, &lay.in_frame, &lay.out_pitch, &lay.out_frame})
         if (!(in >> *v)) *v = 0;
+      int bits[3] = {8, 8, 8};
+      for (int& b : bits)
+        if (!(in >> b)) b = 8;
+      p.y_bits = bits[0]; p.cb_bits = bits[1]; p.cr_bits = bits[2];
       set_ops(p, ops);
       p.out_format = fmt; p.in_format = in_fmt; p.pool_mode = pool;
       if (rc == CSIC_OK) rc = csic_validate(&p, nullptr, 0);
