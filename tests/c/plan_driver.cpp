@@ -3,8 +3,10 @@
 //     [in_pitch in_frame out_pitch out_frame [y_bits cb_bits cr_bits]]
 //     -> family grid stages ctas_per_sm tile_rows nsplit tile_px n_tiles block_threads smem_bytes Ho n_frames tall_ho
 //        slots_per_row in_dense out_dense
-//   D W H a b f n to_rgb tile_px
+//   D W H a b f n to_rgb tile_px [walk]
 //     -> ok tile_px stages threads grid smem
+//        [tiles_per_frame n_tiles A cw hs_sh vhold last_c y_slot c_slot frame_bytes cb_off cr_off]
+//        (with any trailing token: what the decoder's producer reads from DecPlan; "0" when plan_decode declines)
 //   H W H a b f ops fmt in pool n row0 rows full_frames chunk_bytes share_gpus
 //     -> one JSON object: the host plan (plan_host) and, per chunk, the copies (frame_copies) of the direct path
 //        (h2d: caller -> staging, d2h: staging -> caller) and of the bounce path (gather: caller -> bounce, b2d, d2b,
@@ -110,7 +112,13 @@ int main(int argc, char** argv) {
         std::printf("0\n");
         continue;
       }
-      std::printf("1 %u %u %u %u %zu\n", d.P.tile_px, d.P.stages, d.threads, d.grid, d.smem);
+      std::printf("1 %u %u %u %u %zu", d.P.tile_px, d.P.stages, d.threads, d.grid, d.smem);
+      std::string more;
+      if (in >> more)
+        std::printf(" %u %u %u %u %u %u %u %u %u %llu %llu %llu", d.P.tiles_per_frame, d.P.n_tiles, d.P.A, d.P.cw, d.P.hs_sh,
+                    d.P.vhold, d.P.last_c, d.P.y_slot, d.P.c_slot, (unsigned long long)d.P.frame_bytes,
+                    (unsigned long long)d.P.cb_off, (unsigned long long)d.P.cr_off);
+      std::printf("\n");
     } else if (kind == "H") {
       int ops, fmt, in_fmt, pool, row0, rows, full;
       size_t n, chunk, gpus;

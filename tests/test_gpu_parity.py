@@ -675,9 +675,10 @@ def test_decoder_any_width_and_alignment(csic, ctx, no_tma, monkeypatch):
 @pytest.mark.parametrize("W,H,ab", [(1920, 1080, (2, 0)), (1918, 1078, (2, 0)), (333, 500, (2, 2)), (1001, 999, (1, 0))],
                          ids=["1080p420", "1918x1078", "333x500", "1001x999"])
 def test_decoder_full_size_batches(csic, ctx, W, H, ab):
-    """The decoder at bench size (every CTA walks many tiles, the stage ring wraps many times, frames start at every
-    alignment): 32 frames of random planes against a torch gather on the device (YCC888, all frames) and the oracle's
-    ycbcr2rgb (RGB888, first and last frame)."""
+    """The decoder at bench size with the planner's own tiles (every CTA walks many tiles and the stage ring wraps):
+    32 frames of random planes against a torch gather on the device (YCC888, all frames) and the oracle's ycbcr2rgb
+    (RGB888, first and last frame).  1920 takes the 16-pixel path, the other widths the column-phase path; no shape here
+    takes the AL4 path or mixes paths in one launch -- those, and the other regimes, are tests/test_decode_walks.py's."""
     import torch
     p, _ = both_params(csic, W, H, ab[0], ab[1], (8, 8, 8), 1, "CSQ", 0, 0, 4)
     w, h, _, fb = csic.out_shape(p)
