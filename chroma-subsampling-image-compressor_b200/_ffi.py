@@ -59,6 +59,7 @@ PROTOTYPES = {
     "csic_set_option": (_int, [_vp, _int, _i64]),
     "csic_host_bytes": (_int, [_vp, ctypes.POINTER(ctypes.c_uint64)]),
     "csic_last_kernel": (_int, [_vp, ctypes.POINTER(_i32), ctypes.POINTER(_i64)]),
+    "csic_last_walk": (_int, [_vp, ctypes.POINTER(_i32)]),
 }
 
 _lib = None

@@ -231,6 +231,12 @@ class Context:
         check(_ffi.lib().csic_last_kernel(self._h, ctypes.byref(fam), ctypes.byref(n)))
         return fam.value, n.value
 
+    def last_walk(self):
+        """1: the last call's row kernel dealt its tiles from a ticket counter; 0: round robin or another kernel."""
+        t = ctypes.c_int32()
+        check(_ffi.lib().csic_last_walk(self._h, ctypes.byref(t)))
+        return t.value
+
     # -- raw device pointers (ints); asynchronous on `stream` (int cudaStream_t handle, 0/None = ctx stream)
     def process_device(self, p, d_rgb, n_frames, d_out, stream=None):
         check(_ffi.lib().csic_process_device(self._h, ctypes.byref(p), d_rgb, n_frames, d_out, stream or None))

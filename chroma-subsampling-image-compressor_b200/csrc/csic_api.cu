@@ -35,6 +35,11 @@ using csic::kPipe;
 // Input bytes per pipelined chunk.  B200 + PCIe 5 x16, 4K batches (profiles/r2/e2e_chunk_sweep.txt): 16 MB 32.6 k MP/s,
 // 32 MB 32.3 k, 64 MB (round 1) 31.9 k, 128 MB 31.3 k -- the pipeline's fill and drain cost one chunk each per call.
 constexpr size_t kDefaultChunkBytes = 16u << 20;
+constexpr size_t kTicketPairs = 64;
+
+#ifdef CSIC_PROBE_WINDOW
+uint64_t* g_probe = nullptr;   // csic_probe_window: the row kernel's drift-probe buffer for the launches that follow
+#endif
 
 // No C++ exception may cross the C ABI (the caller is a JVM, Python or C): std::thread / std::vector / std::string can
 // throw system_error or bad_alloc inside the host pipeline.
@@ -71,6 +76,15 @@ struct csic_ctx {
   size_t opt_chunk_bytes = kDefaultChunkBytes;
   int opt_no_compact = 0;
   uint64_t h2d_bytes = 0;    // bytes csic_process_host has shipped host -> device so far
+  // The row kernel's ticket counters (KPlan::tickets): kTicketPairs zeroed pairs, the i-th for the i-th stream this
+  // context has launched a ticketed plan on (ticket_pair).  A pair is only ever used by launches enqueued directly on
+  // its stream, which run one after the other, so no two running launches share one -- and every launch leaves it
+  // zeroed for the next.
+  uint32_t* d_tickets = nullptr;
+  struct TicketStream { cudaStream_t st; std::thread::id thread; };
+  TicketStream ticket_streams[kTicketPairs] = {};
+  size_t n_ticket_streams = 0;
+  int last_ticketed = 0;
 };
 
 namespace {
@@ -87,6 +101,25 @@ struct DeviceGuard {
   }
 };
 
+// The counter pair of launches on `st`, or null: the launch then walks its tiles round robin.  A launch being captured
+// into a graph gets none -- the graph may be replayed on any stream, next to anything, and after the context is gone.
+// cudaStreamPerThread names a different stream in every host thread, so there the thread is part of the key.  Past
+// kTicketPairs streams, none.
+uint32_t* ticket_pair(csic_ctx* ctx, cudaStream_t st) {
+  cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+  if (cudaStreamIsCapturing(st, &cap) != cudaSuccess) {   // e.g. the legacy stream while another stream captures
+    cudaGetLastError();                                    // (the launch itself reports whatever is wrong)
+    return nullptr;
+  }
+  if (cap != cudaStreamCaptureStatusNone) return nullptr;
+  const std::thread::id th = st == cudaStreamPerThread ? std::this_thread::get_id() : std::thread::id();
+  size_t i = 0;
+  while (i < ctx->n_ticket_streams && !(ctx->ticket_streams[i].st == st && ctx->ticket_streams[i].thread == th)) ++i;
+  if (i == kTicketPairs) return nullptr;
+  if (i == ctx->n_ticket_streams) ctx->ticket_streams[ctx->n_ticket_streams++] = {st, th};
+  return ctx->d_tickets + 2 * i;
+}
+
 int run(csic_ctx* ctx, const csic_params* p, const void* d_rgb, size_t n_frames, void* d_out, int32_t row0,
         int32_t rows, void* cuda_stream, bool compact = false, const csic::Layout& lay = csic::Layout()) {
   if (!ctx || !p) return CSIC_EINVAL_ARG;
@@ -98,11 +131,19 @@ int run(csic_ctx* ctx, const csic_params* p, const void* d_rgb, size_t n_frames,
   rc = csic::build_plan(*p, d_rgb, d_out, n_frames, row0, rows, compact, lay, base);
   if (rc != CSIC_OK) return rc;
   if (row0 < 0 || rows < 0 || row0 + rows > base.Ho) return CSIC_EINVAL_ARG;
+#ifdef CSIC_PROBE_WINDOW
+  base.probe = g_probe;
+#endif
   DeviceGuard guard(ctx->device);
   cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : ctx->stream;
-  const csic::KernelChoice c = csic::select_kernel(base, ctx->dev, ctx->opt);
+  csic::KernelChoice c = csic::select_kernel(base, ctx->dev, ctx->opt);
+  if (c.family == csic::FAM_ROWS && c.k.ticketed) {
+    c.k.tickets = ticket_pair(ctx, st);
+    if (!c.k.tickets) c.k.ticketed = 0;
+  }
   const int err = csic::launch(c, st);
   ctx->last_family = c.family;
+  ctx->last_ticketed = c.family == csic::FAM_ROWS && c.k.ticketed;
   ctx->launches += 1;
   if (err != (int)cudaSuccess) return cuda_fail((cudaError_t)err, "kernel launch");
   return CSIC_OK;
@@ -124,6 +165,15 @@ int grow_ring(csic_ctx::Ring& r, size_t bytes, Alloc alloc, Release release) {
 extern "C" {
 
 const char* csic_last_error(void) { return g_last_error.c_str(); }
+
+#ifdef CSIC_PROBE_WINDOW
+// Probe builds only (not part of include/csic.h): the device buffer the row kernel's launches from now on record their
+// tile starts and CTA ends into (KPlan::probe: 16 bytes per tile plus 16 per CTA); null turns the probe off.
+CSIC_API int csic_probe_window(void* d_buf) {
+  g_probe = static_cast<uint64_t*>(d_buf);
+  return CSIC_OK;
+}
+#endif
 
 int csic_device_count(void) {
   int n = 0;
@@ -165,6 +215,9 @@ int csic_create(int device, csic_ctx** out) {
     step(cudaEventCreateWithFlags(&c->ev_h2d[i], cudaEventDisableTiming)) &&
         step(cudaEventCreateWithFlags(&c->ev_k[i], cudaEventDisableTiming)) &&
         step(cudaEventCreateWithFlags(&c->ev_d2h[i], cudaEventDisableTiming));
+  if (err == cudaSuccess) step(cudaMalloc(&c->d_tickets, kTicketPairs * 2 * sizeof(uint32_t))) &&
+      step(cudaMemsetAsync(c->d_tickets, 0, kTicketPairs * 2 * sizeof(uint32_t), c->stream)) &&
+      step(cudaStreamSynchronize(c->stream));   // (a non-blocking stream does not wait for a legacy-stream memset)
   if (err == cudaSuccess) step((cudaError_t)csic::set_kernel_attributes(c->dev.max_smem_optin));
   if (err != cudaSuccess) {
     const int rc = cuda_fail(err, "csic_create");
@@ -192,6 +245,7 @@ int csic_destroy(csic_ctx* ctx) {
     if (ctx->ev_k[i]) cudaEventDestroy(ctx->ev_k[i]);
     if (ctx->ev_d2h[i]) cudaEventDestroy(ctx->ev_d2h[i]);
   }
+  if (ctx->d_tickets) cudaFree(ctx->d_tickets);
   for (cudaStream_t st : {ctx->stream, ctx->s_h2d, ctx->s_d2h})
     if (st) cudaStreamDestroy(st);
   delete ctx;
@@ -663,6 +717,12 @@ int csic_synchronize(csic_ctx* ctx) {
 int csic_host_bytes(const csic_ctx* ctx, uint64_t* h2d_total) {
   if (!ctx) return CSIC_EINVAL_ARG;
   if (h2d_total) *h2d_total = ctx->h2d_bytes;
+  return CSIC_OK;
+}
+
+int csic_last_walk(const csic_ctx* ctx, int32_t* ticketed) {
+  if (!ctx) return CSIC_EINVAL_ARG;
+  if (ticketed) *ticketed = ctx->last_ticketed;
   return CSIC_OK;
 }
 

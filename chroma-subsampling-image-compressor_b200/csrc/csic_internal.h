@@ -63,9 +63,16 @@ struct KPlan {
   int32_t stages;
   int32_t block_threads;
   int32_t ctas_per_sm;
+  int32_t ticketed;                      // row kernel: tiles dealt from a per-launch counter (TileDeal, csic_tma.cuh)
+  uint32_t* tickets;                     // that counter pair: set per launch by csic_api.cu, one pair per stream
   uint32_t stage_stride, out_buf_off, out_buf_stride, meta_off, bar_off, smem_bytes;
   uint32_t qmask;                        // my | mcb<<8 | mcr<<16 (per-channel keep masks)
   int32_t tall_ho;                       // flex kernel: != 0 -> the batch is addressed as ONE image of n * Ho rows; rows per original frame
+#ifdef CSIC_PROBE_WINDOW
+  // row kernel drift probe (tools/rows_window_probe.py), null when off: n_tiles records {%globaltimer when the producer
+  // takes the tile, CTA}, indexed by tile, then one record per CTA: {%globaltimer when it is done, 2^32 | CTA}
+  uint64_t* probe;
+#endif
 };
 
 // Constants shared by the planners (csic_plan.cpp) and the kernels.

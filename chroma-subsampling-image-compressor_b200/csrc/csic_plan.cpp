@@ -195,6 +195,11 @@ bool plan_rows_kernel(KPlan& k, int sm_count, size_t max_smem_optin, int force_s
   // (PLANAR 1080p: 0.97 of the copy peak with 3 CTAs vs 0.84 with 2; 16-bit bundles: 0.93 with 4).
   k.ctas_per_sm = (int32_t)std::min<uint32_t>(ctas_for(stages), tiny ? 8u : (k.f == 1 ? 4u : 2u));
   k.stages = stages;
+  // Direct stores at f >= 2 (the 4K headline): tiles from a per-launch counter.  Under the round robin the 296 CTAs of
+  // cfg4 drift up to 157 frames apart over one launch, and HBM serves the scattered stream worse: ticketed 3.055 ms
+  // vs 3.189 ms, the window 1.3 frames at the median instead of 82 (B200, profiles/r3/README.md).  The other row-kernel
+  // plans measured the same either way and keep the round robin.
+  k.ticketed = !staged && k.f >= 2;
   if (tall) commit_tall(k);
   ring_layout(k, (uint32_t)stages, kTileMetaBytes);
   return true;

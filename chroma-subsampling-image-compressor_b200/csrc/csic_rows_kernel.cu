@@ -64,6 +64,14 @@ struct TileMeta {
 };
 static_assert(sizeof(TileMeta) == kTileMetaBytes, "kTileMetaBytes out of sync");
 
+#ifdef CSIC_PROBE_WINDOW
+__device__ __forceinline__ uint64_t globaltimer() {
+  uint64_t t;
+  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+  return t;
+}
+#endif
+
 // Runtime constants of the inner loop, hoisted into registers once per kernel.
 struct LoopConst {
   uint32_t qm0, qm1, qm2;            // YCC888: quantiser keep-masks over the three packed words
@@ -239,26 +247,45 @@ __global__ void __launch_bounds__(kMaxConsumerThreads + 32) csic_rows_kernel(con
   const uint64_t pol = policy_evict_first();   // every byte is touched exactly once: do not keep it in L2
   const Ring ring(sbase + P.bar_off, (uint32_t)P.stages, P.n_tiles);
   ring.init(NC / 32u);                          // one arrive per consumer warp
+  const TileDeal deal{P.tickets};
 
   // ============================== producer warp ==============================================
-  // Walks this CTA's tiles S deep ahead of the consumers.  All lanes track the geometry; the per-row work of a tile
-  // (where a held row finds its chroma, the row's own bulk copy when rows are not contiguous) is spread over the
-  // lanes -- a tile of small frames has up to 64 rows -- and every lane announces its copies on the stage's mbarrier
+  // Walks this CTA's tiles S deep ahead of the consumers: round robin (blockIdx.x, + gridDim.x, ...), or, in a ticketed
+  // plan, blockIdx.x and then whatever tile the launch's counter deals next (TileDeal).  After the last one it hands the
+  // consumers a stage whose meta says "no more tiles" (out_base == 0).  All lanes track the geometry; the per-row work
+  // of a tile (where a held row finds its chroma, the row's own bulk copy when rows are not contiguous) is spread over
+  // the lanes -- a tile of small frames has up to 64 rows -- and every lane announces its copies on the stage's mbarrier
   // (expect_tx); lane 0 describes the tile in TileMeta and arrives once for the warp.
   if (tid >= NC) {
     const uint32_t lane = tid - NC;
     const uint32_t ipb = (uint32_t)P.in_px_bytes;
     const bool one_copy = P.row_step == 1 && P.nsplit == 1 && P.in_dense;   // consecutive rows are contiguous in memory
-    for (uint32_t i = 0; i < ring.n_my; ++i) {
+    uint32_t tile = blockIdx.x;
+    for (uint32_t i = 0;; ++i) {
       const Ring::Pos pos = ring.at(i);
+      // the next tile, taken one ahead: the counter's round trip overlaps the wait for this tile's stage and its copies
+      uint32_t next = tile + gridDim.x;
+      if (P.ticketed && lane == 0 && tile < P.n_tiles) next = deal.take();
       ring.wait_empty(pos, i);
-      const RowTile t = row_tile(P, blockIdx.x + i * gridDim.x);
-      const uint32_t s = pos.s, seg = t.seg, k = t.k, ro0 = t.ro0, nrows = t.nrows;
+      const uint32_t s = pos.s;
+      TileMeta* m = reinterpret_cast<TileMeta*>(smem + P.meta_off) + s;
+      if (tile >= P.n_tiles) {                 // no more tiles: the stage's meta tells the consumers so
+        if (lane == 0) {
+          m->out_base = 0;
+          mbar_arrive(ring.full(s));
+          if (P.ticketed) deal.leave();
+        }
+        break;
+      }
+#ifdef CSIC_PROBE_WINDOW
+      if (lane == 0 && P.probe) { P.probe[2u * tile] = globaltimer(); P.probe[2u * tile + 1u] = blockIdx.x; }
+#endif
+      const RowTile t = row_tile(P, tile);
+      const uint32_t seg = t.seg, k = t.k, ro0 = t.ro0, nrows = t.nrows;
       const uint8_t* frame = P.in + (uint64_t)k * P.in_frame_bytes;
       const uint32_t bar = ring.full(s);
       const uint32_t dst = sbase + s * P.stage_stride;
       const uint32_t aux = dst + (uint32_t)P.tile_rows * P.tile_in_bytes;    // 32-byte window per row
-      TileMeta* m = reinterpret_cast<TileMeta*>(smem + P.meta_off) + s;
       const uint8_t* src = frame + (uint64_t)(ro0 * (uint32_t)P.row_step) * P.in_row_bytes + (uint64_t)seg * P.tile_in_bytes;
 
       // Which rows replay a held chroma pair, and from where?  (KPlan::hfe covers the in-row hold.)
@@ -319,6 +346,7 @@ __global__ void __launch_bounds__(kMaxConsumerThreads + 32) csic_rows_kernel(con
       // meta is published by the release of this arrive and observed after the consumers' acquire-wait; the phase
       // completes when the last announced byte has landed
       if (lane == 0) mbar_arrive(bar);
+      tile = __shfl_sync(0xFFFFFFFFu, next, 0);
     }
     return;
   }
@@ -349,7 +377,7 @@ __global__ void __launch_bounds__(kMaxConsumerThreads + 32) csic_rows_kernel(con
   const int hfe = P.hfe;
   const bool in4 = P.in_px_bytes == 4;
 
-  for (uint32_t i = 0; i < ring.n_my; ++i) {
+  for (uint32_t i = 0;; ++i) {
     const Ring::Pos pos = ring.at(i);
     const uint32_t s = pos.s;
     ring.wait_full(pos);
@@ -357,6 +385,7 @@ __global__ void __launch_bounds__(kMaxConsumerThreads + 32) csic_rows_kernel(con
     const uint32_t in_s = sbase + s * P.stage_stride;
     const uint32_t out_s = sbase + P.out_buf_off + (i & 1u) * P.out_buf_stride;
     const TileMeta* m = reinterpret_cast<const TileMeta*>(smem + P.meta_off) + s;
+    if (m->out_base == 0) break;               // the producer has no more tiles
     uint8_t* out_g = reinterpret_cast<uint8_t*>(m->out_base);
     const uint32_t ngr = m->n_granules & 0x00FFFFFFu, nrc = m->n_granules >> 24;
     const uint32_t out_bytes = ngr * kGranOut;
@@ -394,6 +423,9 @@ __global__ void __launch_bounds__(kMaxConsumerThreads + 32) csic_rows_kernel(con
     if ((tid & 31u) == 0) mbar_arrive(ring.empty(s));
   }
   if (kStaged && tid == 0) tma_store_wait_all();
+#ifdef CSIC_PROBE_WINDOW
+  if (tid == 0 && P.probe) { P.probe[2u * (P.n_tiles + blockIdx.x)] = globaltimer(); P.probe[2u * (P.n_tiles + blockIdx.x) + 1u] = (1ull << 32) | blockIdx.x; }
+#endif
 }
 
 

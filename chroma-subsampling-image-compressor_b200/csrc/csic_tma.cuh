@@ -112,6 +112,25 @@ struct Ring {
 };
 static_assert(kRingBarBytes == 2u * 8u, "a ring stage has one 8-byte full and one 8-byte empty mbarrier");
 
+// Ticket dealing of a persistent grid's tiles (the row kernel in a ticketed plan, KPlan::ticketed): a CTA's first tile is
+// blockIdx.x, each further one gridDim.x + the next value of a counter every CTA of the launch draws from, so that CTAs
+// that run ahead take more tiles and the grid stays on one narrow band of the batch instead of drifting apart over a
+// static round robin (cfg4 on a B200: 1.3 frames in flight at the median instead of 82, profiles/r3/README.md).
+// `ctr` is a pair of words that is zero when the launch starts: [0] tickets drawn, [1] CTAs done drawing.  A CTA calls
+// leave() once, after its last take(); the last one to leave has seen every take() of the launch and zeroes the pair,
+// so the next launch in stream order finds it zero again -- no memset, no host bookkeeping.  Launches that share a pair
+// must therefore never overlap (csic_api.cu: one pair per stream, none for launches captured into a graph).
+struct TileDeal {
+  uint32_t* ctr;
+  __device__ __forceinline__ uint32_t take() const { return gridDim.x + atomicAdd(ctr, 1u); }
+  __device__ __forceinline__ void leave() const {
+    if (atomicAdd(ctr + 1, 1u) == gridDim.x - 1u) {
+      atomicExch(ctr, 0u);
+      atomicExch(ctr + 1, 0u);
+    }
+  }
+};
+
 // Tile `tile` of the row and pooling kernels: segment seg of row tile tb of frame k (tile = (k * tiles_per_band + tb) *
 // nsplit + seg), output rows [ro0, ro0 + nrows).
 struct RowTile {

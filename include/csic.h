@@ -263,6 +263,14 @@ CSIC_API int csic_host_bytes(const csic_ctx* ctx, uint64_t* h2d_total);
  * kernel) and how many kernels it launched. */
 CSIC_API int csic_last_kernel(const csic_ctx* ctx, int32_t* family, int64_t* launches_total);
 
+/* Diagnostics: 1 when the last process call's row kernel dealt its tiles from a ticket counter, 0 when its CTAs walked
+ * them round robin (or another kernel ran).  The planner deals by ticket where that measured faster (direct bundle
+ * stores at f >= 2).  The counter is a pair of words the context keeps per stream (for its first 64 streams), which
+ * every launch leaves zeroed; only launches enqueued directly on that stream use it, so they never overlap.  A launch
+ * captured into a CUDA graph walks round robin and holds no context memory: graphs may be replayed on any stream, at
+ * the same time as other work, and after csic_destroy. */
+CSIC_API int csic_last_walk(const csic_ctx* ctx, int32_t* ticketed);
+
 #ifdef __cplusplus
 }
 #endif
